@@ -15,6 +15,9 @@ At N = 1 the `configs` block adds prove / verify / end-to-end figures for the ot
 each with its cold (first call: generators and tables are built) and warm times.
 --impl reference : the CPU restatement of the reference (oracle/, OpenMP over chunks, all host cores) on a bounded
 sample of the same workload; the real Rust reference cannot be built here (no cargo), see DESIGN.md.
+--dump-outputs DIR : after the timed steps, the proofs and commitments of the last resident step (proofs.npy, commitments.npy) and
+of the last end-to-end step (e2e_proofs.npy, e2e_commitments.npy), bytes as float32.  Inputs and proof seeds depend only on the
+arguments, so two builds run with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -114,7 +117,18 @@ def cpu_reference_run(steps, warmup, sample_chunks=None):
             times.append((t1 - t0, t2 - t1))
     tp = float(np.mean([a for a, _ in times])); tv = float(np.mean([b for _, b in times]))
     return dict(value=Ds / (tp + tv), prove_eps=Ds / tp, verify_eps=Ds / tv, cores=cores, steps=steps, warmup=warmup,
-                sample=f"{chunks} chunks x {m} values ({Ds} elements) of the same workload per step, OpenMP over chunks, {steps} timed steps after {warmup} warm-up", ms=(tp + tv) * 1e3)
+                sample=f"{chunks} chunks x {m} values ({Ds} elements) of the same workload per step, OpenMP over chunks, {steps} timed steps after {warmup} warm-up", ms=(tp + tv) * 1e3,
+                outputs=dict(proofs=p, commitments=c))
+
+
+def dump_outputs(path, arrays):
+    """Write what the timed path returned in its last step as <path>/<name>.npy.  The proof and commitment bytes are stored as
+    float32 (exact for 0..255), so that two builds of the project can be compared output for output."""
+    arrays = {k: np.asarray(a, dtype=np.float32) for k, a in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def wall(f):
@@ -283,7 +297,10 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the `configs` / `strong` blocks (only the contract metric on configs[1])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the proofs and commitments of the last timed step as DIR/<name>.npy (float32; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     w = WORKLOAD
     # stdout carries exactly ONE JSON line: everything any library prints to fd 1 meanwhile (NCCL's version banner at NCCL_DEBUG=VERSION
@@ -296,7 +313,9 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        r = cpu_reference_run(max(1, min(args.steps, 5)), min(args.warmup, 1))
+        r = cpu_reference_run(args.steps, min(args.warmup, 1))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         line = dict(metric=METRIC, value=r["value"], unit="elements/s", n_gpus=args.gpus, steps=args.steps, warmup=args.warmup, ms_per_step=r["ms"], higher_is_better=True,
                     scaling="weak", vs_baseline=None, dtype="u32 limbs (GF(2^255-19), mod l) on CPU u64", data="synthetic", impl="reference", config=bench_config(args.gpus),
                     cpu_baseline=dict(value=r["value"], unit="elements/s", cores=r["cores"], kind="port", sample=r["sample"], prove_eps=r["prove_eps"], verify_eps=r["verify_eps"]),
@@ -364,7 +383,7 @@ def main():
         ok = api.range_verify(proofs, commits, rb, bytes([it % 249 + 2] * 32))
         e2.record(stream); e2.synchronize()
         assert rc == 0 and ok == 1
-        return e0.elapsed_time(e1), e1.elapsed_time(e2)
+        return e0.elapsed_time(e1), e1.elapsed_time(e2), proofs, commits
 
     # cold: the very first prove / verify of this shape on the device derives the Bulletproofs generators and builds their radix-2^11 tables
     cold_p, cold_v, _ = step_resident(0)
@@ -385,6 +404,7 @@ def main():
     for it in range(args.steps):
         a, b, proofs = step_resident(100 + it); t_p += a; t_v += b; per_step.append((round(a, 2), round(b, 2)))
     barrier()
+    outputs = dict(proofs=proofs, commitments=commits_d.cpu().numpy())      # the last timed step's (the profiling pass reuses commits_d)
     if rank == 0:
         print("resident per-step (prove_ms, verify_ms):", per_step, file=sys.stderr)
     launches = lib.rofl_prof_launches(-1)
@@ -393,7 +413,7 @@ def main():
     e_p = e_v = 0.0
     per_step = []
     for it in range(args.steps):
-        a, b = step_e2e(200 + it); e_p += a; e_v += b; per_step.append((round(a, 2), round(b, 2)))
+        a, b, outputs["e2e_proofs"], outputs["e2e_commitments"] = step_e2e(200 + it); e_p += a; e_v += b; per_step.append((round(a, 2), round(b, 2)))
     barrier()
     if rank == 0:
         print("e2e per-step (prove_ms, verify_ms):", per_step, file=sys.stderr)
@@ -427,6 +447,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     K = args.steps
     ms_step = (t_p + t_v) / K
     value = world * D / (ms_step / 1e3)

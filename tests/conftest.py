@@ -30,17 +30,3 @@ def oracle():
     import oracle as o
     o.build()
     return o
-
-
-@pytest.fixture(scope="session")
-def sodium():
-    """libsodium (ristretto255) shipped inside pyzmq's wheel: an independent anchor for the oracle."""
-    import ctypes, glob
-    import zmq  # noqa: F401  (locates site-packages)
-    cands = glob.glob(os.path.join(os.path.dirname(os.path.dirname(zmq.__file__)), "pyzmq.libs", "libsodium*.so*"))
-    if not cands:
-        pytest.skip("libsodium not found")
-    lib = ctypes.CDLL(cands[0])
-    if lib.sodium_init() < 0:
-        pytest.skip("sodium_init failed")
-    return lib

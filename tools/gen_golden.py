@@ -8,6 +8,7 @@ Two kinds of fixtures (the reference itself ships no golden vectors and cannot b
                    tests) for fixed seeds: commitments, range / L2 / square proofs, aggregates and decrypted values.  They
                    freeze the byte-level behaviour so that the GPU box (which has neither /root/reference nor a need to
                    re-derive anything) can compare the CUDA path against committed bytes.
+  sodium.json      libsodium's outputs for the seeded inputs of tests/test_oracle_primitives.py, which compares the oracle with them.
 Usage: python tools/gen_golden.py   (deterministic; re-running must not change the files)
 """
 import ctypes as C
@@ -45,6 +46,32 @@ def sod(lib, name, outlen, *ins):
 
 def sha(b):
     return hashlib.sha256(bytes(b)).hexdigest()
+
+
+def sodium_vectors(lib):
+    """libsodium's answers for the inputs tests/test_oracle_primitives.py draws (same generators, same order), so that the
+    oracle is compared with libsodium without loading it at test time."""
+    out = {"source": "libsodium crypto_core_ristretto255_* / crypto_scalarmult_ristretto255*", "scalar": [], "group": [], "valid": []}
+    rng = np.random.default_rng(1)
+    for _ in range(200):
+        a = (int.from_bytes(rng.bytes(32), "little") % L).to_bytes(32, "little")
+        b = (int.from_bytes(rng.bytes(32), "little") % L).to_bytes(32, "little")
+        w = rng.bytes(64)
+        out["scalar"].append({"a": a.hex(), "b": b.hex(), "wide": w.hex(), "mul": sod(lib, "crypto_core_ristretto255_scalar_mul", 32, a, b).hex(),
+                              "reduce": sod(lib, "crypto_core_ristretto255_scalar_reduce", 32, w).hex()})
+    rng = np.random.default_rng(3)
+    for _ in range(40):
+        h = rng.bytes(64)
+        p = sod(lib, "crypto_core_ristretto255_from_hash", 32, h)
+        s = (int.from_bytes(rng.bytes(32), "little") % L).to_bytes(32, "little")
+        q = sod(lib, "crypto_scalarmult_ristretto255", 32, s, p)
+        out["group"].append({"hash": h.hex(), "point": p.hex(), "scalar": s.hex(), "scalarmult": q.hex(), "scalarmult_base": sod(lib, "crypto_scalarmult_ristretto255_base", 32, s).hex(),
+                             "add": sod(lib, "crypto_core_ristretto255_add", 32, p, q).hex(), "sub": sod(lib, "crypto_core_ristretto255_sub", 32, p, q).hex()})
+    P = 2**255 - 19
+    edge = [bytes(32), bytes([1] + [0] * 31), P.to_bytes(32, "little"), (P - 1).to_bytes(32, "little"), bytes([0xff] * 32), bytes([2] + [0] * 30 + [0x80])]
+    for e in edge + [rng.bytes(32) for _ in range(300)]:
+        out["valid"].append({"bytes": e.hex(), "valid": bool(lib.crypto_core_ristretto255_is_valid_point(C.c_char_p(e)))})
+    return out
 
 
 def main():
@@ -135,10 +162,10 @@ def main():
     prot["bp_gens"] = {"G_party0_first4": np.asarray(oracle.bp_gens("G", 0, 4)).tobytes().hex(), "H_party0_first4": np.asarray(oracle.bp_gens("H", 0, 4)).tobytes().hex(),
                        "G_party5_first2": np.asarray(oracle.bp_gens("G", 5, 2)).tobytes().hex()}
     os.makedirs(os.path.join(ROOT, "tests", "golden"), exist_ok=True)
-    for name, obj in [("primitives.json", prim), ("protocol.json", prot)]:
+    for name, obj in [("primitives.json", prim), ("protocol.json", prot), ("sodium.json", sodium_vectors(lib))]:
         with open(os.path.join(ROOT, "tests", "golden", name), "w") as f:
             json.dump(obj, f, indent=1, sort_keys=True); f.write("\n")
-    print("wrote tests/golden/primitives.json, protocol.json")
+    print("wrote tests/golden/primitives.json, protocol.json, sodium.json")
 
 
 if __name__ == "__main__":
