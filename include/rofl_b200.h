@@ -217,6 +217,12 @@ void *rofl_ctx_stream(rofl_ctx *);        /* the cudaStream_t the context launch
 int rofl_debug_ts_absorb(rofl_ctx *, const uint8_t *V32, size_t m, int n, int label_id);
 int rofl_debug_square_rlc(rofl_ctx *, const uint8_t *proofs160, const uint8_t *commits64, size_t D);   /* the batched square-proof check alone: 1 holds, 0 does not */
 int rofl_debug_verify_weights(rofl_ctx *, const uint8_t *proofs, size_t proof_len, size_t n_proofs, const uint8_t *commits32, size_t D, int range, const uint8_t seed[32], uint8_t *out_weights);
+/* the MSM front end alone (production plan / forced window width / generator tables, then k_finalize): out32[k] = sum_t s[k][t] P_t + sB[k] B + sH[k] H.
+ * scalars32: n_msm x T canonical scalars; points32: T shared or n_msm x T (points_per_msm) encodings, or NULL for BulletproofGens(gen_n, T / (2 gen_n));
+ * path 0 = msm_plan_for(T, n_msm, big_min), 1 = window width c with `knob` slices (c <= 8) / parts (c >= 9), 2 = generator tables.  sB32 / sH32 may be NULL.
+ * info (nullable, 3 ints): width, slices / parts / blocks, kernel (0 k_msm, 1 k_bm_*, 2 k_rt_msm).  0 ok, ROFL_ERR_ARGS (non-canonical scalar), ROFL_ERR_POINT */
+int rofl_debug_msm(rofl_ctx *, const uint8_t *scalars32, size_t n_msm, size_t T, const uint8_t *points32, int points_per_msm, int gen_n,
+                   int path, int c, int knob, size_t big_min, const uint8_t *sB32, const uint8_t *sH32, uint8_t *out32, int *info);
 #ifdef __cplusplus
 }
 #endif

@@ -70,6 +70,7 @@ _SIGS = {
     "rofl_enc_l2_compressed_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_sz, c_u8p, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, C.c_int, c_u8p, c_vp]),
     "rofl_debug_ts_absorb": (C.c_int, [c_vp, c_u8p, c_sz, C.c_int, C.c_int]),
     "rofl_debug_verify_weights": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, c_u8p, c_u8p]),
+    "rofl_debug_msm": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_sz, c_u8p, c_u8p, c_u8p, c_vp]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGS)
 
@@ -291,6 +292,21 @@ class Api:
         rc = self.lib.rofl_debug_verify_weights(self.h, _ptr(p), p.shape[1], p.shape[0], _ptr(c), c.shape[0], rng, _ptr(_seed(seed)), _ptr(w))
         if rc <= ROFL_ERR_CUDA: raise self._err(rc)
         return rc, w
+
+    def debug_msm(self, scalars, points=None, gen_n=0, path=0, c=0, knob=1, big_min=0, sB=None, sH=None):
+        """The MSM front end alone: scalars [n_msm, T, 32] (canonical); points None (generators BulletproofGens(gen_n, T / (2 gen_n)), G then H),
+        [T, 32] shared by every instance or [n_msm, T, 32]; path 0 production plan (big_min as msm_plan_for), 1 window width c with `knob` slices / parts,
+        2 generator tables.  -> (rc, out [n_msm, 32] compressed sums, (width, slices | parts | blocks, kernel))"""
+        s = _u8(scalars); n_msm, T = s.shape[0], s.shape[1]; s = s.reshape(n_msm, T, 32)
+        p = None if points is None else _u8(points)
+        per = 0 if p is None or p.ndim == 2 else 1
+        if p is not None:
+            assert p.shape == ((n_msm, T, 32) if per else (T, 32)), p.shape
+        b = None if sB is None else _u8(sB, 32 * n_msm); h = None if sH is None else _u8(sH, 32 * n_msm)
+        out = np.zeros((n_msm, 32), np.uint8); info = np.zeros(3, np.int32)
+        rc = self.lib.rofl_debug_msm(self.h, _ptr(s), n_msm, T, _ptr(p), per, gen_n, path, c, knob, big_min, _ptr(b), _ptr(h), _ptr(out), _ptr(info))
+        if rc <= ROFL_ERR_CUDA: raise self._err(rc)
+        return rc, out, tuple(int(x) for x in info)
 
     def set_option(self, name, value):
         rc = self.lib.rofl_set_option(self.h, name.encode(), int(value))

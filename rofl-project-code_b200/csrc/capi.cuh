@@ -535,7 +535,7 @@ extern "C" int rofl_enc_l2_compressed_verify_batch(rofl_ctx *c, size_t n_clients
     API_CATCH
 }
 
-// ---- test hooks (tests/test_emul_vs_oracle.py, tests/test_gpu_parity.py) ------------------------------------------------------------------------
+// ---- test hooks (tests/test_emul_vs_oracle.py, tests/test_gpu_parity.py, tests/test_msm_kernels.py) -----------------------------------------------
 // the warp-cooperative V absorb (ts_kernels.cuh, k_ts_absorbV) against the sequential transcript code for the same m commitments: 0 equal, 1 different
 extern "C" int rofl_debug_ts_absorb(rofl_ctx *c, const uint8_t *V32, size_t m, int n, int label_id) {
     API_TRY
@@ -568,5 +568,75 @@ extern "C" int rofl_debug_verify_weights(rofl_ctx *c, const uint8_t *proofs, siz
     lane_guard lg(c->e);
     staged_in dc(commits, 32 * D, lg.s());
     return engine_range_verify(c->e, proofs, plen, np, dc.b.as<uint8_t>(), D, range, seed, nullptr, out_weights);
+    API_CATCH
+}
+// the MSM front end alone: out32[k] = sum_t s[k][t] P_t (+ sB[k] B + sH[k] H), k < n_msm, through the production plan / kernels / k_finalize.
+//   scalars32: n_msm x T canonical scalars; one >= l is ROFL_ERR_ARGS (the signed recoding and the fat-top-window bound assume reduced scalars).
+//   points32: compressed bases, T shared by all instances (points_per_msm = 0) or n_msm x T (1), split into two segments at ceil(T / 2) like the
+//     verifier's commitments | proof points; an undecodable one is ROFL_ERR_POINT.  NULL: the generators BulletproofGens(gen_n, T / (2 gen_n)), G then H.
+//   path 0: msm_plan_for(T, n_msm, big_min); 1: msm_plan_forced(T, c, knob); 2: the generator tables (k_rt_msm, generators only).
+//   sB32 / sH32: n_msm scalars each, or NULL.  info (nullable): window width, slices (k_msm) / parts (k_bm_*) / blocks (k_rt_msm), kernel 0 / 1 / 2.
+extern "C" int rofl_debug_msm(rofl_ctx *c, const uint8_t *scalars32, size_t n_msm, size_t T, const uint8_t *points32, int points_per_msm, int gen_n,
+                              int path, int cw, int knob, size_t big_min, const uint8_t *sB32, const uint8_t *sH32, uint8_t *out32, int *info) {
+    API_TRY
+    if (!scalars32 || !out32 || !n_msm || n_msm > 0xffff || !T || n_msm * T > 0x7fffffffu || path < 0 || path > 2) return ROFL_ERR_ARGS;
+    if (points32 ? path == 2 : (gen_n <= 0 || T % (2 * (size_t)gen_n))) return ROFL_ERR_ARGS;
+    auto canonical = [](std::vector<sc_st> &o, const uint8_t *b, size_t n) {
+        o.resize(n);
+        for (size_t i = 0; i < n; i++) { sc x; sc_frombytes(x, b + 32 * i); if (!sc_is_canonical(x)) return false; sc_to_st(o[i], x); }
+        return true;
+    };
+    std::vector<sc_st> hs, hB, hH;
+    if (!canonical(hs, scalars32, n_msm * T) || (sB32 && !canonical(hB, sB32, n_msm)) || (sH32 && !canonical(hH, sH32, n_msm))) return ROFL_ERR_ARGS;
+    lane_guard lg(c->e); cudaStream_t s = lg.s();
+    staged_in ds(hs.data(), sizeof(sc_st) * hs.size(), s), dB(hB.data(), sizeof(sc_st) * hB.size(), s), dH(hH.data(), sizeof(sc_st) * hH.size(), s);
+    dev_buf dout(32 * n_msm, s);
+    finalize_args f = {}; f.sBa = sB32 ? dB.b.as<sc_st>() : nullptr; f.sHa = sH32 ? dH.b.as<sc_st>() : nullptr; f.tabB = c->e.sh->tabB; f.tabH = c->e.sh->tabH;
+    f.out32 = dout.as<uint8_t>(); f.count = (int)n_msm;
+    int inf[3] = {0, 0, 0};
+    msm_args a = {}; a.v[0].scalars = ds.b.as<sc_st>(); a.split = (uint32_t)n_msm; a.T = (uint32_t)T; a.scalar_stride = (uint32_t)T; a.nseg = 2;
+    auto msm = [&](const msm_plan &pl) {
+        dev_buf d_win(sizeof(p3_st) * pl.out_count(n_msm), s);
+        a.out = d_win.as<p3_st>();
+        run_msm(c->e, s, a, pl, (uint32_t)n_msm);
+        fin_windows(f, d_win.as<p3_st>(), pl);
+        run_finalize(s, f);
+        rt_d2h(out32, dout.p, 32 * n_msm, s); rt_sync(s);
+        inf[0] = pl.c; inf[1] = (int)(pl.big ? pl.parts : pl.slices); inf[2] = pl.big ? 1 : 0;
+    };
+    const msm_plan pl = path == 1 ? msm_plan_forced(T, cw, knob) : msm_plan_for(T, n_msm, big_min);
+    if (points32) {
+        const size_t np = points_per_msm ? n_msm * T : T;
+        const uint32_t h = (uint32_t)((T + 1) / 2), stride = points_per_msm ? (uint32_t)T : 0;
+        staged_in dp(points32, 32 * np, s); dev_buf d_pts(sizeof(p3_st) * np, s), d_bad(sizeof(int), s);
+        rt_memset(d_bad.p, 0, sizeof(int), s);
+        LAUNCH(k_decompress, dim3((unsigned)((np + 127) / 128)), dim3(128), s, d_pts.as<p3_st>(), (uint8_t *)nullptr, dp.b.as<uint8_t>(), np, np, (const p3_st *)nullptr, d_bad.as<int>(), np);
+        int bad = 0; rt_d2h(&bad, d_bad.p, sizeof(int), s); rt_sync(s);
+        if (bad) return ROFL_ERR_POINT;
+        a.v[0].seg[0] = mk_seg(d_pts.as<p3_st>(), h, stride, 1); a.v[0].seg[1] = mk_seg(d_pts.as<p3_st>() + h, (uint32_t)T - h, stride, 1);
+        msm(pl);
+    } else {
+        const int m = (int)(T / (2 * (size_t)gen_n)); const uint32_t N = (uint32_t)(T / 2);
+        tables_use tu(*c->e.sh);
+        engine_gens(c->e, tu, s, gen_n, m);
+        rt_tables rt; const bool have_rt = path == 2 && engine_rt(c->e, tu, s, gen_n, m, rt);
+        const gens_entry g = engine_gens(c->e, tu, s, gen_n, m);
+        if (path == 2) {
+            if (!have_rt) return ROFL_ERR_ARGS;
+            const int nb = rt_blocks(T, (int)n_msm);
+            dev_buf d_part(sizeof(p3_st) * (size_t)nb * n_msm, s);
+            rt_msm_args ra = {}; ra.scalars = ds.b.as<sc_st>(); ra.T = (uint32_t)T; ra.scalar_stride = (uint32_t)T; ra.nG = N; ra.mode = 0; ra.rt = rt; ra.partial = d_part.as<p3_st>();
+            run_rt_msm(c->e, s, ra, nb, (uint32_t)n_msm);
+            f.partial = d_part.as<p3_st>(); f.npartial = nb;
+            run_finalize(s, f);
+            rt_d2h(out32, dout.p, 32 * n_msm, s); rt_sync(s);
+            inf[0] = rt.c; inf[1] = nb; inf[2] = 2;
+        } else {
+            a.v[0].seg[0] = mk_seg(g.G, N, 0, 0); a.v[0].seg[1] = mk_seg(g.H, N, 0, 0);
+            msm(pl);
+        }
+    }
+    if (info) memcpy(info, inf, sizeof(inf));
+    return 0;
     API_CATCH
 }

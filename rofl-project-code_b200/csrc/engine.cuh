@@ -326,16 +326,20 @@ static inline int msm_pick_c(size_t T) {
     return best;
 }
 static inline size_t bm_min_terms() { static const size_t v = getenv("ROFL_BM_MIN") ? (size_t)atoll(getenv("ROFL_BM_MIN")) : (size_t)32768; return v; }
+// a forced plan (tests): window width c (clamped to 3 .. 16) and one more knob -- term slices for k_msm (c <= 8, clamped to 1 .. T), parts per
+// bucket for k_bm_* (c >= 9, clamped to 1 .. 8)
+static inline msm_plan msm_plan_forced(size_t T, int c, int knob) {
+    msm_plan p; p.c = std::max(3, std::min(16, c)); p.nw = msm_nw(p.c); p.slices = 1; p.slice_len = (uint32_t)T;
+    if (p.c > 8) { p.big = true; p.parts = (uint32_t)std::max(1, std::min(8, knob)); return p; }
+    if (T > 0) { p.slices = (uint32_t)std::max<size_t>(1, std::min<size_t>(std::max(knob, 1), T)); p.slice_len = (uint32_t)((T + p.slices - 1) / p.slices); p.slices = (uint32_t)((T + p.slice_len - 1) / p.slice_len); }
+    return p;
+}
 // big_min: smallest T for the sorted wide-window form (0 = the default bm_min_terms(); single verifier-side MSMs pass 2048: k_msm needs 3.6 ms for
 // the 10 000 terms of a configs[0] verification -- 76 blocks walking 32 windows -- the sorted form 0.5 ms)
 static inline msm_plan msm_plan_for(size_t T, size_t n_msm, size_t big_min = 0) {
     msm_plan p; p.c = msm_pick_c(T); p.slices = 1; p.slice_len = (uint32_t)T;
-    if (const char *fc = getenv("ROFL_MSM_C")) {       // test hook: force the window width / slicing
-        p.c = std::max(3, std::min(16, atoi(fc)));
-        if (p.c > 8) { p.big = true; p.parts = getenv("ROFL_MSM_SLICES") ? (uint32_t)std::max(1, std::min(8, atoi(getenv("ROFL_MSM_SLICES")))) : 1; p.nw = msm_nw(p.c); return p; }
-        if (const char *fs = getenv("ROFL_MSM_SLICES")) { p.slices = (uint32_t)std::max<size_t>(1, std::min<size_t>(atoi(fs), T)); p.slice_len = (uint32_t)((T + p.slices - 1) / p.slices); p.slices = (uint32_t)((T + p.slice_len - 1) / p.slice_len); }
-        p.nw = msm_nw(p.c); return p;
-    }
+    if (const char *fc = getenv("ROFL_MSM_C"))         // test hook: force the window width / slicing
+        return msm_plan_forced(T, atoi(fc), getenv("ROFL_MSM_SLICES") ? atoi(getenv("ROFL_MSM_SLICES")) : 1);
     if (T >= (big_min ? big_min : bm_min_terms())) {   // wide windows, buckets sorted in global memory (kernels.cuh K4b): ~64 terms per bucket
         p.big = true; p.c = std::max(9, std::min(16, ilog2_sz(T + 1) - 6)); p.nw = msm_nw(p.c);
         const size_t threads = n_msm * (size_t)p.nw * ((size_t)1 << (p.c - 1));
