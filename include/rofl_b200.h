@@ -190,6 +190,15 @@ int rofl_range_verify_batch(rofl_ctx *, const uint8_t *proofs, size_t proof_len,
 int rofl_enc_l2_compressed_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *enc_values96, size_t D, const uint8_t *square_proofs160, const uint8_t *range_proofs,
                                         size_t proof_len, size_t n_proofs, const uint8_t *square_range_proofs, size_t sq_proof_len, int prove_range, int l2_range,
                                         const uint8_t seed[32], int *out_ok);
+/* K compressed rand proofs (helper_verify, compressed_rand_proof/mod.rs:149-158) in one batched check.  proofs128: n_clients x 128,
+ * pairs64: n_clients x D x 64.  out_ok[k] = exactly what rofl_crp_verify(proofs128[k], pairs64[k], D) returns: 1, 0, ROFL_ERR_FORMAT, -6.
+ * Return value: 0, or < 0 for bad arguments. */
+int rofl_crp_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *proofs128, const uint8_t *pairs64, size_t D, const uint8_t seed[32], int *out_ok);
+/* EncModelParams::verify, EncRangeCompressed arm (params.rs:236-256), for n_clients messages of one shape: enc_values64 n_clients x D x 64,
+ * rand_proofs128 n_clients x 128, range_proofs n_clients x n_proofs x proof_len.  out_ok[k] = exactly what rofl_enc_range_compressed_verify(message k,
+ * check_percentage, seed) returns (1 / 0).  Return value: 0, or ROFL_ERR_ARGS (D == 0, n_proofs == 0, null out_ok). */
+int rofl_enc_range_compressed_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *enc_values64, size_t D, const uint8_t *rand_proofs128, const uint8_t *range_proofs,
+                                           size_t proof_len, size_t n_proofs, int prove_range, float check_percentage, const uint8_t seed[32], int *out_ok);
 
 /* ---- aggregation: EncModelParamsAccumulator::accumulate_other (params.rs:81-124) / pedersen_ops::add_rp_vec_vec
  *      (pedersen_ops.rs:56-69; bindings32.rs:64 `add_commitments`).  points32: n_clients x D encodings, client-major.
@@ -216,6 +225,8 @@ void *rofl_ctx_stream(rofl_ctx *);        /* the cudaStream_t the context launch
  *      scalars (c_i | rho_i, 2 x n_proofs x 32 bytes) rofl_range_verify derives for a call (return value as rofl_range_verify) */
 int rofl_debug_ts_absorb(rofl_ctx *, const uint8_t *V32, size_t m, int n, int label_id);
 int rofl_debug_square_rlc(rofl_ctx *, const uint8_t *proofs160, const uint8_t *commits64, size_t D);   /* the batched square-proof check alone: 1 holds, 0 does not */
+/* the batched compressed-rand-proof check of rofl_crp_verify_batch alone: 1 = the combination over all n_clients proofs held and none is malformed, 0 = it did not */
+int rofl_debug_crp_rlc(rofl_ctx *, size_t n_clients, const uint8_t *proofs128, const uint8_t *pairs64, size_t D, const uint8_t seed[32]);
 int rofl_debug_verify_weights(rofl_ctx *, const uint8_t *proofs, size_t proof_len, size_t n_proofs, const uint8_t *commits32, size_t D, int range, const uint8_t seed[32], uint8_t *out_weights);
 /* the MSM front end alone (production plan / forced window width / generator tables, then k_finalize): out32[k] = sum_t s[k][t] P_t + sB[k] B + sH[k] H.
  * scalars32: n_msm x T canonical scalars; points32: T shared or n_msm x T (points_per_msm) encodings, or NULL for BulletproofGens(gen_n, T / (2 gen_n));

@@ -68,7 +68,10 @@ _SIGS = {
     "rofl_ctx_stream": (c_vp, [c_vp]),
     "rofl_range_verify_batch": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, c_sz, c_sz, C.c_int, c_u8p, c_vp]),
     "rofl_enc_l2_compressed_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_sz, c_u8p, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, C.c_int, c_u8p, c_vp]),
+    "rofl_crp_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_u8p, c_sz, c_u8p, c_vp]),
+    "rofl_enc_range_compressed_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_sz, c_u8p, c_u8p, c_sz, c_sz, C.c_int, C.c_float, c_u8p, c_vp]),
     "rofl_debug_ts_absorb": (C.c_int, [c_vp, c_u8p, c_sz, C.c_int, C.c_int]),
+    "rofl_debug_crp_rlc": (C.c_int, [c_vp, c_sz, c_u8p, c_u8p, c_sz, c_u8p]),
     "rofl_debug_verify_weights": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, c_u8p, c_u8p]),
     "rofl_debug_msm": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_sz, c_u8p, c_u8p, c_u8p, c_vp]),
 }
@@ -282,11 +285,30 @@ class Api:
                                                           _ptr(_seed(seed)), _ptr(ok))
         if rc < 0: raise self._err(rc)
         return ok
+    def crp_verify_batch(self, proofs, pairs, seed=None):
+        """K compressed rand proofs [K, 128] over their pairs [K, D, 64] in one batched check -> int32[K], each exactly crp_verify's verdict"""
+        p = _u8(proofs); K = p.shape[0] if p.ndim > 1 else p.size // 128; p = p.reshape(K, 128); c = _u8(pairs).reshape(K, -1, 64)
+        ok = np.zeros(K, np.int32)
+        rc = self.lib.rofl_crp_verify_batch(self.h, K, _ptr(p), _ptr(c), c.shape[1], _ptr(_seed(seed)), _ptr(ok))
+        if rc < 0: raise self._err(rc)
+        return ok
+    def enc_range_compressed_verify_batch(self, msgs, check_percentage=1.0, seed=None):
+        """K EncRangeCompressed messages of one shape in one call -> int32[K], each exactly enc_range_compressed_verify's verdict"""
+        K = len(msgs); enc = _u8(np.stack([m["enc_values"] for m in msgs])).reshape(K, -1, 64); rp = _u8(np.stack([m["rand_proof"] for m in msgs])).reshape(K, 128)
+        p = _u8(np.stack([m["range_proof"] for m in msgs])); p = p.reshape(K, p.shape[1], -1)
+        ok = np.zeros(K, np.int32)
+        rc = self.lib.rofl_enc_range_compressed_verify_batch(self.h, K, _ptr(enc), enc.shape[1], _ptr(rp), _ptr(p), p.shape[2], p.shape[1], msgs[0]["range_bits"], check_percentage,
+                                                             _ptr(_seed(seed)), _ptr(ok))
+        if rc < 0: raise self._err(rc)
+        return ok
 
     # ---- test hooks
     def debug_ts_absorb(self, V32, n, label_id=0):
         v = _u8(V32).reshape(-1, 32)
         return self.lib.rofl_debug_ts_absorb(self.h, _ptr(v), v.shape[0], n, label_id)
+    def debug_crp_rlc(self, proofs, pairs, seed=None):
+        p = _u8(proofs).reshape(-1, 128); K = p.shape[0]; c = _u8(pairs).reshape(K, -1, 64)
+        return self.lib.rofl_debug_crp_rlc(self.h, K, _ptr(p), _ptr(c), c.shape[1], _ptr(_seed(seed)))
     def debug_verify_weights(self, proofs, commits, rng, seed):
         p = _u8(proofs); p = p.reshape(p.shape[0], -1); c = _u8(commits).reshape(-1, 32); w = np.zeros((2, p.shape[0], 32), np.uint8)
         rc = self.lib.rofl_debug_verify_weights(self.h, _ptr(p), p.shape[1], p.shape[0], _ptr(c), c.shape[0], rng, _ptr(_seed(seed)), _ptr(w))

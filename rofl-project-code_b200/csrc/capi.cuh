@@ -534,6 +534,37 @@ extern "C" int rofl_enc_l2_compressed_verify_batch(rofl_ctx *c, size_t n_clients
     return 0;
     API_CATCH
 }
+// K compressed rand proofs (compressed_rand_proof/mod.rs:149-158) in one batched check (engine.cuh, engine_crp_verify_batch).
+// out_ok[k] = exactly what rofl_crp_verify(proofs128[k], pairs64[k], D) returns.
+extern "C" int rofl_crp_verify_batch(rofl_ctx *c, size_t n_clients, const uint8_t *proofs128, const uint8_t *pairs64, size_t D, const uint8_t seed[32], int *out_ok) {
+    API_TRY return engine_crp_verify_batch(c->e, proofs128, pairs64, nullptr, D, n_clients, seed, out_ok); API_CATCH
+}
+// EncModelParams::verify, EncRangeCompressed arm (params.rs:236-256), for n_clients messages of one shape: the compressed rand proofs of all
+// clients in one batched check, the range proofs over the first round(D * check_percentage) L halves of every client in another
+// (engine_range_verify_batch).  The K rand-proof transcripts run on host threads while the range batch runs on this thread.
+// out_ok[k] = exactly what rofl_enc_range_compressed_verify(message k, ...) returns (1 / 0).
+extern "C" int rofl_enc_range_compressed_verify_batch(rofl_ctx *c, size_t n_clients, const uint8_t *enc_values64, size_t D, const uint8_t *rand_proofs128,
+                                                      const uint8_t *range_proofs, size_t plen, size_t n_proofs, int prove_range, float check_percentage,
+                                                      const uint8_t seed[32], int *out_ok) {
+    API_TRY
+    const size_t K = n_clients;
+    if (!D || !n_proofs || !out_ok) return ROFL_ERR_ARGS;
+    if (!K) return 0;
+    if (!enc_values64 || !rand_proofs128) return ROFL_ERR_ARGS;
+    const size_t num = (size_t)llroundf((float)D * check_percentage);                                                                   // :243-244
+    if (D > CRP_MAX_D || num == 0 || num > D) { for (size_t k = 0; k < K; k++) out_ok[k] = 0; return 0; }
+    lane_guard lg(c->e); cudaStream_t s = lg.s();
+    staged_in dp(enc_values64, 64 * D * K, s); dev_buf dL(32 * num * K, s);
+    LAUNCH(k_pairs_gather_L, dim3((unsigned)((num * K + 255) / 256)), dim3(256), s, dL.as<uint8_t>(), dp.b.as<uint8_t>(), D, num, K);
+    std::vector<int> ok_crp(K, 0), ok_range(K, 0);
+    crp_batch b(c->e, s, rand_proofs128, enc_values64, dp.b.as<uint8_t>(), D, K);
+    crp_batch_begin(b);
+    const int rc = engine_range_verify_batch(c->e, range_proofs, plen, n_proofs, dL.as<uint8_t>(), num, K, prove_range, seed, ok_range.data());
+    crp_batch_end(b, seed, ok_crp.data());
+    for (size_t k = 0; k < K; k++) out_ok[k] = (rc == 0 && ok_crp[k] == 1 && ok_range[k] == 1) ? 1 : 0;    // a bad range argument is a reject of every message, as there
+    return 0;
+    API_CATCH
+}
 
 // ---- test hooks (tests/test_emul_vs_oracle.py, tests/test_gpu_parity.py, tests/test_msm_kernels.py) -----------------------------------------------
 // the warp-cooperative V absorb (ts_kernels.cuh, k_ts_absorbV) against the sequential transcript code for the same m commitments: 0 equal, 1 different
@@ -559,6 +590,16 @@ extern "C" int rofl_debug_square_rlc(rofl_ctx *c, const uint8_t *proofs, const u
     lane_guard lg(c->e); cudaStream_t s = lg.s();
     staged_in dp(proofs, 160 * D, s), dc(commits, 64 * D, s);
     return square_verify_rlc(c->e, s, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D);
+    API_CATCH
+}
+// the batched compressed-rand-proof check alone (engine.cuh, engine_crp_verify_batch): 1 = the combination over all K proofs held and no proof is
+// malformed, 0 = it did not (the verdicts then came from the per-client checks), < 0 as rofl_crp_verify_batch.  Host buffers as there.
+extern "C" int rofl_debug_crp_rlc(rofl_ctx *c, size_t n_clients, const uint8_t *proofs128, const uint8_t *pairs64, size_t D, const uint8_t seed[32]) {
+    API_TRY
+    if (!n_clients || !D || D > CRP_MAX_D) return ROFL_ERR_ARGS;
+    std::vector<int> ok(n_clients); int holds = 0;
+    const int rc = engine_crp_verify_batch(c->e, proofs128, pairs64, nullptr, D, n_clients, seed, ok.data(), &holds);
+    return rc < 0 ? rc : holds;
     API_CATCH
 }
 // the batching scalars (c_i | rho_i, 2 x n_proofs x 32 bytes) the verifier derives for this call; return value as rofl_range_verify

@@ -23,7 +23,8 @@
 #include <cstdio>
 
 enum { ROFL_ERR_BITSIZE_ = -7 };          // include/rofl_b200.h ROFL_ERR_BITSIZE
-enum { DOM_RANGE_PROVE = 1, DOM_RANGE_VERIFY = 2, DOM_SQUARE = 3, DOM_L2_PROVE = 4, DOM_L2_VERIFY = 5, DOM_CRP = 6, DOM_RND_VEC = 7, DOM_RANDPROOF = 8, DOM_SQUARE_RAND = 9 };
+enum { DOM_RANGE_PROVE = 1, DOM_RANGE_VERIFY = 2, DOM_SQUARE = 3, DOM_L2_PROVE = 4, DOM_L2_VERIFY = 5, DOM_CRP = 6, DOM_RND_VEC = 7, DOM_RANDPROOF = 8, DOM_SQUARE_RAND = 9,
+       DOM_CRP_BATCH = 0x62707263 /* "crpb" as LE32: the weights of engine_crp_verify_batch */ };
 enum { PROF_FOLD = 0, PROF_MSM = 1, PROF_COMMIT = 2, PROF_SQUARE = 3, PROF_RTMSM = 4, PROF_TAIL = 5, PROF_FRZ = 6, PROF_SLOTS = 8 };
 
 struct gens_entry { int n = 0; int cap = 0; niels_st *G = nullptr, *H = nullptr;
@@ -1188,8 +1189,10 @@ static int engine_crp_prove(rofl_engine &e, const float *d_values, const uint8_t
     sc_tobytes(h_proof + 64, zm); sc_tobytes(h_proof + 96, zr);
     return 0;
 }
-// returns 1 valid, 0 invalid, -1 FormatError (from_bytes: mod.rs:118-134, el_gamal.rs:113-123), -6 too many pairs
-static int engine_crp_verify(rofl_engine &e, const uint8_t *h_proof, const uint8_t *h_pairs, size_t D) {
+// returns 1 valid, 0 invalid, -1 FormatError (from_bytes: mod.rs:118-134, el_gamal.rs:113-123), -6 too many pairs.
+// The check given the challenge: c_known = c when the caller already ran crp_challenge over these pairs (the batched verifier's per-client
+// re-check), else it is computed here while the device decompresses; d_pairs = the pairs already on the device (nullable: staged from h_pairs).
+static int engine_crp_verify(rofl_engine &e, const uint8_t *h_proof, const uint8_t *h_pairs, size_t D, const sc *c_known = nullptr, const uint8_t *d_pairs_in = nullptr) {
     if (D > CRP_MAX_D) return -6;
     sc zm, zr; sc_frombytes(zm, h_proof + 64); sc_frombytes(zr, h_proof + 96);
     if (!sc_is_canonical(zm) || !sc_is_canonical(zr)) return -1;
@@ -1201,11 +1204,11 @@ static int engine_crp_verify(rofl_engine &e, const uint8_t *h_proof, const uint8
     rt_h2d(d_cp32.p, h_proof, 64, s);
     LAUNCH(k_decompress, dim3(1), dim3(128), s, d_cp.as<p3_st>(), (uint8_t *)nullptr, d_cp32.as<uint8_t>(), (size_t)2, (size_t)2, (const p3_st *)nullptr, d_bad.as<int>(), (size_t)2);
     if (D) {
-        rt_h2d(d_pairs.p, h_pairs, 64 * D, s);
-        LAUNCH(k_pairs_split, dim3((unsigned)((D + 255) / 256)), dim3(256), s, d_LR32.as<uint8_t>(), d_LR32.as<uint8_t>() + 32 * D, d_pairs.as<uint8_t>(), D);
+        if (!d_pairs_in) rt_h2d(d_pairs.p, h_pairs, 64 * D, s);
+        LAUNCH(k_pairs_split, dim3((unsigned)((D + 255) / 256)), dim3(256), s, d_LR32.as<uint8_t>(), d_LR32.as<uint8_t>() + 32 * D, d_pairs_in ? d_pairs_in : d_pairs.as<uint8_t>(), D);
         LAUNCH(k_decompress, dim3((unsigned)((2 * D + 127) / 128)), dim3(128), s, d_LR.as<p3_st>(), (uint8_t *)nullptr, d_LR32.as<uint8_t>(), 2 * D, 2 * D, (const p3_st *)nullptr, d_bad.as<int>() + 1, 2 * D);
     }
-    sc c; crp_challenge(c, h_pairs, D, h_proof);                   // overlaps the decompression
+    sc c; if (c_known) c = *c_known; else crp_challenge(c, h_pairs, D, h_proof);                   // overlaps the decompression
     // sum_i c^(i+1) L_i and sum_i c^(i+1) R_i: two MSMs that share their scalars
     sc nzm, nzr, zero; sc_neg(nzm, zm); sc_neg(nzr, zr); sc_0(zero);
     sc_st h_s[4]; sc_to_st(h_s[0], nzm); sc_to_st(h_s[1], nzr); sc_to_st(h_s[2], nzr); sc_to_st(h_s[3], zero);      // sB = [-z_m, -z_r], sH = [-z_r, 0]
@@ -1232,6 +1235,134 @@ static int engine_crp_verify(rofl_engine &e, const uint8_t *h_proof, const uint8
     int id[2], bad[2]; rt_d2h(id, d_id.p, sizeof(id), s); rt_d2h(bad, d_bad.p, sizeof(bad), s); rt_sync(s);
     if (bad[0]) return -1;
     return (id[0] && id[1]) ? 1 : 0;
+}
+
+// Server side: the compressed rand proofs of K clients in ONE check.  Client k's proof holds iff
+//   C'_L,k + sum_i c_k^(i+1) L_k,i - z_m,k B - z_r,k H = 0   and   C'_R,k + sum_i c_k^(i+1) R_k,i - z_r,k B = 0;
+// with Fiat-Shamir weights rho_k both are summed over the clients and checked by one MSM with two outputs that share their scalars
+// (v[0] over L | C'_L, v[1] over R | C'_R; T = K (D + 1) terms) and one k_finalize whose fixed-base coefficients carry the signs:
+//   sB = [-sum rho_k z_m,k, -sum rho_k z_r,k],  sH = [-sum rho_k z_r,k, 0].
+// The weights: digest_k = SHA3-256(c_k | z_m,k | z_r,k) (c_k binds client k's pairs and C'), root = SHA3-256(seed | "crpb" | LE64 K | LE64 D |
+// digest_0 .. digest_(K-1)), rho_k = the low 128 bits of ChaCha20(SHA3-256(root | LE64 k)) (the next block while they are zero).
+// The K transcripts (crp_challenge: one sequential Merlin transcript over all D pairs per client) run on host threads from begin() to end(),
+// while the device decompresses and the caller may queue more work on its stream (the whole-message batch runs its range batch there).
+// Those threads do host work only: they never take a lane.  Clients are processed in groups of at most CRP_BATCH_TERMS terms.
+// Verdicts: the combined check holds and no client of the group is malformed -> 1; otherwise malformed clients get -1 and every other client
+// is re-checked on its own with the challenge already computed (engine_crp_verify given c), so each verdict is exactly rofl_crp_verify's.
+#define CRP_BATCH_TERMS ((size_t)1 << 24)
+struct crp_batch {
+    rofl_engine &e; cudaStream_t s;
+    const uint8_t *h_proofs, *h_pairs, *d_pairs; size_t D, K, G;
+    std::vector<sc> c; std::vector<uint8_t> fmt;                                   // fmt[k]: z_m or z_r not canonical
+    dev_buf d_cp, d_P, d_bad;
+    std::thread th; std::string err;
+    crp_batch(rofl_engine &eng, cudaStream_t st, const uint8_t *hp, const uint8_t *hpairs, const uint8_t *dpairs, size_t D_, size_t K_)
+        : e(eng), s(st), h_proofs(hp), h_pairs(hpairs), d_pairs(dpairs), D(D_), K(K_), G(std::max<size_t>(1, std::min(K_, CRP_BATCH_TERMS / (D_ + 1)))),
+          c(K_), fmt(K_, 0), d_cp(64 * K_, st), d_P(sizeof(p3_st) * 2 * (G * (D_ + 1)), st), d_bad(sizeof(int) * K_, st) {}
+    ~crp_batch() { if (th.joinable()) th.join(); }
+    crp_batch(const crp_batch &) = delete; crp_batch &operator=(const crp_batch &) = delete;
+    void decompress(size_t k0, size_t g) {
+        const size_t n = 2 * g * (D + 1);
+        LAUNCH(k_crp_batch_points, dim3((unsigned)((n + 127) / 128)), dim3(128), s, d_P.as<p3_st>(), d_pairs + 64 * D * k0, d_cp.as<uint8_t>() + 64 * k0, D, (uint32_t)g, d_bad.as<int>() + k0);
+    }
+};
+// D >= 1, D <= CRP_MAX_D, K >= 1; the caller holds a lane (s is its stream) and has put the K x D pairs at d_pairs
+static void crp_batch_begin(crp_batch &b) {
+    std::vector<uint8_t> cp(64 * b.K);
+    for (size_t k = 0; k < b.K; k++) {
+        const uint8_t *p = b.h_proofs + 128 * k; memcpy(&cp[64 * k], p, 64);
+        sc zm, zr; sc_frombytes(zm, p + 64); sc_frombytes(zr, p + 96);
+        b.fmt[k] = !sc_is_canonical(zm) || !sc_is_canonical(zr);
+    }
+    rt_h2d(b.d_cp.p, cp.data(), cp.size(), b.s); rt_memset(b.d_bad.p, 0, sizeof(int) * b.K, b.s);
+    b.decompress(0, std::min(b.G, b.K));
+    b.th = std::thread([&b] {
+        try { parallel_for(b.K, b.e.host_threads, [&b](size_t k) { crp_challenge(b.c[k], b.h_pairs + 64 * b.D * k, b.D, b.h_proofs + 128 * k); }); }
+        catch (const std::exception &ex) { b.err = ex.what(); }
+    });
+}
+// holds (nullable): 1 when the combined check of every group held, else 0
+static void crp_batch_end(crp_batch &b, const uint8_t seed[32], int *out, int *holds = nullptr) {
+    rofl_engine &e = b.e; cudaStream_t s = b.s; const size_t K = b.K, D = b.D;
+    b.th.join();
+    if (!b.err.empty()) throw std::runtime_error(b.err);
+    std::vector<uint8_t> root_in(32 + 4 + 16 + 32 * K);
+    memcpy(root_in.data(), seed, 32);
+    for (int i = 0; i < 4; i++) root_in[32 + i] = (uint8_t)((uint32_t)DOM_CRP_BATCH >> (8 * i));
+    for (int i = 0; i < 8; i++) { root_in[36 + i] = (uint8_t)((uint64_t)K >> (8 * i)); root_in[44 + i] = (uint8_t)((uint64_t)D >> (8 * i)); }
+    for (size_t k = 0; k < K; k++) {
+        uint8_t m[96]; sc_tobytes(m, b.c[k]); memcpy(m + 32, b.h_proofs + 128 * k + 64, 64);
+        sha3_256(&root_in[52 + 32 * k], m, 96);
+    }
+    uint8_t root[32]; sha3_256(root, root_in.data(), root_in.size());
+    std::vector<sc> rho(K);
+    for (size_t k = 0; k < K; k++) {
+        uint8_t kb[40], key[32]; memcpy(kb, root, 32);
+        for (int i = 0; i < 8; i++) kb[32 + i] = (uint8_t)((uint64_t)k >> (8 * i));
+        sha3_256(key, kb, 40); uint32_t kw[8]; key_words(kw, key);
+        for (uint64_t ctr = 0;; ctr++) {
+            uint32_t w[16]; chacha20_block_words(w, kw, ctr);
+            sc_0(rho[k]); for (int i = 0; i < 4; i++) rho[k].v[i] = w[i];
+            if (w[0] | w[1] | w[2] | w[3]) break;
+        }
+    }
+    const int bits = std::max(2, ilog2_sz(D + 2));
+    pow_tab ct = {nullptr, bits / 2, bits - bits / 2};
+    const size_t tabn = pow_tab_size(ct);
+    std::vector<int> bad(K, 0);
+    if (holds) *holds = 1;
+    for (size_t k0 = 0; k0 < K; k0 += b.G) {
+        const size_t g = std::min(b.G, K - k0), n = g * (D + 1);
+        bool any_fmt = false; for (size_t k = k0; k < k0 + g; k++) any_fmt = any_fmt || b.fmt[k];
+        int id[2] = {0, 0};
+        if (!any_fmt) {
+            if (k0) b.decompress(k0, g);
+            std::vector<sc_st> h_pow2(32 * g), h_rho(g); sc sB0, sB1, t; sc_0(sB0); sc_0(sB1);
+            for (size_t j = 0; j < g; j++) {
+                const size_t k = k0 + j; sc zm, zr; sc_frombytes(zm, b.h_proofs + 128 * k + 64); sc_frombytes(zr, b.h_proofs + 128 * k + 96);
+                sc_pow2_table(&h_pow2[32 * j], b.c[k]); sc_to_st(h_rho[j], rho[k]);
+                sc_mul(t, rho[k], zm); sc_add(sB0, sB0, t); sc_mul(t, rho[k], zr); sc_add(sB1, sB1, t);
+            }
+            sc_neg(sB0, sB0); sc_neg(sB1, sB1); sc zero; sc_0(zero);
+            sc_st h_s[4]; sc_to_st(h_s[0], sB0); sc_to_st(h_s[1], sB1); sc_to_st(h_s[2], sB1); sc_to_st(h_s[3], zero);       // sB = [-sum rho z_m, -sum rho z_r], sH = [-sum rho z_r, 0]
+            dev_buf d_pow2(sizeof(sc_st) * 32 * g, s), d_tab(sizeof(sc_st) * tabn * g, s), d_rho(sizeof(sc_st) * g, s), d_sc(sizeof(sc_st) * n, s), d_s(sizeof(h_s), s), d_id(sizeof(int) * 2, s);
+            rt_h2d(d_pow2.p, h_pow2.data(), sizeof(sc_st) * h_pow2.size(), s); rt_h2d(d_rho.p, h_rho.data(), sizeof(sc_st) * g, s); rt_h2d(d_s.p, h_s, sizeof(h_s), s);
+            LAUNCH(k_pow_tables, dim3((unsigned)((tabn + 255) / 256), (unsigned)g), dim3(256), s, d_tab.as<sc_st>(), d_pow2.as<sc_st>(), ct.L, ct.H);
+            ct.tab = d_tab.as<sc_st>();
+            LAUNCH(k_crp_batch_scalars, dim3((unsigned)((n + 255) / 256)), dim3(256), s, d_sc.as<sc_st>(), D, (uint32_t)g, ct, d_rho.as<sc_st>());
+            const msm_plan pl = msm_plan_for(n, 2);
+            dev_buf d_win(sizeof(p3_st) * pl.out_count(2), s);
+            msm_args a = {}; a.v[0].scalars = d_sc.as<sc_st>(); a.v[1].scalars = d_sc.as<sc_st>(); a.split = 1; a.T = (uint32_t)n; a.scalar_stride = 0; a.nseg = 1; a.out = d_win.as<p3_st>();
+            a.v[0].seg[0] = mk_seg(b.d_P.as<p3_st>(), (uint32_t)n, 0, 1); a.v[1].seg[0] = mk_seg(b.d_P.as<p3_st>() + n, (uint32_t)n, 0, 1);
+            run_msm(e, s, a, pl, 2);
+            finalize_args f = {}; fin_windows(f, d_win.as<p3_st>(), pl); f.sBa = d_s.as<sc_st>(); f.sHa = d_s.as<sc_st>() + 2; f.tabB = e.sh->tabB; f.tabH = e.sh->tabH;
+            f.is_id = d_id.as<int>(); f.count = 2;
+            run_finalize(s, f);
+            rt_d2h(id, d_id.p, sizeof(id), s); rt_d2h(&bad[k0], b.d_bad.as<int>() + k0, sizeof(int) * g, s); rt_sync(s);
+            bool all = id[0] && id[1]; for (size_t k = k0; k < k0 + g; k++) all = all && !bad[k];
+            if (all) { for (size_t k = k0; k < k0 + g; k++) out[k] = 1; continue; }
+        }
+        if (holds) *holds = 0;
+        for (size_t k = k0; k < k0 + g; k++)
+            out[k] = b.fmt[k] ? -1 : engine_crp_verify(e, b.h_proofs + 128 * k, b.h_pairs + 64 * D * k, D, &b.c[k], b.d_pairs + 64 * D * k);
+    }
+}
+// K compressed rand proofs (h_proofs K x 128, h_pairs K x D x 64 host; d_pairs the same pairs on the device, nullable) in one batched check;
+// out[k] = exactly engine_crp_verify(proof k, pairs k, D).  Returns 0, -2 for bad arguments.  holds: as crp_batch_end (left alone when no check runs)
+static int engine_crp_verify_batch(rofl_engine &e, const uint8_t *h_proofs, const uint8_t *h_pairs, const uint8_t *d_pairs, size_t D, size_t K, const uint8_t seed[32], int *out,
+                                   int *holds = nullptr) {
+    if (!out) return -2;
+    if (K == 0) return 0;
+    if (!h_proofs || (D && !h_pairs)) return -2;
+    if (D > CRP_MAX_D) { for (size_t k = 0; k < K; k++) out[k] = -6; return 0; }
+    if (D == 0) { for (size_t k = 0; k < K; k++) out[k] = engine_crp_verify(e, h_proofs + 128 * k, h_pairs, 0); return 0; }
+    lane_guard lg(e); cudaStream_t s = lg.s();
+    dev_buf d_own(d_pairs ? 16 : 64 * D * K, s);
+    if (!d_pairs) rt_h2d(d_own.p, h_pairs, 64 * D * K, s);
+    crp_batch b(e, s, h_proofs, h_pairs, d_pairs ? d_pairs : d_own.as<uint8_t>(), D, K);
+    crp_batch_begin(b);
+    crp_batch_end(b, seed, out, holds);
+    return 0;
 }
 
 // rand_proof_vec::{create_randproof_vec(_existing), verify_randproof_vec} (kind 1) and square_rand_proof_vec::{create_l2rangeproof_vec(_existing),

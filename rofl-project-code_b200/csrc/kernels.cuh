@@ -1246,6 +1246,41 @@ KERNEL void LB(256, 2) k_pairs_split(uint8_t *L, uint8_t *R, const uint8_t *pair
     uint8_t b[32]; ld_bytes32(b, pairs + 64 * i); st_bytes32(L + 32 * i, b); ld_bytes32(b, pairs + 64 * i + 32); st_bytes32(R + 32 * i, b);
 }
 KLAUNCH(k_pairs_split, false, (uint8_t *L, uint8_t *R, const uint8_t *pairs, size_t D), (L, R, pairs, D))
+// L halves of the first `num` of the D pairs of each of K updates -> out[K x num x 32] (the Pedersen commitments a prefix range check is about)
+KERNEL void LB(256, 2) k_pairs_gather_L(uint8_t *out, const uint8_t *pairs, size_t D, size_t num, size_t K) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= K * num) return;
+    const size_t k = i / num, j = i % num;
+    uint8_t b[32]; ld_bytes32(b, pairs + 64 * (k * D + j)); st_bytes32(out + 32 * i, b);
+}
+KLAUNCH(k_pairs_gather_L, false, (uint8_t *out, const uint8_t *pairs, size_t D, size_t num, size_t K), (out, pairs, D, num, K))
+// Batched check of G compressed rand proofs (engine.cuh, engine_crp_verify_batch).  Points: n = G D + G terms per side,
+//   P[0, n)  = L of every client (client-major) | C'_L of every client,   P[n, 2n) = R ... | C'_R ...
+// from pairs[G x D x 64] and cp[G x 64] (C'_L | C'_R); an undecodable encoding sets bad[client] and contributes the identity.
+KERNEL void LB(128, 2) k_crp_batch_points(p3_st *P, const uint8_t *pairs, const uint8_t *cp, size_t D, uint32_t G, int *bad) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, GD = (size_t)G * D, n = GD + G;
+    if (i >= 2 * n) return;
+    const size_t which = i >= n ? 1 : 0, j = i - which * n;
+    const bool pair = j < GD;
+    const uint8_t *src = pair ? pairs + 64 * j + 32 * which : cp + 64 * (j - GD) + 32 * which;
+    uint8_t b[32]; ld_bytes32(b, src);
+    ge_p3 p; if (!ge_decompress(p, b)) { atomicOr(bad + (pair ? j / D : j - GD), 1); ge_p3_0(p); }
+    st_p3(P + i, p);
+}
+KLAUNCH(k_crp_batch_points, false, (p3_st *P, const uint8_t *pairs, const uint8_t *cp, size_t D, uint32_t G, int *bad), (P, pairs, cp, D, G, bad))
+// the MSM scalars of that check: s[k D + i] = rho_k c_k^(i+1) (the split power table of c_k is table k of ctab), s[G D + k] = rho_k.
+// Nothing is negated here: the signs live in the fixed-base coefficients of k_finalize (negated short weights would share one bucket).
+KERNEL void LB(256, 2) k_crp_batch_scalars(sc_st *s, size_t D, uint32_t G, pow_tab ctab, const sc_st *rho) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, GD = (size_t)G * D;
+    if (i >= GD + G) return;
+    sc r;
+    if (i < GD) {
+        const size_t k = i / D;
+        sc pw, w; pow_tab_get(pw, ctab, (int)k, i - k * D + 1); ld_sc(w, rho + k); sc_mul(r, pw, w);
+    } else ld_sc(r, rho + (i - GD));
+    st_sc(s + i, r);
+}
+KLAUNCH(k_crp_batch_scalars, false, (sc_st *s, size_t D, uint32_t G, pow_tab ctab, const sc_st *rho), (s, D, G, ctab, rho))
 #endif
 
 // ===================================================================================================================
@@ -1347,6 +1382,9 @@ void launch_k_crp_sums(dim3 g_, dim3 b_, cudaStream_t s_, sc_st *partial, const 
 void launch_k_crp_pows(dim3 g_, dim3 b_, cudaStream_t s_, sc_st *out, size_t D, pow_tab ctab);
 void launch_k_pairs_join(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *pairs, const uint8_t *L, const uint8_t *R, size_t D);
 void launch_k_pairs_split(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *L, uint8_t *R, const uint8_t *pairs, size_t D);
+void launch_k_pairs_gather_L(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const uint8_t *pairs, size_t D, size_t num, size_t K);
+void launch_k_crp_batch_points(dim3 g_, dim3 b_, cudaStream_t s_, p3_st *P, const uint8_t *pairs, const uint8_t *cp, size_t D, uint32_t G, int *bad);
+void launch_k_crp_batch_scalars(dim3 g_, dim3 b_, cudaStream_t s_, sc_st *s, size_t D, uint32_t G, pow_tab ctab, const sc_st *rho);
 
 // ===================================================================================================================
 // RT path: per-generator radix-256 tables in HBM (512 KB per generator: 32 windows x 128 affine-Niels multiples).
