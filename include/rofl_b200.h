@@ -62,7 +62,8 @@ void rofl_set_host_threads(rofl_ctx *ctx, int n);          /* host threads used 
  * groups on separate queues, "tail_np" largest half-size handled by the fused tail kernel (0 = off), "rt_bits" table radix, "rt_per" table-MSM
  * terms per thread, "tail_ncta" thread blocks (one cluster) per chunk in the tail kernel (1, 2, 4, 8), "frozen" 0/1 frozen-level middle rounds,
  * "nt_unfold" / "nt_unfold_min" unfolded rounds without tables, "ts_host_m" chunk size above which commitments are absorbed on the host,
- * "max_lanes" concurrent callers, "drop_tables", "trim" (hand cached scratch back to CUDA).
+ * "max_lanes" concurrent callers, "drop_tables", "trim" (hand cached scratch back to CUDA), "sigma_rlc_terms" MSM terms per range of the
+ * batched rand / square-rand proof check (1 .. 2^24, the default).
  * returns 0, -2 unknown name */
 int rofl_set_option(rofl_ctx *ctx, const char *name, long value);
 
@@ -199,6 +200,23 @@ int rofl_crp_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *proofs128
  * check_percentage, seed) returns (1 / 0).  Return value: 0, or ROFL_ERR_ARGS (D == 0, n_proofs == 0, null out_ok). */
 int rofl_enc_range_compressed_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *enc_values64, size_t D, const uint8_t *rand_proofs128, const uint8_t *range_proofs,
                                            size_t proof_len, size_t n_proofs, int prove_range, float check_percentage, const uint8_t seed[32], int *out_ok);
+/* K x D rand proofs (rand_proof_vec::verify_randproof_vec) / square-rand proofs (square_rand_proof_vec::verify_l2rangeproof_vec) in one batched
+ * check.  proofs128 / proofs192: n_clients x D x 128 | 192, pairs64 / commits96: n_clients x D x 64 | 96.  out_ok[k] = exactly what
+ * rofl_rand_verify / rofl_square_rand_verify(proofs k, commits k, D) returns: 1, 0, ROFL_ERR_FORMAT (D == 0: 1 for every client).
+ * Return value: 0, or ROFL_ERR_ARGS (null out_ok, null buffers). */
+int rofl_rand_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *proofs128, const uint8_t *pairs64, size_t D, const uint8_t seed[32], int *out_ok);
+int rofl_square_rand_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *proofs192, const uint8_t *commits96, size_t D, const uint8_t seed[32], int *out_ok);
+/* EncModelParams::verify, EncRange arm (params.rs:186-203), for n_clients messages of one shape: enc_values64 n_clients x D x 64,
+ * rand_proofs128 n_clients x D x 128, range_proofs n_clients x n_proofs x proof_len.  out_ok[k] = exactly what rofl_enc_range_verify(message k,
+ * check_percentage, seed) returns (1 / 0).  Return value: 0, or ROFL_ERR_ARGS (D == 0, n_proofs == 0, null out_ok). */
+int rofl_enc_range_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *enc_values64, size_t D, const uint8_t *rand_proofs128, const uint8_t *range_proofs,
+                                size_t proof_len, size_t n_proofs, int prove_range, float check_percentage, const uint8_t seed[32], int *out_ok);
+/* EncModelParams::verify, EncL2 arm (params.rs:205-233), for n_clients messages of one shape: enc_values96 n_clients x D x 96, square_proofs192
+ * n_clients x D x 192, range_proofs n_clients x n_proofs x proof_len, square_range_proofs n_clients x sq_proof_len.  out_ok[k] = exactly what
+ * rofl_enc_l2_verify(message k, ..., seed) returns (1 / 0).  Return value: 0, or ROFL_ERR_ARGS (D == 0, n_proofs == 0, null out_ok). */
+int rofl_enc_l2_verify_batch(rofl_ctx *, size_t n_clients, const uint8_t *enc_values96, size_t D, const uint8_t *square_proofs192, const uint8_t *range_proofs,
+                             size_t proof_len, size_t n_proofs, const uint8_t *square_range_proofs, size_t sq_proof_len, int prove_range, int l2_range,
+                             const uint8_t seed[32], int *out_ok);
 
 /* ---- aggregation: EncModelParamsAccumulator::accumulate_other (params.rs:81-124) / pedersen_ops::add_rp_vec_vec
  *      (pedersen_ops.rs:56-69; bindings32.rs:64 `add_commitments`).  points32: n_clients x D encodings, client-major.
@@ -227,6 +245,9 @@ int rofl_debug_ts_absorb(rofl_ctx *, const uint8_t *V32, size_t m, int n, int la
 int rofl_debug_square_rlc(rofl_ctx *, const uint8_t *proofs160, const uint8_t *commits64, size_t D);   /* the batched square-proof check alone: 1 holds, 0 does not */
 /* the batched compressed-rand-proof check of rofl_crp_verify_batch alone: 1 = the combination over all n_clients proofs held and none is malformed, 0 = it did not */
 int rofl_debug_crp_rlc(rofl_ctx *, size_t n_clients, const uint8_t *proofs128, const uint8_t *pairs64, size_t D, const uint8_t seed[32]);
+/* the batched check of rofl_rand_verify_batch (kind 1) / rofl_square_rand_verify_batch (kind 2) alone, over n_elems elements of one update and at any
+ * size: 1 = the combination over all elements held and none is malformed, 0 = it did not */
+int rofl_debug_sigma_rlc(rofl_ctx *, int kind, size_t n_elems, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32]);
 int rofl_debug_verify_weights(rofl_ctx *, const uint8_t *proofs, size_t proof_len, size_t n_proofs, const uint8_t *commits32, size_t D, int range, const uint8_t seed[32], uint8_t *out_weights);
 /* the MSM front end alone (production plan / forced window width / generator tables, then k_finalize): out32[k] = sum_t s[k][t] P_t + sB[k] B + sH[k] H.
  * scalars32: n_msm x T canonical scalars; points32: T shared or n_msm x T (points_per_msm) encodings, or NULL for BulletproofGens(gen_n, T / (2 gen_n));

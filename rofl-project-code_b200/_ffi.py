@@ -72,6 +72,11 @@ _SIGS = {
     "rofl_enc_range_compressed_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_sz, c_u8p, c_u8p, c_sz, c_sz, C.c_int, C.c_float, c_u8p, c_vp]),
     "rofl_debug_ts_absorb": (C.c_int, [c_vp, c_u8p, c_sz, C.c_int, C.c_int]),
     "rofl_debug_crp_rlc": (C.c_int, [c_vp, c_sz, c_u8p, c_u8p, c_sz, c_u8p]),
+    "rofl_rand_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_u8p, c_sz, c_u8p, c_vp]),
+    "rofl_square_rand_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_u8p, c_sz, c_u8p, c_vp]),
+    "rofl_enc_range_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_sz, c_u8p, c_u8p, c_sz, c_sz, C.c_int, C.c_float, c_u8p, c_vp]),
+    "rofl_enc_l2_verify_batch": (C.c_int, [c_vp, c_sz, c_u8p, c_sz, c_u8p, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, C.c_int, c_u8p, c_vp]),
+    "rofl_debug_sigma_rlc": (C.c_int, [c_vp, C.c_int, c_sz, c_u8p, c_u8p, c_u8p]),
     "rofl_debug_verify_weights": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, c_u8p, c_u8p]),
     "rofl_debug_msm": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_sz, c_u8p, c_u8p, c_u8p, c_vp]),
 }
@@ -301,6 +306,38 @@ class Api:
                                                              _ptr(_seed(seed)), _ptr(ok))
         if rc < 0: raise self._err(rc)
         return ok
+    def rand_verify_batch(self, proofs, pairs, seed=None):
+        """K x D rand proofs [K, D, 128] over their pairs [K, D, 64] in one batched check -> int32[K], each exactly rand_verify's verdict"""
+        c = _u8(pairs); K = c.shape[0]; c = c.reshape(K, -1, 64); p = _u8(proofs).reshape(K, c.shape[1], 128)
+        ok = np.zeros(K, np.int32)
+        rc = self.lib.rofl_rand_verify_batch(self.h, K, _ptr(p), _ptr(c), c.shape[1], _ptr(_seed(seed)), _ptr(ok))
+        if rc < 0: raise self._err(rc)
+        return ok
+    def square_rand_verify_batch(self, proofs, commits, seed=None):
+        """K x D square-rand proofs [K, D, 192] over their commitments [K, D, 96] in one batched check -> int32[K], each exactly square_rand_verify's verdict"""
+        c = _u8(commits); K = c.shape[0]; c = c.reshape(K, -1, 96); p = _u8(proofs).reshape(K, c.shape[1], 192)
+        ok = np.zeros(K, np.int32)
+        rc = self.lib.rofl_square_rand_verify_batch(self.h, K, _ptr(p), _ptr(c), c.shape[1], _ptr(_seed(seed)), _ptr(ok))
+        if rc < 0: raise self._err(rc)
+        return ok
+    def enc_range_verify_batch(self, msgs, check_percentage=1.0, seed=None):
+        """K EncRange messages of one shape in one call -> int32[K], each exactly enc_range_verify's verdict"""
+        K = len(msgs); enc = _u8(np.stack([m["enc_values"] for m in msgs])).reshape(K, -1, 64); rp = _u8(np.stack([m["rand_proof"] for m in msgs])).reshape(K, -1, 128)
+        p = _u8(np.stack([m["range_proof"] for m in msgs])); p = p.reshape(K, p.shape[1], -1)
+        ok = np.zeros(K, np.int32)
+        rc = self.lib.rofl_enc_range_verify_batch(self.h, K, _ptr(enc), enc.shape[1], _ptr(rp), _ptr(p), p.shape[2], p.shape[1], msgs[0]["range_bits"], check_percentage,
+                                                  _ptr(_seed(seed)), _ptr(ok))
+        if rc < 0: raise self._err(rc)
+        return ok
+    def enc_l2_verify_batch(self, msgs, seed=None):
+        """K EncL2 messages of one shape in one call -> int32[K], each exactly enc_l2_verify's verdict"""
+        K = len(msgs); enc = _u8(np.stack([m["enc_values"] for m in msgs])).reshape(K, -1, 96); sp = _u8(np.stack([m["square_proof"] for m in msgs])).reshape(K, -1, 192)
+        rp = _u8(np.stack([m["range_proof"] for m in msgs])); rp = rp.reshape(K, rp.shape[1], -1); sq = _u8(np.stack([m["square_range_proof"] for m in msgs])).reshape(K, -1)
+        ok = np.zeros(K, np.int32)
+        rc = self.lib.rofl_enc_l2_verify_batch(self.h, K, _ptr(enc), enc.shape[1], _ptr(sp), _ptr(rp), rp.shape[2], rp.shape[1], _ptr(sq), sq.shape[1], msgs[0]["range_bits"],
+                                               msgs[0]["l2_range_bits"], _ptr(_seed(seed)), _ptr(ok))
+        if rc < 0: raise self._err(rc)
+        return ok
 
     # ---- test hooks
     def debug_ts_absorb(self, V32, n, label_id=0):
@@ -309,6 +346,11 @@ class Api:
     def debug_crp_rlc(self, proofs, pairs, seed=None):
         p = _u8(proofs).reshape(-1, 128); K = p.shape[0]; c = _u8(pairs).reshape(K, -1, 64)
         return self.lib.rofl_debug_crp_rlc(self.h, K, _ptr(p), _ptr(c), c.shape[1], _ptr(_seed(seed)))
+    def debug_sigma_rlc(self, kind, proofs, commits, seed=None):
+        """the batched rand (kind 1) / square-rand (kind 2) proof check alone over all elements as one update: 1 held, 0 did not"""
+        pw, cw = (128, 64) if kind == 1 else (192, 96)
+        p = _u8(proofs).reshape(-1, pw); c = _u8(commits).reshape(-1, cw)
+        return self.lib.rofl_debug_sigma_rlc(self.h, kind, p.shape[0], _ptr(p), _ptr(c), _ptr(_seed(seed)))
     def debug_verify_weights(self, proofs, commits, rng, seed):
         p = _u8(proofs); p = p.reshape(p.shape[0], -1); c = _u8(commits).reshape(-1, 32); w = np.zeros((2, p.shape[0], 32), np.uint8)
         rc = self.lib.rofl_debug_verify_weights(self.h, _ptr(p), p.shape[1], p.shape[0], _ptr(c), c.shape[0], rng, _ptr(_seed(seed)), _ptr(w))

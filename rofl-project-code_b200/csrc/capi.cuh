@@ -31,6 +31,7 @@ extern "C" int rofl_set_option(rofl_ctx *c, const char *name, long value) {
     else if (n == "nt_unfold_min") c->e.nt_unfold_min = (int)std::max<long>(2, std::min<long>(1 << 30, value));
     else if (n == "ts_host_m") c->e.ts_host_m = (int)std::max<long>(0, std::min<long>(1 << 30, value));
     else if (n == "max_lanes") c->e.max_lanes = (int)std::max<long>(1, std::min<long>(64, value));
+    else if (n == "sigma_rlc_terms") c->e.sigma_rlc_terms = (size_t)std::max<long>(1, std::min<long>(1L << 24, value));
     else return ROFL_ERR_ARGS;
     return ROFL_OK;
 }
@@ -566,6 +567,91 @@ extern "C" int rofl_enc_range_compressed_verify_batch(rofl_ctx *c, size_t n_clie
     API_CATCH
 }
 
+// K x D rand proofs (rand_proof_vec::verify_randproof_vec, kind 1) or square-rand proofs (square_rand_proof_vec::verify_l2rangeproof_vec, kind 2)
+// in one batched check (engine.cuh, sigma_verify_groups).  out[k] = exactly what sigma_verify_host(kind, proofs k, commits k, D) returns: 1 / 0 / -1.
+static int sigma_verify_batch_host(rofl_ctx *c, int kind, size_t K, const uint8_t *proofs, const uint8_t *commits, size_t D, const uint8_t seed[32], int *out) {
+    if (!out) return ROFL_ERR_ARGS;
+    if (!K) return 0;
+    if (!D) { for (size_t k = 0; k < K; k++) out[k] = 1; return 0; }
+    if (!proofs || !commits || !seed) return ROFL_ERR_ARGS;
+    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    lane_guard lg(c->e); cudaStream_t s = lg.s();
+    staged_in dp(proofs, pw * D * K, s), dc(commits, cw * D * K, s); dev_buf dres(2 * sizeof(int) * K, s);
+    std::vector<int> res(2 * K);
+    for (size_t k = 0; k < K; k++) { res[2 * k] = 1; res[2 * k + 1] = 0; }
+    rt_h2d(dres.p, res.data(), sizeof(int) * 2 * K, s);
+    sigma_verify_groups(c->e, s, kind, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D * K, seed, D, dres.as<int>());
+    rt_d2h(res.data(), dres.p, sizeof(int) * 2 * K, s); rt_sync(s);
+    for (size_t k = 0; k < K; k++) out[k] = res[2 * k + 1] ? -1 : res[2 * k] ? 1 : 0;
+    return 0;
+}
+extern "C" int rofl_rand_verify_batch(rofl_ctx *c, size_t n_clients, const uint8_t *proofs128, const uint8_t *pairs64, size_t D, const uint8_t seed[32], int *out_ok) {
+    API_TRY return sigma_verify_batch_host(c, 1, n_clients, proofs128, pairs64, D, seed, out_ok); API_CATCH
+}
+extern "C" int rofl_square_rand_verify_batch(rofl_ctx *c, size_t n_clients, const uint8_t *proofs192, const uint8_t *commits96, size_t D, const uint8_t seed[32], int *out_ok) {
+    API_TRY return sigma_verify_batch_host(c, 2, n_clients, proofs192, commits96, D, seed, out_ok); API_CATCH
+}
+// EncModelParams::verify, EncRange arm (params.rs:186-203), for n_clients messages of one shape: the K x D rand proofs in one batched check, the
+// range proofs over the first round(D * check_percentage) L halves of every client in another (engine_range_verify_batch).
+// out_ok[k] = exactly what rofl_enc_range_verify(message k, ...) returns (1 / 0).
+extern "C" int rofl_enc_range_verify_batch(rofl_ctx *c, size_t n_clients, const uint8_t *enc_values64, size_t D, const uint8_t *rand_proofs128, const uint8_t *range_proofs,
+                                           size_t plen, size_t n_proofs, int prove_range, float check_percentage, const uint8_t seed[32], int *out_ok) {
+    API_TRY
+    const size_t K = n_clients;
+    if (!D || !n_proofs || !out_ok) return ROFL_ERR_ARGS;
+    if (!K) return 0;
+    if (!enc_values64 || !rand_proofs128 || !seed) return ROFL_ERR_ARGS;
+    const size_t num = (size_t)llroundf((float)D * check_percentage);
+    if (num == 0 || num > D) { for (size_t k = 0; k < K; k++) out_ok[k] = 0; return 0; }
+    lane_guard lg(c->e); cudaStream_t s = lg.s();
+    staged_in dpf(rand_proofs128, 128 * D * K, s), dp(enc_values64, 64 * D * K, s); dev_buf dres(2 * sizeof(int) * K, s), dL(32 * num * K, s);
+    std::vector<int> res(2 * K), ok_range(K, 0);
+    for (size_t k = 0; k < K; k++) { res[2 * k] = 1; res[2 * k + 1] = 0; }
+    rt_h2d(dres.p, res.data(), sizeof(int) * 2 * K, s);
+    sigma_verify_groups(c->e, s, 1, dpf.b.as<uint8_t>(), dp.b.as<uint8_t>(), D * K, seed, D, dres.as<int>());
+    LAUNCH(k_pairs_gather_L, dim3((unsigned)((num * K + 255) / 256)), dim3(256), s, dL.as<uint8_t>(), dp.b.as<uint8_t>(), D, num, K);
+    rt_d2h(res.data(), dres.p, sizeof(int) * 2 * K, s); rt_sync(s);
+    const int rc = engine_range_verify_batch(c->e, range_proofs, plen, n_proofs, dL.as<uint8_t>(), num, K, prove_range, seed, ok_range.data());
+    for (size_t k = 0; k < K; k++)                         // a rand-proof format error and a bad range argument are rejects, as there
+        out_ok[k] = (rc == 0 && res[2 * k] == 1 && res[2 * k + 1] == 0 && ok_range[k] == 1) ? 1 : 0;
+    return 0;
+    API_CATCH
+}
+// EncModelParams::verify, EncL2 arm (params.rs:205-233), for n_clients messages of one shape: the K x D square-rand proofs in one batched check,
+// the range proofs over all c.L of every client in another, the sums of c_sq per client, the K sum-of-squares proofs in a third.
+// out_ok[k] = exactly what rofl_enc_l2_verify(message k, ...) returns (1 / 0: that arm rejects, rather than refuses, undecodable points).
+extern "C" int rofl_enc_l2_verify_batch(rofl_ctx *c, size_t n_clients, const uint8_t *enc_values96, size_t D, const uint8_t *square_proofs192, const uint8_t *range_proofs,
+                                        size_t plen, size_t n_proofs, const uint8_t *square_range_proofs, size_t sq_plen, int prove_range, int l2_range,
+                                        const uint8_t seed[32], int *out_ok) {
+    API_TRY
+    const size_t K = n_clients;
+    if (!D || !n_proofs || !out_ok) return ROFL_ERR_ARGS;
+    if (!K) return 0;
+    if (!enc_values96 || !square_proofs192 || !seed) return ROFL_ERR_ARGS;
+    lane_guard lg(c->e); cudaStream_t s = lg.s();
+    staged_in de(enc_values96, 96 * D * K, s), dsp(square_proofs192, 192 * D * K, s);
+    dev_buf dL(32 * D * K, s), dSc(64 * D * K, s), dCsq(32 * D * K, s), dres(2 * sizeof(int) * K, s);
+    std::vector<int> res(2 * K), ok_range(K, 0), ok_sum(K, 0), bad(K, 0);
+    for (size_t k = 0; k < K; k++) { res[2 * k] = 1; res[2 * k + 1] = 0; }
+    rt_h2d(dres.p, res.data(), sizeof(int) * 2 * K, s);
+    sigma_verify_groups(c->e, s, 2, dsp.b.as<uint8_t>(), de.b.as<uint8_t>(), D * K, seed, D, dres.as<int>());
+    LAUNCH(k_split96, dim3((unsigned)((D * K + 255) / 256)), dim3(256), s, dL.as<uint8_t>(), dSc.as<uint8_t>(), dCsq.as<uint8_t>(), de.b.as<uint8_t>(), D * K);
+    // sum_i c_sq,i per client; a c_sq that does not decode is a reject of its message
+    const int nb = (int)std::max<size_t>(1, std::min<size_t>(64, (D + 127) / 128));
+    dev_buf dpart(sizeof(p3_st) * nb * K, s), dbad(sizeof(int) * K, s), dsum(32 * K, s);
+    rt_memset(dbad.p, 0, sizeof(int) * K, s);
+    LAUNCH_COOP(k_points_sum, dim3(nb, (unsigned)K), dim3(128), s, dpart.as<p3_st>(), dCsq.as<uint8_t>(), D, dbad.as<int>());
+    { finalize_args f = {}; f.partial = dpart.as<p3_st>(); f.npartial = nb; f.tabB = c->e.sh->tabB; f.tabH = c->e.sh->tabH; f.out32 = dsum.as<uint8_t>(); f.count = (int)K; run_finalize(s, f); }
+    std::vector<uint8_t> sums(32 * K);
+    rt_d2h(res.data(), dres.p, sizeof(int) * 2 * K, s); rt_d2h(bad.data(), dbad.p, sizeof(int) * K, s); rt_d2h(sums.data(), dsum.p, 32 * K, s); rt_sync(s);
+    const int rr = engine_range_verify_batch(c->e, range_proofs, plen, n_proofs, dL.as<uint8_t>(), D, K, prove_range, seed, ok_range.data());
+    const int rs = engine_l2_verify_batch(c->e, square_range_proofs, sq_plen, sums.data(), K, l2_range, seed, ok_sum.data());
+    for (size_t k = 0; k < K; k++)
+        out_ok[k] = (rr == 0 && rs == 0 && res[2 * k] == 1 && res[2 * k + 1] == 0 && ok_range[k] == 1 && !bad[k] && ok_sum[k] == 1) ? 1 : 0;
+    return 0;
+    API_CATCH
+}
+
 // ---- test hooks (tests/test_emul_vs_oracle.py, tests/test_gpu_parity.py, tests/test_msm_kernels.py) -----------------------------------------------
 // the warp-cooperative V absorb (ts_kernels.cuh, k_ts_absorbV) against the sequential transcript code for the same m commitments: 0 equal, 1 different
 extern "C" int rofl_debug_ts_absorb(rofl_ctx *c, const uint8_t *V32, size_t m, int n, int label_id) {
@@ -600,6 +686,17 @@ extern "C" int rofl_debug_crp_rlc(rofl_ctx *c, size_t n_clients, const uint8_t *
     std::vector<int> ok(n_clients); int holds = 0;
     const int rc = engine_crp_verify_batch(c->e, proofs128, pairs64, nullptr, D, n_clients, seed, ok.data(), &holds);
     return rc < 0 ? rc : holds;
+    API_CATCH
+}
+// the batched rand-proof (kind 1) / square-rand-proof (kind 2) check of sigma_verify_groups alone, over n_elems elements as one update and without the
+// size threshold: 1 = every range's combination held and no element is malformed, 0 = not.  proofs n_elems x 128 | 192, commits n_elems x 64 | 96 (host)
+extern "C" int rofl_debug_sigma_rlc(rofl_ctx *c, int kind, size_t n_elems, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32]) {
+    API_TRY
+    if ((kind != 1 && kind != 2) || !n_elems || !proofs || !commits || !seed) return ROFL_ERR_ARGS;
+    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    lane_guard lg(c->e); cudaStream_t s = lg.s();
+    staged_in dp(proofs, pw * n_elems, s), dc(commits, cw * n_elems, s);
+    return sigma_verify_rlc(c->e, s, kind, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), n_elems, seed);
     API_CATCH
 }
 // the batching scalars (c_i | rho_i, 2 x n_proofs x 32 bytes) the verifier derives for this call; return value as rofl_range_verify

@@ -24,7 +24,9 @@
 
 enum { ROFL_ERR_BITSIZE_ = -7 };          // include/rofl_b200.h ROFL_ERR_BITSIZE
 enum { DOM_RANGE_PROVE = 1, DOM_RANGE_VERIFY = 2, DOM_SQUARE = 3, DOM_L2_PROVE = 4, DOM_L2_VERIFY = 5, DOM_CRP = 6, DOM_RND_VEC = 7, DOM_RANDPROOF = 8, DOM_SQUARE_RAND = 9,
-       DOM_CRP_BATCH = 0x62707263 /* "crpb" as LE32: the weights of engine_crp_verify_batch */ };
+       DOM_CRP_BATCH = 0x62707263 /* "crpb" as LE32: the weights of engine_crp_verify_batch */,
+       DOM_RP_RLC = 0x6c727072 /* "rprl": the weights of the batched rand-proof check (sigma_verify_rlc, kind 1) */,
+       DOM_SRP_RLC = 0x6c727273 /* "srrl": the same for square-rand proofs (kind 2) */ };
 enum { PROF_FOLD = 0, PROF_MSM = 1, PROF_COMMIT = 2, PROF_SQUARE = 3, PROF_RTMSM = 4, PROF_TAIL = 5, PROF_FRZ = 6, PROF_SLOTS = 8 };
 
 struct gens_entry { int n = 0; int cap = 0; niels_st *G = nullptr, *H = nullptr;
@@ -79,6 +81,7 @@ struct rofl_engine {
     int ts_host_m = 8192;                 // chunks with more commitments than this absorb them on the host (absorb_commitments)
     int rt_per = 2;                       // table-MSM terms per thread and block: short blocks let the other groups' small kernels in quickly
     double rt_mem_frac = 0.45;            // tables may take this fraction of the free device memory
+    size_t sigma_rlc_terms = (size_t)1 << 24;      // MSM terms per range of the batched rand / square-rand proof check (sigma_verify_rlc)
 };
 static thread_local lane *tl_lane = nullptr; static thread_local rofl_engine *tl_lane_engine = nullptr; static thread_local int tl_lane_depth = 0;
 static inline lane *lane_new() {
@@ -1391,10 +1394,80 @@ static int engine_sigma_verify(rofl_engine &e, int kind, const uint8_t *d_proofs
     lane_guard lg(e);
     cudaStream_t s = lg.s();
     dev_buf d_res(2 * sizeof(int), s); int init[2] = {1, 0}; rt_h2d(d_res.p, init, sizeof(init), s);
-    LAUNCH(k_sigma_verify, dim3((unsigned)((D + 127) / 128)), dim3(128), s, kind, d_proofs, d_commits, D, e.sh->tabB, e.sh->tabH, d_res.as<int>());
+    LAUNCH(k_sigma_verify, dim3((unsigned)((D + 127) / 128)), dim3(128), s, kind, d_proofs, d_commits, D, e.sh->tabB, e.sh->tabH, d_res.as<int>(), (size_t)0);
     int res[2]; rt_d2h(res, d_res.p, sizeof(res), s); rt_sync(s);
     if (res[1]) return -1;
     return res[0] ? 1 : 0;
+}
+
+// All N rand proofs (kind 1) or square-rand proofs (kind 2) of a call, in updates of `group` elements, in random linear combinations
+// (kernels.cuh, k_sigma_rlc_*): the weights come from one hash tree over all N elements; the elements are then checked in ranges of at most
+// e.sigma_rlc_terms MSM terms (4 or 6 per element), one MSM and one k_finalize per range.  A range may start or end inside an update.
+// failed (nullable) receives the element ranges [i0, i1) whose check did not hold or that touch an update with a malformed element.
+// Returns 1 when every range held and no element is malformed, else 0.  The caller holds a lane; s is its stream.
+static int sigma_verify_rlc(rofl_engine &e, cudaStream_t s, int kind, const uint8_t *d_proofs, const uint8_t *d_commits, size_t N, const uint8_t seed[32],
+                            size_t group = 0, std::vector<std::pair<size_t, size_t>> *failed = nullptr) {
+    if (!group) group = N;
+    const size_t np = kind == 1 ? 4 : 6, K = (N + group - 1) / group;
+    const size_t R = std::max<size_t>(1, std::min(e.sigma_rlc_terms, CRP_BATCH_TERMS) / np);          // elements per range
+    const size_t n1 = (N + 63) / 64, n2 = (n1 + 63) / 64, rmax = std::min(R, N), nbmax = (rmax + 127) / 128;
+    dev_buf d_dig(32 * N, s), d_chal(sizeof(sc_st) * N, s), d_l1(32 * n1, s), d_l2(32 * n2, s), d_bad(sizeof(int) * K, s);
+    dev_buf d_scal(sizeof(sc_st) * np * rmax, s), d_part(sizeof(sc_st) * 2 * nbmax, s), d_pts(sizeof(p3_st) * np * rmax, s), d_sum(sizeof(sc_st) * 2, s), d_id(sizeof(int), s);
+    rt_memset(d_bad.p, 0, sizeof(int) * K, s);
+    sigma_rlc_args a = {}; a.kind = kind; a.proofs = d_proofs; a.commits = d_commits; a.N = N; a.group = group; a.tag = kind == 1 ? DOM_RP_RLC : DOM_SRP_RLC;
+    memcpy(a.seed, seed, 32);
+    a.digest = d_dig.as<uint8_t>(); a.chal = d_chal.as<sc_st>(); a.scal = d_scal.as<sc_st>(); a.partial = d_part.as<sc_st>(); a.pts = d_pts.as<p3_st>(); a.bad = d_bad.as<int>();
+    LAUNCH(k_sigma_rlc_prep, dim3((unsigned)((N + 127) / 128)), dim3(128), s, a);
+    const uint8_t *cur = d_dig.as<uint8_t>(); size_t n = N; uint8_t *bufs[2] = {d_l1.as<uint8_t>(), d_l2.as<uint8_t>()}; int which = 0;
+    do {                                                   // hash tree, 64 digests per node
+        const size_t nn = (n + 63) / 64;
+        LAUNCH(k_hash_tree, dim3((unsigned)((nn + 127) / 128)), dim3(128), s, bufs[which], cur, n);
+        cur = bufs[which]; which ^= 1; n = nn;
+    } while (n > 1);
+    a.root = cur;
+    std::vector<int> bad(K);
+    int all = 1;
+    for (size_t i0 = 0; i0 < N; i0 += R) {
+        const size_t r = std::min(R, N - i0), T = np * r, k0 = i0 / group, k1 = (i0 + r - 1) / group + 1;
+        const unsigned nb = (unsigned)((r + 127) / 128);
+        const msm_plan pl = msm_plan_for(T, 1, 2048);
+        a.i0 = i0; a.n = r; a.wbits = pl.c * ((125 + pl.c - 1) / pl.c) - 1;
+        LAUNCH_COOP(k_sigma_rlc_scalars, dim3(nb), dim3(128), s, a);
+        LAUNCH_COOP(k_sc_sum, dim3(1), dim3(256), s, d_sum.as<sc_st>(), d_part.as<sc_st>(), (int)nb, 2);
+        LAUNCH(k_sigma_rlc_points, dim3((unsigned)((T + 127) / 128)), dim3(128), s, a);
+        dev_buf d_win(sizeof(p3_st) * pl.out_count(1), s);
+        msm_args m = {}; m.v[0].scalars = d_scal.as<sc_st>(); m.split = 1; m.T = (uint32_t)T; m.scalar_stride = (uint32_t)T; m.nseg = 1; m.out = d_win.as<p3_st>();
+        m.v[0].seg[0] = mk_seg(d_pts.p, (uint32_t)T, 0, 1);
+        run_msm(e, s, m, pl, 1);
+        finalize_args f = {}; fin_windows(f, d_win.as<p3_st>(), pl); f.sBa = d_sum.as<sc_st>(); f.sHa = d_sum.as<sc_st>() + 1; f.tabB = e.sh->tabB; f.tabH = e.sh->tabH; f.is_id = d_id.as<int>(); f.count = 1;
+        run_finalize(s, f);
+        int id = 0; rt_d2h(&id, d_id.p, sizeof(int), s); rt_d2h(&bad[k0], d_bad.as<int>() + k0, sizeof(int) * (k1 - k0), s); rt_sync(s);
+        bool ok = id == 1; for (size_t k = k0; k < k1; k++) ok = ok && !bad[k];
+        if (!ok) { all = 0; if (failed) failed->push_back({i0, i0 + r}); }
+    }
+    return all;
+}
+// verdicts of the rand / square-rand proofs of N elements in updates of `group` elements each (group = 0: one update): d_res = (all valid, format
+// error) per update, initialised to (1, 0) by the caller -- exactly what k_sigma_verify gives.  Calls of at least 256 elements go through the
+// batched check first; every update a failed range touches is then checked element by element (k_sigma_verify), each update at most once.
+static void sigma_verify_groups(rofl_engine &e, cudaStream_t s, int kind, const uint8_t *d_proofs, const uint8_t *d_commits, size_t N, const uint8_t seed[32],
+                                size_t group, int *d_res) {
+    if (!N) return;
+    if (!group) group = N;
+    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    void *tk = rt_prof_begin(PROF_SQUARE, s);
+    std::vector<std::pair<size_t, size_t>> failed;
+    if (N < 256) failed.push_back({0, N});
+    else sigma_verify_rlc(e, s, kind, d_proofs, d_commits, N, seed, group, &failed);
+    size_t next = 0;                                       // first update not yet checked element by element
+    for (const auto &rg : failed) {
+        const size_t k0 = std::max(next, rg.first / group), k1 = (rg.second - 1) / group + 1;
+        if (k0 >= k1) continue;
+        const size_t j0 = k0 * group, n = std::min(N, k1 * group) - j0;
+        LAUNCH(k_sigma_verify, dim3((unsigned)((n + 127) / 128)), dim3(128), s, kind, d_proofs + pw * j0, d_commits + cw * j0, n, e.sh->tabB, e.sh->tabH, d_res + 2 * k0, group);
+        next = k1;
+    }
+    rt_prof_end(PROF_SQUARE, tk, s);
 }
 
 // sum of D compressed points -> compressed (device in, host out); -4 if one does not decode

@@ -1062,9 +1062,12 @@ KERNEL void LB(128, 1) k_sigma_prove(sigma_args a) {
     for (int k = 0; k < cw; k++) st_bytes32(a.commits + 32 * (cw * i + k), com + 32 * k);
 }
 KLAUNCH(k_sigma_prove, false, (sigma_args a), (a))
-KERNEL void LB(128, 1) k_sigma_verify(int kind, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result) {
+//   group: elements per update when several updates are checked in one launch (result = 2 ints per update, counted from the launch's first
+//   element, which starts an update); 0 = one update
+KERNEL void LB(128, 1) k_sigma_verify(int kind, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result, size_t group) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= D) return;
+    if (group) result += 2 * (i / group);
     uint8_t proof[192], com[96];
     const int pw = kind == 1 ? 4 : 6, cw = kind == 1 ? 2 : 3;
     for (int k = 0; k < pw; k++) ld_bytes32(proof + 32 * k, proofs + 32 * (pw * i + k));
@@ -1073,7 +1076,109 @@ KERNEL void LB(128, 1) k_sigma_verify(int kind, const uint8_t *proofs, const uin
     if (rc < 0) atomicOr(result + 1, 1);
     else if (rc == 0) atomicAnd(result, 0);
 }
-KLAUNCH(k_sigma_verify, false, (int kind, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result), (kind, proofs, commits, D, tabB, tabH, result))
+KLAUNCH(k_sigma_verify, false, (int kind, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result, size_t group),
+        (kind, proofs, commits, D, tabB, tabH, result, group))
+#endif
+
+// ---- the same verdict for ALL rand proofs (kind 1) or square-rand proofs (kind 2) of a call with ONE random linear combination per range of
+//        elements (engine.cuh, sigma_verify_groups).  Per element, kind 1 checks (rand_verify_one)
+//          z_m B + z_r H == C'_L + c L          z_r B == C'_R + c R
+//        and kind 2 (square_rand_verify_one) additionally            z_m L + z_r2 H == C'_sq + c C_sq       (z_r = z_r1).
+//   Weighted by rho_i, sigma_i (and tau_i) and negated, the sum over the elements of a range is one MSM plus two fixed-base terms:
+//     kind 1:  sum_i rho C'_L + rho c L + sigma C'_R + sigma c R                                          - (sum rho z_m + sigma z_r) B - (sum rho z_r) H == 0
+//     kind 2:  sum_i rho C'_L + (rho c - tau z_m) L + sigma C'_R + sigma c R + tau C'_sq + tau c C_sq     - (sum rho z_m + sigma z_r1) B - (sum rho z_r1 + tau z_r2) H == 0
+//   Weights: key_i = SHA3-256(root | seed | tag | LE64 N | LE64 i) over the N elements of the call, root = the hash tree (k_hash_tree) over
+//   leaf_i = SHA3-256(0x00 | commitments_i | proof_i); one ChaCha20 block of key_i gives rho = words 0..4, sigma = 5..9, tau = 10..14, each masked
+//   to wbits bits.  They stay short and positive: the signs live in the fixed-base coefficients only (see k_sq_rlc_scalars).
+//   A malformed element (non-canonical response, undecodable point) sets the bad flag of its update (element i belongs to update i / group).
+//   k_sigma_rlc_prep:    format checks, challenge c_i, leaf digest_i                         (one thread per element of the call)
+//   k_hash_tree:         the tree above
+//   k_sigma_rlc_scalars: weights, the 4 / 6 point scalars of the element, block sums of the B and H scalars      (elements [i0, i0 + n))
+//   k_sigma_rlc_points:  the 4 / 6 points of each element of the range                       (one thread per point)
+//   Point (and scalar) w of element i, w < 2 * kind + 2: even w from the proof, odd w from the commitments, word w / 2 of each:
+//     C'_L, L, C'_R, R (, C'_sq, C_sq)
+struct sigma_rlc_args {
+    int kind; const uint8_t *proofs, *commits; size_t N, group, i0, n; uint32_t tag; uint8_t seed[32];
+    uint8_t *digest; sc_st *chal; const uint8_t *root; sc_st *scal, *partial; p3_st *pts; int *bad; int wbits;
+};
+#ifdef KG_SQUARE
+KERNEL void LB(128, 1) k_sigma_rlc_prep(sigma_rlc_args a) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.N) return;
+    const int pw = a.kind == 1 ? 4 : 6, cw = a.kind == 1 ? 2 : 3;
+    uint8_t buf[288];                                                              // commitments | proof
+    for (int k = 0; k < cw; k++) ld_bytes32(buf + 32 * k, a.commits + 32 * (cw * i + k));
+    for (int k = 0; k < pw; k++) ld_bytes32(buf + 32 * (cw + k), a.proofs + 32 * (pw * i + k));
+    const uint8_t *com = buf, *proof = buf + 32 * cw;
+    sc z; bool ok = true;
+    for (int k = pw / 2; k < pw; k++) { sc_frombytes(z, proof + 32 * k); ok = ok && sc_is_canonical(z); }
+    if (!ok) atomicOr(a.bad + i / a.group, 1);
+    sc c;
+    if (a.kind == 1) rp_transcript_challenge(c, com, proof); else srp_transcript_challenge(c, com, proof);
+    st_sc(a.chal + i, c);
+    uint8_t dg[32]; { sponge sp; sponge_init(sp, 136); const uint8_t tag = 0x00; sponge_absorb(sp, &tag, 1); sponge_absorb(sp, buf, 32 * (cw + pw)); sponge_finish(sp, 0x06); sponge_squeeze(sp, dg, 32); }
+    st_bytes32(a.digest + 32 * i, dg);
+}
+KLAUNCH(k_sigma_rlc_prep, false, (sigma_rlc_args a), (a))
+KERNEL void LB(128, 1) k_sigma_rlc_scalars(sigma_rlc_args a) {
+    __shared__ sc_st buf[128];
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; const int tid = threadIdx.x;
+    sc sB, sH; sc_0(sB); sc_0(sH);
+    if (t < a.n) {
+        const size_t i = a.i0 + t;
+        const int pw = a.kind == 1 ? 4 : 6;
+        uint8_t kb[84], key[32]; ld_bytes32(kb, a.root);
+        for (int k = 0; k < 32; k++) kb[32 + k] = a.seed[k];
+        for (int k = 0; k < 4; k++) kb[64 + k] = (uint8_t)(a.tag >> (8 * k));
+        for (int k = 0; k < 8; k++) { kb[68 + k] = (uint8_t)((uint64_t)a.N >> (8 * k)); kb[76 + k] = (uint8_t)((uint64_t)i >> (8 * k)); }
+        sha3_256(key, kb, 84);
+        uint32_t kw[8], w[16];
+        for (int k = 0; k < 8; k++) kw[k] = (uint32_t)key[4 * k] | ((uint32_t)key[4 * k + 1] << 8) | ((uint32_t)key[4 * k + 2] << 16) | ((uint32_t)key[4 * k + 3] << 24);
+        chacha20_block_words(w, kw, 0);
+        sc rho, sig, tau; sc_0(rho); sc_0(sig); sc_0(tau);
+        for (int k = 0; k < 5; k++) { rho.v[k] = w[k]; sig.v[k] = w[5 + k]; tau.v[k] = w[10 + k]; }
+        { const int full = a.wbits >> 5, rem = a.wbits & 31;
+          for (int k = 0; k < 5; k++) { const uint32_t m = k < full ? 0xffffffffu : (k == full ? ((1u << rem) - 1u) : 0u); rho.v[k] &= m; sig.v[k] &= m; tau.v[k] &= m; } }
+        uint8_t zb[32]; sc zm, zr, c, u, v;
+        const uint8_t *pf = a.proofs + 32 * (pw * i + pw / 2);                     // z_m | z_r (| z_r2)
+        ld_bytes32(zb, pf); sc_frombytes(zm, zb);
+        ld_bytes32(zb, pf + 32); sc_frombytes(zr, zb);
+        ld_sc(c, a.chal + i);
+        sc_st *o = a.scal + pw * t;
+        st_sc(o, rho);                                                             // C'_L: rho
+        sc_mul(u, rho, c);
+        st_sc(o + 2, sig);                                                         // C'_R: sigma
+        sc_mul(v, sig, c); st_sc(o + 3, v);                                        // R:    sigma c
+        sc_mul(sB, rho, zm); sc_mul(v, sig, zr); sc_add(sB, sB, v); sc_neg(sB, sB); // B:    -(rho z_m + sigma z_r)
+        sc_mul(sH, rho, zr);                                                       // H:    -(rho z_r (+ tau z_r2))
+        if (a.kind == 2) {
+            sc zr2; ld_bytes32(zb, pf + 64); sc_frombytes(zr2, zb);
+            sc_mul(v, tau, zm); sc_sub(u, u, v);                                   // L:    rho c - tau z_m
+            st_sc(o + 4, tau);                                                     // C'_sq: tau
+            sc_mul(v, tau, c); st_sc(o + 5, v);                                    // C_sq: tau c
+            sc_mul(v, tau, zr2); sc_add(sH, sH, v);
+        }
+        st_sc(o + 1, u);                                                           // L:    rho c (kind 1)
+        sc_neg(sH, sH);
+    }
+    block_sum_sc(sB, buf, tid, 128);
+    if (tid == 0) st_sc(a.partial + 2 * (size_t)blockIdx.x, sB);
+    block_sum_sc(sH, buf, tid, 128);
+    if (tid == 0) st_sc(a.partial + 2 * (size_t)blockIdx.x + 1, sH);
+}
+KLAUNCH(k_sigma_rlc_scalars, true, (sigma_rlc_args a), (a))
+KERNEL void LB(128, 2) k_sigma_rlc_points(sigma_rlc_args a) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int pw = a.kind == 1 ? 4 : 6, cw = a.kind == 1 ? 2 : 3;
+    if (t >= (size_t)pw * a.n) return;
+    const size_t i = a.i0 + t / pw; const int w = (int)(t % pw);
+    const uint8_t *src = (w & 1) ? a.commits + 32 * (cw * i + (w >> 1)) : a.proofs + 32 * (pw * i + (w >> 1));
+    uint8_t enc[32]; ld_bytes32(enc, src);
+    ge_p3 P;
+    if (!ge_decompress(P, enc)) { atomicOr(a.bad + i / a.group, 1); ge_p3_0(P); }
+    st_p3(a.pts + t, P);
+}
+KLAUNCH(k_sigma_rlc_points, false, (sigma_rlc_args a), (a))
 #endif
 
 // ===================================================================================================================
@@ -1362,7 +1467,10 @@ void launch_k_verify_tables(dim3 g_, dim3 b_, cudaStream_t s_, sc_st *tab, vtab_
 void launch_k_verify_scalars(dim3 g_, dim3 b_, cudaStream_t s_, sc_st *gh, const sc_st *tab, vtab_layout t, const sc_st *chal, int chal_stride, int n, int C);
 void launch_k_square_prove(dim3 g_, dim3 b_, cudaStream_t s_, square_args a);
 void launch_k_sigma_prove(dim3 g_, dim3 b_, cudaStream_t s_, sigma_args a);
-void launch_k_sigma_verify(dim3 g_, dim3 b_, cudaStream_t s_, int kind, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result);
+void launch_k_sigma_verify(dim3 g_, dim3 b_, cudaStream_t s_, int kind, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result, size_t group);
+void launch_k_sigma_rlc_prep(dim3 g_, dim3 b_, cudaStream_t s_, sigma_rlc_args a);
+void launch_k_sigma_rlc_scalars(dim3 g_, dim3 b_, cudaStream_t s_, sigma_rlc_args a);
+void launch_k_sigma_rlc_points(dim3 g_, dim3 b_, cudaStream_t s_, sigma_rlc_args a);
 void launch_k_square_verify(dim3 g_, dim3 b_, cudaStream_t s_, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result, size_t group);
 void launch_k_sq_rlc_prep(dim3 g_, dim3 b_, cudaStream_t s_, sq_rlc_args a);
 void launch_k_hash_tree(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const uint8_t *in, size_t n);

@@ -68,6 +68,13 @@ extern "C" {
     pub fn rofl_enc_range_compressed_verify_batch(ctx: *mut rofl_ctx, n_clients: size_t, enc_values64: *const u8, d: size_t, rand_proofs128: *const u8, range_proofs: *const u8,
                                                   proof_len: size_t, n_proofs: size_t, prove_range: c_int, check_percentage: c_float, seed32: *const u8,
                                                   out_ok: *mut c_int) -> c_int;
+    pub fn rofl_rand_verify_batch(ctx: *mut rofl_ctx, n_clients: size_t, proofs128: *const u8, pairs64: *const u8, d: size_t, seed32: *const u8, out_ok: *mut c_int) -> c_int;
+    pub fn rofl_square_rand_verify_batch(ctx: *mut rofl_ctx, n_clients: size_t, proofs192: *const u8, commits96: *const u8, d: size_t, seed32: *const u8, out_ok: *mut c_int) -> c_int;
+    pub fn rofl_enc_range_verify_batch(ctx: *mut rofl_ctx, n_clients: size_t, enc_values64: *const u8, d: size_t, rand_proofs128: *const u8, range_proofs: *const u8,
+                                       proof_len: size_t, n_proofs: size_t, prove_range: c_int, check_percentage: c_float, seed32: *const u8, out_ok: *mut c_int) -> c_int;
+    pub fn rofl_enc_l2_verify_batch(ctx: *mut rofl_ctx, n_clients: size_t, enc_values96: *const u8, d: size_t, square_proofs192: *const u8, range_proofs: *const u8,
+                                    proof_len: size_t, n_proofs: size_t, square_range_proofs: *const u8, sq_proof_len: size_t, prove_range: c_int, l2_range: c_int,
+                                    seed32: *const u8, out_ok: *mut c_int) -> c_int;
     pub fn rofl_aggregate(ctx: *mut rofl_ctx, points32: *const u8, n_clients: size_t, d: size_t, init_unity: c_int, out32: *mut u8) -> c_int;
     pub fn rofl_dlog(ctx: *mut rofl_ctx, points32: *const u8, d: size_t, table_size: u64, bsgs_bits: c_int, n_bits: c_int, frac: c_int, out_scalars32: *mut u8, out_f32: *mut c_float) -> c_int;
     pub fn rofl_ctx_stream(ctx: *mut rofl_ctx) -> *mut c_void;

@@ -39,3 +39,23 @@ pub fn verify_l2rangeproof_vec(randproof_vec: &Vec<SquareRandProof>, commit_vec:
         _ => Err(ProofError::FormatError.into()),
     }
 }
+
+/// Server side, the square-rand proofs of all clients of a round in one batched check (random linear combinations over every element; the
+/// reference calls verify_l2rangeproof_vec once per client).  Every client must have the same number of elements.  One verdict per client,
+/// identical to verify_l2rangeproof_vec's.
+pub fn verify_l2rangeproof_vec_batch(randproofs: &[&Vec<SquareRandProof>], commits: &[&Vec<SquareRandProofCommitments>]) -> Vec<Result<bool, L2RangeProofError>> {
+    let k = randproofs.len();
+    assert!(k > 0 && commits.len() == k);
+    let d = commits[0].len();
+    let (mut p, mut c) = (Vec::with_capacity(192 * d * k), Vec::with_capacity(96 * d * k));
+    for (ps, cs) in randproofs.iter().zip(commits) {
+        if ps.len() != cs.len() || cs.len() != d { panic!("verify_l2rangeproof_vec_batch: every client needs {} proofs and commitments", d); }
+        for x in ps.iter() { p.extend_from_slice(&x.to_bytes()); }
+        for x in cs.iter() { c.extend_from_slice(&x.to_bytes()); }
+    }
+    let mut ok = vec![0i32; k];
+    let seed = b200::seed();
+    let rc = unsafe { ffi::rofl_square_rand_verify_batch(b200::ctx(), k, p.as_ptr(), c.as_ptr(), d, seed.as_ptr(), ok.as_mut_ptr()) };
+    assert!(rc == 0, "verify_l2rangeproof_vec_batch: rofl_b200 error {}: {}", rc, b200::last_error());
+    ok.into_iter().map(|r| match r { 1 => Ok(true), 0 => Ok(false), _ => Err(ProofError::FormatError.into()) }).collect()
+}
