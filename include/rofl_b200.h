@@ -63,7 +63,8 @@ void rofl_set_host_threads(rofl_ctx *ctx, int n);          /* host threads used 
  * terms per thread, "tail_ncta" thread blocks (one cluster) per chunk in the tail kernel (1, 2, 4, 8), "frozen" 0/1 frozen-level middle rounds,
  * "nt_unfold" / "nt_unfold_min" unfolded rounds without tables, "ts_host_m" chunk size above which commitments are absorbed on the host,
  * "max_lanes" concurrent callers, "drop_tables", "trim" (hand cached scratch back to CUDA), "sigma_rlc_terms" MSM terms per range of the
- * batched rand / square-rand proof check (1 .. 2^24, the default).
+ * batched rand / square-rand proof check (1 .. 2^24, the default), "crp_batch_terms" MSM terms per client group of the batched compressed-rand-proof
+ * check (1 .. 2^24, the default; a group holds at least one client).
  * returns 0, -2 unknown name */
 int rofl_set_option(rofl_ctx *ctx, const char *name, long value);
 
@@ -249,6 +250,20 @@ int rofl_debug_crp_rlc(rofl_ctx *, size_t n_clients, const uint8_t *proofs128, c
  * size: 1 = the combination over all elements held and none is malformed, 0 = it did not */
 int rofl_debug_sigma_rlc(rofl_ctx *, int kind, size_t n_elems, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32]);
 int rofl_debug_verify_weights(rofl_ctx *, const uint8_t *proofs, size_t proof_len, size_t n_proofs, const uint8_t *commits32, size_t D, int range, const uint8_t seed[32], uint8_t *out_weights);
+/* the terms of one batched check as its production code computed them (nothing is derived by the hook).  family 0: square proofs (proofs
+ * n_clients x D x 160, commits x 64); 1: rand proofs (x 128, x 64); 2: square-rand proofs (x 192, x 96) -- families 0-2 also below the size thresholds of
+ * the public calls; 3: compressed rand proofs (proofs n_clients x 128, commits = the pairs n_clients x D x 64, D <= 900 000).
+ *   root32: the digest the weights are keyed from; chal32: the challenge of every element (families 0-2, n_clients x D) or client (3, n_clients);
+ *   ranges: per range of elements (client group for family 3) 8 int64: i0, n, MSM window width c, weight bits wbits (0 for family 3: 128-bit rho_k),
+ *     is_id of output 0 and 1 (-1: no such output), index of its first scalar in scalars32, index of its first flag in bad;
+ *   scalars32: the MSM scalars of every range in term order; coef32: per range sB[0], sB[1], sH[0], sH[1] as given to k_finalize (zero where unused);
+ *   bad: per range, the bad flags of the clients it touches (family 0: the one format flag word);
+ *   verdicts: per client, what the public batch call returns for it (1 / 0 / -1; family 3 as rofl_crp_verify).
+ *   cap / cnt: capacities of ranges, scalars32, bad, and what the call produced.
+ * returns 1 = every range's combination held and nothing was malformed, 0 = not, ROFL_ERR_ARGS (also when a capacity is short: cnt tells the need) */
+int rofl_debug_rlc_terms(rofl_ctx *, int family, size_t n_clients, size_t D, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32],
+                         uint8_t *root32, uint8_t *chal32, int64_t *ranges, uint8_t *scalars32, uint8_t *coef32, int *bad, int *verdicts,
+                         const size_t cap[3], size_t cnt[3]);
 /* the MSM front end alone (production plan / forced window width / generator tables, then k_finalize): out32[k] = sum_t s[k][t] P_t + sB[k] B + sH[k] H.
  * scalars32: n_msm x T canonical scalars; points32: T shared or n_msm x T (points_per_msm) encodings, or NULL for BulletproofGens(gen_n, T / (2 gen_n));
  * path 0 = msm_plan_for(T, n_msm, big_min), 1 = window width c with `knob` slices (c <= 8) / parts (c >= 9), 2 = generator tables.  sB32 / sH32 may be NULL.

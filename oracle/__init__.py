@@ -180,6 +180,19 @@ def crp_prove(values, value_com, blind, n_bits=16, frac=7, seed=SEED0):
 def crp_verify(proof, pairs):
     p = _u8(pairs).reshape(-1, 64)
     return lib().orc_crp_verify(_p(_u8(proof, 128)), _p(p), C.c_size_t(p.shape[0]))
+# challenges of the sigma proofs, from the oracle's own transcripts (the batched verifiers' weights are keyed on them)
+def _challenge(name, com, cp, *mid):
+    o = np.zeros(32, np.uint8); com = _u8(com); cp = _u8(cp).copy()
+    getattr(lib(), name)(_p(o), _p(com), *mid, _p(cp)); return o.tobytes()
+def sq_challenge(commits64, proof160):
+    """square proof: commitments c_l | c_sq, proof C'_l | C'_sq | z_m | z_r1 | z_r2"""
+    return _challenge("orc_sq_challenge", _u8(commits64, 64), _u8(proof160, 160)[:64])
+def rp_challenge(pair64, proof128):
+    return _challenge("orc_rp_challenge", _u8(pair64, 64), _u8(proof128, 128)[:64])
+def srp_challenge(commits96, proof192):
+    return _challenge("orc_srp_challenge", _u8(commits96, 96), _u8(proof192, 192)[:96])
+def crp_challenge(proof128, pairs):
+    p = _u8(pairs).reshape(-1, 64); return _challenge("orc_crp_challenge", p, _u8(proof128, 128)[:64], C.c_size_t(p.shape[0]))
 def aggregate(pts, init=0):
     a = _u8(pts); assert a.ndim == 3 and a.shape[2] == 32
     o = np.zeros((a.shape[1], 32), np.uint8); rc = lib().orc_aggregate(_p(o), _p(a), C.c_size_t(a.shape[0]), C.c_size_t(a.shape[1]), init); assert rc == 0; return o

@@ -289,6 +289,12 @@ static void sq_transcript_start(transcript *t, const uint8_t cl[32], const uint8
     transcript_append(t, "dom-sep", (const uint8_t *)"randomness proof v1", 19);                 /* transcript.rs:20-22 */
     transcript_append(t, "C_eg", cl, 32); transcript_append(t, "C_ped", csq, 32);
 }
+/* the challenge of one square proof (dealer.rs:20-27,49-53): com64 = c_l | c_sq, cp64 = C'_l | C'_sq */
+EXPORT void orc_sq_challenge(uint8_t o[32], const uint8_t com64[64], const uint8_t cp64[64]) {
+    transcript t; sc c; sq_transcript_start(&t, com64, com64 + 32);
+    transcript_append(&t, "C_prime_eg", cp64, 32); transcript_append(&t, "C_prime_ped", cp64 + 32, 32);
+    ts_challenge(&t, "c", &c); sc_tobytes(o, &c);
+}
 /* create_l2rangeproof_vec_existing (square_proof_vec/mod.rs:19-75) -> SquareProof::prove_existing (square_proof/mod.rs:42-58).
  * proofs_out: D*160 (C'_l|C'_sq|z_m|z_r1|z_r2), commits_out: D*64 (c_l|c_sq).  returns 0, 1 WrongNumBlindingFactors n/a, -4 bad point */
 EXPORT int orc_square_prove(uint8_t *proofs_out, uint8_t *commits_out, const float *values, const uint8_t *value_com,
@@ -326,6 +332,7 @@ static void rp_challenge(sc *c, const uint8_t pair[64], const uint8_t cp[64]) {
     transcript_append(&t, "C", pair, 64); transcript_append(&t, "C_prime", cp, 64);               /* dealer.rs:20-21,42 */
     ts_challenge(&t, "c", c);
 }
+EXPORT void orc_rp_challenge(uint8_t o[32], const uint8_t pair[64], const uint8_t cp[64]) { sc c; rp_challenge(&c, pair, cp); sc_tobytes(o, &c); }
 EXPORT int orc_rand_prove(uint8_t *proofs_out, uint8_t *pairs_out, const float *values, const uint8_t *value_com, const uint8_t *rv, size_t D, int n_bits, int frac, const uint8_t seed[32]) {
     if (!fp_ok(n_bits, frac)) return -2;
     init_pc(); uint8_t key[32]; orc_derive_key(key, seed, DOM_RANDPROOF, 0); int rc = 0; ge Bp; ge_base(&Bp);
@@ -371,6 +378,7 @@ static void srp_challenge(sc *c, const uint8_t com[96], const uint8_t cp[96]) {
     transcript_append(&t, "C_prime_eg", cp, 64); transcript_append(&t, "C_prime_ped", cp + 64, 32);
     ts_challenge(&t, "c", c);
 }
+EXPORT void orc_srp_challenge(uint8_t o[32], const uint8_t com[96], const uint8_t cp[96]) { sc c; srp_challenge(&c, com, cp); sc_tobytes(o, &c); }
 EXPORT int orc_square_rand_prove(uint8_t *proofs_out, uint8_t *commits_out, const float *values, const uint8_t *value_com, const uint8_t *r1v, const uint8_t *r2v, size_t D,
                                  int n_bits, int frac, const uint8_t seed[32]) {
     if (!fp_ok(n_bits, frac)) return -2;
@@ -429,6 +437,7 @@ static void crp_transcript(transcript *t, const uint8_t *pairs, size_t D, const 
     transcript_append(t, "C_prime_eg", cprime, 64);                                                /* dealer.rs:53-54 */
     ts_challenge(t, "c", c);
 }
+EXPORT void orc_crp_challenge(uint8_t o[32], const uint8_t *pairs, size_t D, const uint8_t cprime[64]) { transcript t; sc c; crp_transcript(&t, pairs, D, cprime, &c); sc_tobytes(o, &c); }
 EXPORT int orc_crp_prove(uint8_t proof_out[128], uint8_t *pairs_out, const float *values, const uint8_t *value_com, const uint8_t *rv, size_t D,
                          int n_bits, int frac, const uint8_t seed[32]) {
     if (!fp_ok(n_bits, frac)) return -2;

@@ -79,6 +79,7 @@ _SIGS = {
     "rofl_debug_sigma_rlc": (C.c_int, [c_vp, C.c_int, c_sz, c_u8p, c_u8p, c_u8p]),
     "rofl_debug_verify_weights": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, c_u8p, c_u8p]),
     "rofl_debug_msm": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_sz, c_u8p, c_u8p, c_u8p, c_vp]),
+    "rofl_debug_rlc_terms": (C.c_int, [c_vp, C.c_int, c_sz, c_sz, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_vp, c_u8p, c_u8p, c_vp, c_vp, c_vp, c_vp]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGS)
 
@@ -351,6 +352,35 @@ class Api:
         pw, cw = (128, 64) if kind == 1 else (192, 96)
         p = _u8(proofs).reshape(-1, pw); c = _u8(commits).reshape(-1, cw)
         return self.lib.rofl_debug_sigma_rlc(self.h, kind, p.shape[0], _ptr(p), _ptr(c), _ptr(_seed(seed)))
+    RLC_WIDTHS = {0: (160, 64), 1: (128, 64), 2: (192, 96), 3: (128, 64)}
+    def debug_rlc_terms(self, family, proofs, commits, seed, max_ranges=None):
+        """The terms of one batched check as its production code computed them (rofl_debug_rlc_terms).  family 0 square, 1 rand, 2 square-rand
+        proofs: proofs [K, D, pw], commits [K, D, cw]; 3 compressed rand proofs: proofs [K, 128], commits = pairs [K, D, 64].
+        -> dict(held, root (32 bytes), chal [K * D or K, 32], verdicts [K], ranges: list of dicts (i0, n, c, wbits, is_id (2), scal [T, 32],
+        sB (2 x 32 bytes), sH (2 x 32 bytes), bad [clients touched]))"""
+        pw, cw = self.RLC_WIDTHS[family]
+        c = _u8(commits); K = c.shape[0]; c = c.reshape(K, -1, cw); D = c.shape[1]
+        p = _u8(proofs).reshape(K, -1) if family == 3 else _u8(proofs).reshape(K, D, pw)
+        N = K if family == 3 else K * D
+        nsc = K * (D + 1) if family == 3 else (6 if family == 2 else 4) * N
+        cap = np.array([max_ranges or min(N, 1 << 16), nsc, (max_ranges or min(N, 1 << 16)) + K], np.uintp)
+        for _ in range(2):                                   # a second call only when the first capacities were short
+            cnt = np.zeros(3, np.uintp); root = np.zeros(32, np.uint8); chal = np.zeros((N, 32), np.uint8); verd = np.zeros(K, np.int32)
+            rng = np.zeros((int(cap[0]), 8), np.int64); sc = np.zeros((int(cap[1]), 32), np.uint8); coef = np.zeros((int(cap[0]), 4, 32), np.uint8); bad = np.zeros(int(cap[2]), np.int32)
+            rc = self.lib.rofl_debug_rlc_terms(self.h, family, K, D, _ptr(p), _ptr(c), _ptr(_u8(seed, 32)), _ptr(root), _ptr(chal), _ptr(rng), _ptr(sc), _ptr(coef), _ptr(bad),
+                                               _ptr(verd), _ptr(cap), _ptr(cnt))
+            if rc == -2 and (cnt > cap).any():
+                cap = np.maximum(cap, cnt); continue
+            break
+        if rc < 0: raise self._err(rc)
+        ranges = []
+        for j in range(int(cnt[0])):
+            i0, n, w, wbits, id0, id1, os_, ob = (int(x) for x in rng[j])
+            T = (int(cnt[1]) if j + 1 == cnt[0] else int(rng[j + 1][6])) - os_
+            nb = (int(cnt[2]) if j + 1 == cnt[0] else int(rng[j + 1][7])) - ob
+            ranges.append(dict(i0=i0, n=n, c=w, wbits=wbits, is_id=(id0, id1), scal=sc[os_:os_ + T], sB=(coef[j, 0].tobytes(), coef[j, 1].tobytes()),
+                               sH=(coef[j, 2].tobytes(), coef[j, 3].tobytes()), bad=bad[ob:ob + nb].tolist()))
+        return dict(held=rc, root=root.tobytes(), chal=chal, verdicts=verd.tolist(), ranges=ranges)
     def debug_verify_weights(self, proofs, commits, rng, seed):
         p = _u8(proofs); p = p.reshape(p.shape[0], -1); c = _u8(commits).reshape(-1, 32); w = np.zeros((2, p.shape[0], 32), np.uint8)
         rc = self.lib.rofl_debug_verify_weights(self.h, _ptr(p), p.shape[1], p.shape[0], _ptr(c), c.shape[0], rng, _ptr(_seed(seed)), _ptr(w))

@@ -32,6 +32,7 @@ extern "C" int rofl_set_option(rofl_ctx *c, const char *name, long value) {
     else if (n == "ts_host_m") c->e.ts_host_m = (int)std::max<long>(0, std::min<long>(1 << 30, value));
     else if (n == "max_lanes") c->e.max_lanes = (int)std::max<long>(1, std::min<long>(64, value));
     else if (n == "sigma_rlc_terms") c->e.sigma_rlc_terms = (size_t)std::max<long>(1, std::min<long>(1L << 24, value));
+    else if (n == "crp_batch_terms") c->e.crp_batch_terms = (size_t)std::max<long>(1, std::min<long>(1L << 24, value));
     else return ROFL_ERR_ARGS;
     return ROFL_OK;
 }
@@ -697,6 +698,53 @@ extern "C" int rofl_debug_sigma_rlc(rofl_ctx *c, int kind, size_t n_elems, const
     lane_guard lg(c->e); cudaStream_t s = lg.s();
     staged_in dp(proofs, pw * n_elems, s), dc(commits, cw * n_elems, s);
     return sigma_verify_rlc(c->e, s, kind, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), n_elems, seed);
+    API_CATCH
+}
+// the terms of one batched check, copied from the buffers of its production code (engine.cuh rlc_tap) and derived by nothing here: family 0 the square
+// proofs (square_verify_groups), 1 / 2 the rand / square-rand proofs (sigma_verify_groups), both over n_clients updates of D elements and below their size
+// thresholds too, 3 the compressed rand proofs of n_clients clients of D pairs (engine_crp_verify_batch; commits = the pairs).  See include/rofl_b200.h.
+extern "C" int rofl_debug_rlc_terms(rofl_ctx *c, int family, size_t n_clients, size_t D, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32],
+                                    uint8_t *root32, uint8_t *chal32, int64_t *ranges, uint8_t *scalars32, uint8_t *coef32, int *bad, int *verdicts,
+                                    const size_t cap[3], size_t cnt[3]) {
+    API_TRY
+    const size_t K = n_clients;
+    if (family < 0 || family > 3 || !K || !D || !proofs || !commits || !seed || !root32 || !chal32 || !ranges || !scalars32 || !coef32 || !bad || !verdicts || !cap || !cnt)
+        return ROFL_ERR_ARGS;
+    if (family == 3 && D > CRP_MAX_D) return ROFL_ERR_ARGS;
+    rlc_tap tap;
+    if (family == 3) {
+        const int rc = engine_crp_verify_batch(c->e, proofs, commits, nullptr, D, K, seed, verdicts, nullptr, &tap);
+        if (rc < 0) return rc;
+    } else {
+        const size_t pw = family == 0 ? 160 : family == 1 ? 128 : 192, cw = family == 2 ? 96 : 64;
+        lane_guard lg(c->e); cudaStream_t s = lg.s();
+        staged_in dp(proofs, pw * D * K, s), dc(commits, cw * D * K, s); dev_buf dres(2 * sizeof(int) * K, s);
+        std::vector<int> res(2 * K);
+        for (size_t k = 0; k < K; k++) { res[2 * k] = 1; res[2 * k + 1] = 0; }
+        rt_h2d(dres.p, res.data(), sizeof(int) * 2 * K, s);
+        if (family == 0) square_verify_groups(c->e, s, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D * K, D, dres.as<int>(), &tap);
+        else sigma_verify_groups(c->e, s, family, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D * K, seed, D, dres.as<int>(), &tap);
+        rt_d2h(res.data(), dres.p, sizeof(int) * 2 * K, s); rt_sync(s);
+        for (size_t k = 0; k < K; k++) verdicts[k] = res[2 * k + 1] ? -1 : res[2 * k] ? 1 : 0;
+    }
+    size_t nsc = 0, nbad = 0;
+    for (const auto &r : tap.ranges) { nsc += r.scal.size(); nbad += r.bad.size(); }
+    cnt[0] = tap.ranges.size(); cnt[1] = nsc; cnt[2] = nbad;
+    if (cnt[0] > cap[0] || nsc > cap[1] || nbad > cap[2]) return ROFL_ERR_ARGS;
+    memcpy(root32, tap.root, 32);
+    for (size_t i = 0; i < tap.chal.size(); i++) memcpy(chal32 + 32 * i, &tap.chal[i], 32);
+    size_t os = 0, ob = 0;
+    for (size_t j = 0; j < tap.ranges.size(); j++) {
+        const rlc_tap::range &r = tap.ranges[j];
+        const int64_t info[8] = {(int64_t)r.i0, (int64_t)r.n, r.c, r.wbits, r.is_id[0], r.is_id[1], (int64_t)os, (int64_t)ob};
+        memcpy(ranges + 8 * j, info, sizeof(info));
+        for (size_t t = 0; t < r.scal.size(); t++) memcpy(scalars32 + 32 * (os + t), &r.scal[t], 32);
+        const sc_st *cf[4] = {&r.sB[0], &r.sB[1], &r.sH[0], &r.sH[1]};
+        for (int q = 0; q < 4; q++) memcpy(coef32 + 128 * j + 32 * q, cf[q], 32);
+        memcpy(bad + ob, r.bad.data(), sizeof(int) * r.bad.size());
+        os += r.scal.size(); ob += r.bad.size();
+    }
+    return tap.held;
     API_CATCH
 }
 // the batching scalars (c_i | rho_i, 2 x n_proofs x 32 bytes) the verifier derives for this call; return value as rofl_range_verify

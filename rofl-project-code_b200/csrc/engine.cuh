@@ -82,6 +82,7 @@ struct rofl_engine {
     int rt_per = 2;                       // table-MSM terms per thread and block: short blocks let the other groups' small kernels in quickly
     double rt_mem_frac = 0.45;            // tables may take this fraction of the free device memory
     size_t sigma_rlc_terms = (size_t)1 << 24;      // MSM terms per range of the batched rand / square-rand proof check (sigma_verify_rlc)
+    size_t crp_batch_terms = (size_t)1 << 24;      // MSM terms per client group of the batched compressed-rand-proof check (crp_batch)
 };
 static thread_local lane *tl_lane = nullptr; static thread_local rofl_engine *tl_lane_engine = nullptr; static thread_local int tl_lane_depth = 0;
 static inline lane *lane_new() {
@@ -1065,11 +1066,27 @@ static int engine_square_prove(rofl_engine &e, const float *d_values, const uint
     if (flags & 1) return -98;
     return 0;
 }
+// bits of the batched checks' weights for an MSM of window width c: the smallest c * w - 1 >= 125 (125 .. 134 for c = 3 .. 16), so that the top
+// window holds c - 1 uniform bits and the signed recoding never carries out of it (kernels.cuh k_sq_rlc_scalars).  Not c * ceil(125 / c) - 1:
+// that is 124 at c = 5, the width msm_plan_for picks for 157 .. 521 terms (small calls and the last range of a long one).
+static inline int rlc_wbits(int c) { return c * ((126 + c - 1) / c) - 1; }
+// Test hook (rofl_debug_rlc_terms): copies of what a batched check computed, taken from the buffers it already has.  The checks take a nullable
+// pointer to one; with nullptr they issue exactly their production launches and copies.
+struct rlc_tap {
+    struct range {
+        size_t i0 = 0, n = 0; int c = 0, wbits = 0;          // elements (clients for the compressed rand proofs) [i0, i0 + n), MSM window width, weight bits
+        int is_id[2] = {-1, -1};                             // k_finalize's identity test per output (-1: no such output)
+        std::vector<sc_st> scal; sc_st sB[2] = {}, sH[2] = {};   // MSM scalars in term order, fixed-base coefficients as given to k_finalize
+        std::vector<int> bad;                                // bad flags of the clients the range touches (square proofs: the one flag word)
+    };
+    uint8_t root[32] = {}; std::vector<sc_st> chal; std::vector<range> ranges; int held = 0;
+};
 // All D square proofs of a call in ONE random linear combination (kernels.cuh, k_sq_rlc_*): 1 = every proof valid and well-formed, 0 = ask the
 // per-element kernel (the combination failed or some element is malformed: the exact verdict, per update, comes from k_square_verify).
-static int square_verify_rlc(rofl_engine &e, cudaStream_t s, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D) {
+// tap (test hook): also runs below the size threshold and without ROFL_SQ_RLC.
+static int square_verify_rlc(rofl_engine &e, cudaStream_t s, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D, rlc_tap *tap = nullptr) {
     static const int on = getenv("ROFL_SQ_RLC") ? atoi(getenv("ROFL_SQ_RLC")) : 1;
-    if (!on || D < 256 || 4 * D > 0x7fffffffu) return 0;
+    if ((!tap && (!on || D < 256)) || 4 * D > 0x7fffffffu) return 0;
     const unsigned nb = (unsigned)((D + 127) / 128);
     const size_t n1 = (D + 63) / 64, n2 = (n1 + 63) / 64;
     dev_buf d_dig(32 * D, s), d_chal(sizeof(sc_st) * D, s), d_scal(sizeof(sc_st) * 4 * D, s), d_part(sizeof(sc_st) * 2 * nb, s), d_pts(sizeof(p3_st) * 4 * D, s);
@@ -1086,7 +1103,7 @@ static int square_verify_rlc(rofl_engine &e, cudaStream_t s, const uint8_t *d_pr
     } while (n > 1);
     a.root = cur;
     const msm_plan pl = msm_plan_for(4 * D, 1, 2048);
-    a.wbits = pl.c * ((125 + pl.c - 1) / pl.c) - 1;
+    a.wbits = rlc_wbits(pl.c);
     LAUNCH_COOP(k_sq_rlc_scalars, dim3(nb), dim3(128), s, a);
     LAUNCH_COOP(k_sc_sum, dim3(1), dim3(256), s, d_sum.as<sc_st>(), d_part.as<sc_st>(), (int)nb, 2);
     LAUNCH(k_sq_rlc_points, dim3((unsigned)((4 * D + 127) / 128)), dim3(128), s, a);
@@ -1096,14 +1113,24 @@ static int square_verify_rlc(rofl_engine &e, cudaStream_t s, const uint8_t *d_pr
     run_msm(e, s, m, pl, 1);
     finalize_args f = {}; fin_windows(f, d_win.as<p3_st>(), pl); f.sBa = d_sum.as<sc_st>(); f.sHa = d_sum.as<sc_st>() + 1; f.tabB = e.sh->tabB; f.tabH = e.sh->tabH; f.is_id = d_id.as<int>(); f.count = 1;
     run_finalize(s, f);
-    int flags = 0, id = 0; rt_d2h(&flags, d_flags.p, sizeof(int), s); rt_d2h(&id, d_id.p, sizeof(int), s); rt_sync(s);
-    return (flags == 0 && id == 1) ? 1 : 0;
+    int flags = 0, id = 0; rt_d2h(&flags, d_flags.p, sizeof(int), s); rt_d2h(&id, d_id.p, sizeof(int), s);
+    rlc_tap::range r;
+    if (tap) {
+        r.n = D; r.c = pl.c; r.wbits = a.wbits; r.scal.resize(4 * D); tap->chal.resize(D);
+        rt_d2h(tap->root, cur, 32, s); rt_d2h(tap->chal.data(), d_chal.p, sizeof(sc_st) * D, s); rt_d2h(r.scal.data(), d_scal.p, sizeof(sc_st) * 4 * D, s);
+        rt_d2h(&r.sB[0], d_sum.p, sizeof(sc_st), s); rt_d2h(&r.sH[0], d_sum.as<sc_st>() + 1, sizeof(sc_st), s);
+    }
+    rt_sync(s);
+    const int held = (flags == 0 && id == 1) ? 1 : 0;
+    if (tap) { r.is_id[0] = id; r.bad = {flags}; tap->ranges.push_back(std::move(r)); tap->held = held; }
+    return held;
 }
 // verdicts of the square proofs of `D` elements in updates of `group` elements each (group = 0: one update): d_res = (all valid, format error) per
 // update, initialised to (1, 0) by the caller.  The batched check first; the per-element kernel only when it does not hold.
-static void square_verify_groups(rofl_engine &e, cudaStream_t s, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D, size_t group, int *d_res) {
+static void square_verify_groups(rofl_engine &e, cudaStream_t s, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D, size_t group, int *d_res,
+                                 rlc_tap *tap = nullptr) {
     void *tk = rt_prof_begin(PROF_SQUARE, s);
-    if (square_verify_rlc(e, s, d_proofs, d_commits, D) != 1)
+    if (square_verify_rlc(e, s, d_proofs, d_commits, D, tap) != 1)
         LAUNCH(k_square_verify, dim3((unsigned)((D + 127) / 128)), dim3(128), s, d_proofs, d_commits, D, e.sh->tabB, e.sh->tabH, d_res, group);
     rt_prof_end(PROF_SQUARE, tk, s);
 }
@@ -1249,7 +1276,8 @@ static int engine_crp_verify(rofl_engine &e, const uint8_t *h_proof, const uint8
 // digest_0 .. digest_(K-1)), rho_k = the low 128 bits of ChaCha20(SHA3-256(root | LE64 k)) (the next block while they are zero).
 // The K transcripts (crp_challenge: one sequential Merlin transcript over all D pairs per client) run on host threads from begin() to end(),
 // while the device decompresses and the caller may queue more work on its stream (the whole-message batch runs its range batch there).
-// Those threads do host work only: they never take a lane.  Clients are processed in groups of at most CRP_BATCH_TERMS terms.
+// Those threads do host work only: they never take a lane.  Clients are processed in groups of at most e.crp_batch_terms terms (default and
+// upper bound CRP_BATCH_TERMS; a group holds at least one client).
 // Verdicts: the combined check holds and no client of the group is malformed -> 1; otherwise malformed clients get -1 and every other client
 // is re-checked on its own with the challenge already computed (engine_crp_verify given c), so each verdict is exactly rofl_crp_verify's.
 #define CRP_BATCH_TERMS ((size_t)1 << 24)
@@ -1260,7 +1288,7 @@ struct crp_batch {
     dev_buf d_cp, d_P, d_bad;
     std::thread th; std::string err;
     crp_batch(rofl_engine &eng, cudaStream_t st, const uint8_t *hp, const uint8_t *hpairs, const uint8_t *dpairs, size_t D_, size_t K_)
-        : e(eng), s(st), h_proofs(hp), h_pairs(hpairs), d_pairs(dpairs), D(D_), K(K_), G(std::max<size_t>(1, std::min(K_, CRP_BATCH_TERMS / (D_ + 1)))),
+        : e(eng), s(st), h_proofs(hp), h_pairs(hpairs), d_pairs(dpairs), D(D_), K(K_), G(std::max<size_t>(1, std::min(K_, eng.crp_batch_terms / (D_ + 1)))),
           c(K_), fmt(K_, 0), d_cp(64 * K_, st), d_P(sizeof(p3_st) * 2 * (G * (D_ + 1)), st), d_bad(sizeof(int) * K_, st) {}
     ~crp_batch() { if (th.joinable()) th.join(); }
     crp_batch(const crp_batch &) = delete; crp_batch &operator=(const crp_batch &) = delete;
@@ -1284,8 +1312,8 @@ static void crp_batch_begin(crp_batch &b) {
         catch (const std::exception &ex) { b.err = ex.what(); }
     });
 }
-// holds (nullable): 1 when the combined check of every group held, else 0
-static void crp_batch_end(crp_batch &b, const uint8_t seed[32], int *out, int *holds = nullptr) {
+// holds (nullable): 1 when the combined check of every group held, else 0.  tap: the test hook's copies (rlc_tap; the range i0 / n are clients)
+static void crp_batch_end(crp_batch &b, const uint8_t seed[32], int *out, int *holds = nullptr, rlc_tap *tap = nullptr) {
     rofl_engine &e = b.e; cudaStream_t s = b.s; const size_t K = b.K, D = b.D;
     b.th.join();
     if (!b.err.empty()) throw std::runtime_error(b.err);
@@ -1298,6 +1326,7 @@ static void crp_batch_end(crp_batch &b, const uint8_t seed[32], int *out, int *h
         sha3_256(&root_in[52 + 32 * k], m, 96);
     }
     uint8_t root[32]; sha3_256(root, root_in.data(), root_in.size());
+    if (tap) { memcpy(tap->root, root, 32); tap->chal.resize(K); for (size_t k = 0; k < K; k++) sc_to_st(tap->chal[k], b.c[k]); }
     std::vector<sc> rho(K);
     for (size_t k = 0; k < K; k++) {
         uint8_t kb[40], key[32]; memcpy(kb, root, 32);
@@ -1314,6 +1343,7 @@ static void crp_batch_end(crp_batch &b, const uint8_t seed[32], int *out, int *h
     const size_t tabn = pow_tab_size(ct);
     std::vector<int> bad(K, 0);
     if (holds) *holds = 1;
+    if (tap) tap->held = 1;
     for (size_t k0 = 0; k0 < K; k0 += b.G) {
         const size_t g = std::min(b.G, K - k0), n = g * (D + 1);
         bool any_fmt = false; for (size_t k = k0; k < k0 + g; k++) any_fmt = any_fmt || b.fmt[k];
@@ -1341,11 +1371,19 @@ static void crp_batch_end(crp_batch &b, const uint8_t seed[32], int *out, int *h
             finalize_args f = {}; fin_windows(f, d_win.as<p3_st>(), pl); f.sBa = d_s.as<sc_st>(); f.sHa = d_s.as<sc_st>() + 2; f.tabB = e.sh->tabB; f.tabH = e.sh->tabH;
             f.is_id = d_id.as<int>(); f.count = 2;
             run_finalize(s, f);
-            rt_d2h(id, d_id.p, sizeof(id), s); rt_d2h(&bad[k0], b.d_bad.as<int>() + k0, sizeof(int) * g, s); rt_sync(s);
+            rt_d2h(id, d_id.p, sizeof(id), s); rt_d2h(&bad[k0], b.d_bad.as<int>() + k0, sizeof(int) * g, s);
+            rlc_tap::range r;
+            if (tap) { r.scal.resize(n); rt_d2h(r.scal.data(), d_sc.p, sizeof(sc_st) * n, s); }
+            rt_sync(s);
+            if (tap) {
+                r.i0 = k0; r.n = g; r.c = pl.c; r.is_id[0] = id[0]; r.is_id[1] = id[1]; r.bad.assign(&bad[k0], &bad[k0] + g);
+                r.sB[0] = h_s[0]; r.sB[1] = h_s[1]; r.sH[0] = h_s[2]; r.sH[1] = h_s[3]; tap->ranges.push_back(std::move(r));
+            }
             bool all = id[0] && id[1]; for (size_t k = k0; k < k0 + g; k++) all = all && !bad[k];
             if (all) { for (size_t k = k0; k < k0 + g; k++) out[k] = 1; continue; }
         }
         if (holds) *holds = 0;
+        if (tap) tap->held = 0;
         for (size_t k = k0; k < k0 + g; k++)
             out[k] = b.fmt[k] ? -1 : engine_crp_verify(e, b.h_proofs + 128 * k, b.h_pairs + 64 * D * k, D, &b.c[k], b.d_pairs + 64 * D * k);
     }
@@ -1353,7 +1391,7 @@ static void crp_batch_end(crp_batch &b, const uint8_t seed[32], int *out, int *h
 // K compressed rand proofs (h_proofs K x 128, h_pairs K x D x 64 host; d_pairs the same pairs on the device, nullable) in one batched check;
 // out[k] = exactly engine_crp_verify(proof k, pairs k, D).  Returns 0, -2 for bad arguments.  holds: as crp_batch_end (left alone when no check runs)
 static int engine_crp_verify_batch(rofl_engine &e, const uint8_t *h_proofs, const uint8_t *h_pairs, const uint8_t *d_pairs, size_t D, size_t K, const uint8_t seed[32], int *out,
-                                   int *holds = nullptr) {
+                                   int *holds = nullptr, rlc_tap *tap = nullptr) {
     if (!out) return -2;
     if (K == 0) return 0;
     if (!h_proofs || (D && !h_pairs)) return -2;
@@ -1364,7 +1402,7 @@ static int engine_crp_verify_batch(rofl_engine &e, const uint8_t *h_proofs, cons
     if (!d_pairs) rt_h2d(d_own.p, h_pairs, 64 * D * K, s);
     crp_batch b(e, s, h_proofs, h_pairs, d_pairs ? d_pairs : d_own.as<uint8_t>(), D, K);
     crp_batch_begin(b);
-    crp_batch_end(b, seed, out, holds);
+    crp_batch_end(b, seed, out, holds, tap);
     return 0;
 }
 
@@ -1404,9 +1442,9 @@ static int engine_sigma_verify(rofl_engine &e, int kind, const uint8_t *d_proofs
 // (kernels.cuh, k_sigma_rlc_*): the weights come from one hash tree over all N elements; the elements are then checked in ranges of at most
 // e.sigma_rlc_terms MSM terms (4 or 6 per element), one MSM and one k_finalize per range.  A range may start or end inside an update.
 // failed (nullable) receives the element ranges [i0, i1) whose check did not hold or that touch an update with a malformed element.
-// Returns 1 when every range held and no element is malformed, else 0.  The caller holds a lane; s is its stream.
+// Returns 1 when every range held and no element is malformed, else 0.  The caller holds a lane; s is its stream.  tap: the test hook's copies (rlc_tap)
 static int sigma_verify_rlc(rofl_engine &e, cudaStream_t s, int kind, const uint8_t *d_proofs, const uint8_t *d_commits, size_t N, const uint8_t seed[32],
-                            size_t group = 0, std::vector<std::pair<size_t, size_t>> *failed = nullptr) {
+                            size_t group = 0, std::vector<std::pair<size_t, size_t>> *failed = nullptr, rlc_tap *tap = nullptr) {
     if (!group) group = N;
     const size_t np = kind == 1 ? 4 : 6, K = (N + group - 1) / group;
     const size_t R = std::max<size_t>(1, std::min(e.sigma_rlc_terms, CRP_BATCH_TERMS) / np);          // elements per range
@@ -1425,13 +1463,14 @@ static int sigma_verify_rlc(rofl_engine &e, cudaStream_t s, int kind, const uint
         cur = bufs[which]; which ^= 1; n = nn;
     } while (n > 1);
     a.root = cur;
+    if (tap) { tap->chal.resize(N); rt_d2h(tap->root, cur, 32, s); rt_d2h(tap->chal.data(), d_chal.p, sizeof(sc_st) * N, s); }
     std::vector<int> bad(K);
     int all = 1;
     for (size_t i0 = 0; i0 < N; i0 += R) {
         const size_t r = std::min(R, N - i0), T = np * r, k0 = i0 / group, k1 = (i0 + r - 1) / group + 1;
         const unsigned nb = (unsigned)((r + 127) / 128);
         const msm_plan pl = msm_plan_for(T, 1, 2048);
-        a.i0 = i0; a.n = r; a.wbits = pl.c * ((125 + pl.c - 1) / pl.c) - 1;
+        a.i0 = i0; a.n = r; a.wbits = rlc_wbits(pl.c);
         LAUNCH_COOP(k_sigma_rlc_scalars, dim3(nb), dim3(128), s, a);
         LAUNCH_COOP(k_sc_sum, dim3(1), dim3(256), s, d_sum.as<sc_st>(), d_part.as<sc_st>(), (int)nb, 2);
         LAUNCH(k_sigma_rlc_points, dim3((unsigned)((T + 127) / 128)), dim3(128), s, a);
@@ -1441,24 +1480,30 @@ static int sigma_verify_rlc(rofl_engine &e, cudaStream_t s, int kind, const uint
         run_msm(e, s, m, pl, 1);
         finalize_args f = {}; fin_windows(f, d_win.as<p3_st>(), pl); f.sBa = d_sum.as<sc_st>(); f.sHa = d_sum.as<sc_st>() + 1; f.tabB = e.sh->tabB; f.tabH = e.sh->tabH; f.is_id = d_id.as<int>(); f.count = 1;
         run_finalize(s, f);
-        int id = 0; rt_d2h(&id, d_id.p, sizeof(int), s); rt_d2h(&bad[k0], d_bad.as<int>() + k0, sizeof(int) * (k1 - k0), s); rt_sync(s);
+        int id = 0; rt_d2h(&id, d_id.p, sizeof(int), s); rt_d2h(&bad[k0], d_bad.as<int>() + k0, sizeof(int) * (k1 - k0), s);
+        rlc_tap::range tr;
+        if (tap) { tr.scal.resize(T); rt_d2h(tr.scal.data(), d_scal.p, sizeof(sc_st) * T, s); rt_d2h(&tr.sB[0], d_sum.p, sizeof(sc_st), s); rt_d2h(&tr.sH[0], d_sum.as<sc_st>() + 1, sizeof(sc_st), s); }
+        rt_sync(s);
         bool ok = id == 1; for (size_t k = k0; k < k1; k++) ok = ok && !bad[k];
         if (!ok) { all = 0; if (failed) failed->push_back({i0, i0 + r}); }
+        if (tap) { tr.i0 = i0; tr.n = r; tr.c = pl.c; tr.wbits = a.wbits; tr.is_id[0] = id; tr.bad.assign(&bad[k0], &bad[k0] + (k1 - k0)); tap->ranges.push_back(std::move(tr)); }
     }
+    if (tap) tap->held = all;
     return all;
 }
 // verdicts of the rand / square-rand proofs of N elements in updates of `group` elements each (group = 0: one update): d_res = (all valid, format
 // error) per update, initialised to (1, 0) by the caller -- exactly what k_sigma_verify gives.  Calls of at least 256 elements go through the
 // batched check first; every update a failed range touches is then checked element by element (k_sigma_verify), each update at most once.
+// tap (test hook): the batched check also runs below 256 elements.
 static void sigma_verify_groups(rofl_engine &e, cudaStream_t s, int kind, const uint8_t *d_proofs, const uint8_t *d_commits, size_t N, const uint8_t seed[32],
-                                size_t group, int *d_res) {
+                                size_t group, int *d_res, rlc_tap *tap = nullptr) {
     if (!N) return;
     if (!group) group = N;
     const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
     void *tk = rt_prof_begin(PROF_SQUARE, s);
     std::vector<std::pair<size_t, size_t>> failed;
-    if (N < 256) failed.push_back({0, N});
-    else sigma_verify_rlc(e, s, kind, d_proofs, d_commits, N, seed, group, &failed);
+    if (N < 256 && !tap) failed.push_back({0, N});
+    else sigma_verify_rlc(e, s, kind, d_proofs, d_commits, N, seed, group, &failed, tap);
     size_t next = 0;                                       // first update not yet checked element by element
     for (const auto &rg : failed) {
         const size_t k0 = std::max(next, rg.first / group), k1 = (rg.second - 1) / group + 1;

@@ -998,7 +998,7 @@ KERNEL void LB(128, 1) k_sq_rlc_scalars(sq_rlc_args a) {
         uint32_t kw[8], w[16];
         for (int k = 0; k < 8; k++) kw[k] = (uint32_t)key[4 * k] | ((uint32_t)key[4 * k + 1] << 8) | ((uint32_t)key[4 * k + 2] << 16) | ((uint32_t)key[4 * k + 3] << 24);
         chacha20_block_words(w, kw, 0);
-        // weights of wbits = c * ceil(125 / c) - 1 bits (125 .. 134) for the MSM's window width c: their top window then holds c - 1 uniform bits and the
+        // weights of wbits = c * ceil(126 / c) - 1 bits (125 .. 134, engine.cuh rlc_wbits) for the MSM's window width c: their top window then holds c - 1 uniform bits and the
         // recoding never carries out of it.  (With 128-bit weights at c = 16 half of all short scalars got the digit +1 in the window above -- ONE bucket
         // with millions of points, seconds of serial additions; at other widths the few-bit top window had the same effect on a smaller scale.)
         sc rho, sig; sc_0(rho); sc_0(sig);
