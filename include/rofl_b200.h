@@ -257,7 +257,7 @@ int rofl_debug_verify_weights(rofl_ctx *, const uint8_t *proofs, size_t proof_le
  *   ranges: per range of elements (client group for family 3) 8 int64: i0, n, MSM window width c, weight bits wbits (0 for family 3: 128-bit rho_k),
  *     is_id of output 0 and 1 (-1: no such output), index of its first scalar in scalars32, index of its first flag in bad;
  *   scalars32: the MSM scalars of every range in term order; coef32: per range sB[0], sB[1], sH[0], sH[1] as given to k_finalize (zero where unused);
- *   bad: per range, the bad flags of the clients it touches (family 0: the one format flag word);
+ *   bad: per range, the bad flags of the clients it touches;
  *   verdicts: per client, what the public batch call returns for it (1 / 0 / -1; family 3 as rofl_crp_verify).
  *   cap / cnt: capacities of ranges, scalars32, bad, and what the call produced.
  * returns 1 = every range's combination held and nothing was malformed, 0 = not, ROFL_ERR_ARGS (also when a capacity is short: cnt tells the need) */

@@ -204,7 +204,7 @@ extern "C" int rofl_l2_verify(rofl_ctx *c, const uint8_t *proof, size_t plen, co
 static int sigma_prove_host(rofl_ctx *c, int kind, const float *v, const uint8_t *vc, const uint8_t *r1, const uint8_t *r2, size_t D, int n_bits, int frac, const uint8_t seed[32],
                             uint8_t *proofs, uint8_t *commits) {
     if (!D) return 0;
-    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    const size_t pw = 32 * sigma_kind_of(kind).pw, cw = 32 * sigma_kind_of(kind).cw;
     lane_guard lg(c->e); cudaStream_t s = lg.s();
     staged_in dv(v, 4 * D, s), dvc(vc, vc ? 32 * D : 0, s), d1(r1, 32 * D, s), d2(r2, r2 ? 32 * D : 0, s); dev_buf dp(pw * D, s), dc(cw * D, s);
     int rc = engine_sigma_prove(c->e, kind, dv.b.as<float>(), vc ? dvc.b.as<uint8_t>() : nullptr, d1.b.as<uint8_t>(), r2 ? d2.b.as<uint8_t>() : nullptr, D, n_bits, frac, seed, dp.as<uint8_t>(), dc.as<uint8_t>());
@@ -214,7 +214,7 @@ static int sigma_prove_host(rofl_ctx *c, int kind, const float *v, const uint8_t
 }
 static int sigma_verify_host(rofl_ctx *c, int kind, const uint8_t *proofs, const uint8_t *commits, size_t D) {
     if (!D) return 1;
-    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    const size_t pw = 32 * sigma_kind_of(kind).pw, cw = 32 * sigma_kind_of(kind).cw;
     lane_guard lg(c->e);
     staged_in dp(proofs, pw * D, lg.s()), dc(commits, cw * D, lg.s());
     return engine_sigma_verify(c->e, kind, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D);
@@ -516,7 +516,7 @@ extern "C" int rofl_enc_l2_compressed_verify_batch(rofl_ctx *c, size_t n_clients
     rt_memset(dbad.p, 0, sizeof(int) * K, s); rt_h2d(dres.p, res.data(), sizeof(int) * 2 * K, s);
     LAUNCH(k_validate_points, dim3((unsigned)((3 * D * K + 127) / 128)), dim3(128), s, de.b.as<uint8_t>(), (size_t)32, (size_t)0, 3 * D * K, dbad.as<int>(), 3 * D);
     LAUNCH(k_split96, dim3((unsigned)((D * K + 255) / 256)), dim3(256), s, dL.as<uint8_t>(), dSc.as<uint8_t>(), dCsq.as<uint8_t>(), de.b.as<uint8_t>(), D * K);
-    square_verify_groups(c->e, s, dsp.b.as<uint8_t>(), dSc.as<uint8_t>(), D * K, D, dres.as<int>());     // all K x D square proofs in one batched check, else element by element
+    sigma_verify_groups(c->e, s, 0, dsp.b.as<uint8_t>(), dSc.as<uint8_t>(), D * K, nullptr, D, dres.as<int>());   // all K x D square proofs in one batched check, else element by element
     // sum_i c_sq,i per client (params.rs:267)
     const int nb = (int)std::max<size_t>(1, std::min<size_t>(64, (D + 127) / 128));
     dev_buf dpart(sizeof(p3_st) * nb * K, s), dbad2(sizeof(int) * K, s), dsum(32 * K, s);
@@ -575,7 +575,7 @@ static int sigma_verify_batch_host(rofl_ctx *c, int kind, size_t K, const uint8_
     if (!K) return 0;
     if (!D) { for (size_t k = 0; k < K; k++) out[k] = 1; return 0; }
     if (!proofs || !commits || !seed) return ROFL_ERR_ARGS;
-    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    const size_t pw = 32 * sigma_kind_of(kind).pw, cw = 32 * sigma_kind_of(kind).cw;
     lane_guard lg(c->e); cudaStream_t s = lg.s();
     staged_in dp(proofs, pw * D * K, s), dc(commits, cw * D * K, s); dev_buf dres(2 * sizeof(int) * K, s);
     std::vector<int> res(2 * K);
@@ -669,14 +669,16 @@ extern "C" int rofl_debug_ts_absorb(rofl_ctx *c, const uint8_t *V32, size_t m, i
     return (memcmp(t.st, got.st, sizeof(t.st)) || t.pos != got.pos || t.pos_begin != got.pos_begin) ? 1 : 0;
     API_CATCH
 }
-// the batched square-proof check alone (engine.cuh, square_verify_rlc): 1 = the random linear combination over all D proofs holds and every element is
-// well-formed, 0 = it does not (rofl_square_verify then decides element by element).  proofs D x 160, commits D x 64, host buffers.
+// the batched square-proof check alone (engine.cuh, sigma_verify_rlc kind 0): 1 = the random linear combination over all D proofs holds and every
+// element is well-formed, 0 = it does not or D is below the size threshold (rofl_square_verify then decides element by element).  proofs D x 160,
+// commits D x 64, host buffers.
 extern "C" int rofl_debug_square_rlc(rofl_ctx *c, const uint8_t *proofs, const uint8_t *commits, size_t D) {
     API_TRY
     if (!D) return ROFL_ERR_ARGS;
+    if (D < SIGMA_RLC_MIN) return 0;
     lane_guard lg(c->e); cudaStream_t s = lg.s();
     staged_in dp(proofs, 160 * D, s), dc(commits, 64 * D, s);
-    return square_verify_rlc(c->e, s, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D);
+    return sigma_verify_rlc(c->e, s, 0, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D, nullptr);
     API_CATCH
 }
 // the batched compressed-rand-proof check alone (engine.cuh, engine_crp_verify_batch): 1 = the combination over all K proofs held and no proof is
@@ -694,15 +696,15 @@ extern "C" int rofl_debug_crp_rlc(rofl_ctx *c, size_t n_clients, const uint8_t *
 extern "C" int rofl_debug_sigma_rlc(rofl_ctx *c, int kind, size_t n_elems, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32]) {
     API_TRY
     if ((kind != 1 && kind != 2) || !n_elems || !proofs || !commits || !seed) return ROFL_ERR_ARGS;
-    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    const size_t pw = 32 * sigma_kind_of(kind).pw, cw = 32 * sigma_kind_of(kind).cw;
     lane_guard lg(c->e); cudaStream_t s = lg.s();
     staged_in dp(proofs, pw * n_elems, s), dc(commits, cw * n_elems, s);
     return sigma_verify_rlc(c->e, s, kind, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), n_elems, seed);
     API_CATCH
 }
-// the terms of one batched check, copied from the buffers of its production code (engine.cuh rlc_tap) and derived by nothing here: family 0 the square
-// proofs (square_verify_groups), 1 / 2 the rand / square-rand proofs (sigma_verify_groups), both over n_clients updates of D elements and below their size
-// thresholds too, 3 the compressed rand proofs of n_clients clients of D pairs (engine_crp_verify_batch; commits = the pairs).  See include/rofl_b200.h.
+// the terms of one batched check, copied from the buffers of its production code (engine.cuh rlc_tap) and derived by nothing here: family 0 / 1 / 2
+// the square / rand / square-rand proofs (sigma_verify_groups, that kind) over n_clients updates of D elements and below its size threshold too,
+// 3 the compressed rand proofs of n_clients clients of D pairs (engine_crp_verify_batch; commits = the pairs).  See include/rofl_b200.h.
 extern "C" int rofl_debug_rlc_terms(rofl_ctx *c, int family, size_t n_clients, size_t D, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32],
                                     uint8_t *root32, uint8_t *chal32, int64_t *ranges, uint8_t *scalars32, uint8_t *coef32, int *bad, int *verdicts,
                                     const size_t cap[3], size_t cnt[3]) {
@@ -716,14 +718,13 @@ extern "C" int rofl_debug_rlc_terms(rofl_ctx *c, int family, size_t n_clients, s
         const int rc = engine_crp_verify_batch(c->e, proofs, commits, nullptr, D, K, seed, verdicts, nullptr, &tap);
         if (rc < 0) return rc;
     } else {
-        const size_t pw = family == 0 ? 160 : family == 1 ? 128 : 192, cw = family == 2 ? 96 : 64;
+        const size_t pw = 32 * sigma_kind_of(family).pw, cw = 32 * sigma_kind_of(family).cw;
         lane_guard lg(c->e); cudaStream_t s = lg.s();
         staged_in dp(proofs, pw * D * K, s), dc(commits, cw * D * K, s); dev_buf dres(2 * sizeof(int) * K, s);
         std::vector<int> res(2 * K);
         for (size_t k = 0; k < K; k++) { res[2 * k] = 1; res[2 * k + 1] = 0; }
         rt_h2d(dres.p, res.data(), sizeof(int) * 2 * K, s);
-        if (family == 0) square_verify_groups(c->e, s, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D * K, D, dres.as<int>(), &tap);
-        else sigma_verify_groups(c->e, s, family, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D * K, seed, D, dres.as<int>(), &tap);
+        sigma_verify_groups(c->e, s, family, dp.b.as<uint8_t>(), dc.b.as<uint8_t>(), D * K, seed, D, dres.as<int>(), &tap);
         rt_d2h(res.data(), dres.p, sizeof(int) * 2 * K, s); rt_sync(s);
         for (size_t k = 0; k < K; k++) verdicts[k] = res[2 * k + 1] ? -1 : res[2 * k] ? 1 : 0;
     }

@@ -25,7 +25,8 @@
 enum { ROFL_ERR_BITSIZE_ = -7 };          // include/rofl_b200.h ROFL_ERR_BITSIZE
 enum { DOM_RANGE_PROVE = 1, DOM_RANGE_VERIFY = 2, DOM_SQUARE = 3, DOM_L2_PROVE = 4, DOM_L2_VERIFY = 5, DOM_CRP = 6, DOM_RND_VEC = 7, DOM_RANDPROOF = 8, DOM_SQUARE_RAND = 9,
        DOM_CRP_BATCH = 0x62707263 /* "crpb" as LE32: the weights of engine_crp_verify_batch */,
-       DOM_RP_RLC = 0x6c727072 /* "rprl": the weights of the batched rand-proof check (sigma_verify_rlc, kind 1) */,
+       DOM_SQ_RLC = 0x6c727173 /* "sqrl": the weights of the batched square-proof check (sigma_verify_rlc, kind 0) */,
+       DOM_RP_RLC = 0x6c727072 /* "rprl": the same for rand proofs (kind 1) */,
        DOM_SRP_RLC = 0x6c727273 /* "srrl": the same for square-rand proofs (kind 2) */ };
 enum { PROF_FOLD = 0, PROF_MSM = 1, PROF_COMMIT = 2, PROF_SQUARE = 3, PROF_RTMSM = 4, PROF_TAIL = 5, PROF_FRZ = 6, PROF_SLOTS = 8 };
 
@@ -81,7 +82,7 @@ struct rofl_engine {
     int ts_host_m = 8192;                 // chunks with more commitments than this absorb them on the host (absorb_commitments)
     int rt_per = 2;                       // table-MSM terms per thread and block: short blocks let the other groups' small kernels in quickly
     double rt_mem_frac = 0.45;            // tables may take this fraction of the free device memory
-    size_t sigma_rlc_terms = (size_t)1 << 24;      // MSM terms per range of the batched rand / square-rand proof check (sigma_verify_rlc)
+    size_t sigma_rlc_terms = (size_t)1 << 24;      // MSM terms per range of the batched rand / square-rand proof check (sigma_verify_rlc; not square proofs)
     size_t crp_batch_terms = (size_t)1 << 24;      // MSM terms per client group of the batched compressed-rand-proof check (crp_batch)
 };
 static thread_local lane *tl_lane = nullptr; static thread_local rofl_engine *tl_lane_engine = nullptr; static thread_local int tl_lane_depth = 0;
@@ -1046,7 +1047,8 @@ static int engine_l2_verify(rofl_engine &e, const uint8_t *h_proof, size_t plen,
 }
 
 // =============================================================================================================================
-// square_proof_vec::create_l2rangeproof_vec_existing / verify_l2rangeproof_vec (square_proof_vec/mod.rs:19-75,130-160); device pointers
+// square_proof_vec::create_l2rangeproof_vec_existing (square_proof_vec/mod.rs:19-75); device pointers.  The verify (engine_square_verify) follows
+// the batched check it uses, sigma_verify_groups
 // =============================================================================================================================
 static int engine_square_prove(rofl_engine &e, const float *d_values, const uint8_t *d_value_com, const uint8_t *d_r1, const uint8_t *d_r2, size_t D,
                                int n_bits, int frac, const uint8_t seed[32], uint8_t *d_proofs, uint8_t *d_commits) {
@@ -1067,7 +1069,7 @@ static int engine_square_prove(rofl_engine &e, const float *d_values, const uint
     return 0;
 }
 // bits of the batched checks' weights for an MSM of window width c: the smallest c * w - 1 >= 125 (125 .. 134 for c = 3 .. 16), so that the top
-// window holds c - 1 uniform bits and the signed recoding never carries out of it (kernels.cuh k_sq_rlc_scalars).  Not c * ceil(125 / c) - 1:
+// window holds c - 1 uniform bits and the signed recoding never carries out of it (kernels.cuh k_sigma_rlc_scalars).  Not c * ceil(125 / c) - 1:
 // that is 124 at c = 5, the width msm_plan_for picks for 157 .. 521 terms (small calls and the last range of a long one).
 static inline int rlc_wbits(int c) { return c * ((126 + c - 1) / c) - 1; }
 // Test hook (rofl_debug_rlc_terms): copies of what a batched check computed, taken from the buffers it already has.  The checks take a nullable
@@ -1077,73 +1079,10 @@ struct rlc_tap {
         size_t i0 = 0, n = 0; int c = 0, wbits = 0;          // elements (clients for the compressed rand proofs) [i0, i0 + n), MSM window width, weight bits
         int is_id[2] = {-1, -1};                             // k_finalize's identity test per output (-1: no such output)
         std::vector<sc_st> scal; sc_st sB[2] = {}, sH[2] = {};   // MSM scalars in term order, fixed-base coefficients as given to k_finalize
-        std::vector<int> bad;                                // bad flags of the clients the range touches (square proofs: the one flag word)
+        std::vector<int> bad;                                // bad flags of the clients the range touches
     };
     uint8_t root[32] = {}; std::vector<sc_st> chal; std::vector<range> ranges; int held = 0;
 };
-// All D square proofs of a call in ONE random linear combination (kernels.cuh, k_sq_rlc_*): 1 = every proof valid and well-formed, 0 = ask the
-// per-element kernel (the combination failed or some element is malformed: the exact verdict, per update, comes from k_square_verify).
-// tap (test hook): also runs below the size threshold and without ROFL_SQ_RLC.
-static int square_verify_rlc(rofl_engine &e, cudaStream_t s, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D, rlc_tap *tap = nullptr) {
-    static const int on = getenv("ROFL_SQ_RLC") ? atoi(getenv("ROFL_SQ_RLC")) : 1;
-    if ((!tap && (!on || D < 256)) || 4 * D > 0x7fffffffu) return 0;
-    const unsigned nb = (unsigned)((D + 127) / 128);
-    const size_t n1 = (D + 63) / 64, n2 = (n1 + 63) / 64;
-    dev_buf d_dig(32 * D, s), d_chal(sizeof(sc_st) * D, s), d_scal(sizeof(sc_st) * 4 * D, s), d_part(sizeof(sc_st) * 2 * nb, s), d_pts(sizeof(p3_st) * 4 * D, s);
-    dev_buf d_l1(32 * n1, s), d_l2(32 * n2, s), d_flags(sizeof(int), s), d_sum(sizeof(sc_st) * 2, s), d_id(sizeof(int), s);
-    rt_memset(d_flags.p, 0, sizeof(int), s);
-    sq_rlc_args a = {}; a.proofs = d_proofs; a.commits = d_commits; a.D = D; a.digest = d_dig.as<uint8_t>(); a.chal = d_chal.as<sc_st>(); a.scal = d_scal.as<sc_st>();
-    a.partial = d_part.as<sc_st>(); a.pts = d_pts.as<p3_st>(); a.flags = d_flags.as<int>();
-    LAUNCH(k_sq_rlc_prep, dim3(nb), dim3(128), s, a);
-    const uint8_t *cur = d_dig.as<uint8_t>(); size_t n = D; uint8_t *bufs[2] = {d_l1.as<uint8_t>(), d_l2.as<uint8_t>()}; int which = 0;
-    do {                                                   // hash tree, 64 digests per node
-        const size_t nn = (n + 63) / 64;
-        LAUNCH(k_hash_tree, dim3((unsigned)((nn + 127) / 128)), dim3(128), s, bufs[which], cur, n);
-        cur = bufs[which]; which ^= 1; n = nn;
-    } while (n > 1);
-    a.root = cur;
-    const msm_plan pl = msm_plan_for(4 * D, 1, 2048);
-    a.wbits = rlc_wbits(pl.c);
-    LAUNCH_COOP(k_sq_rlc_scalars, dim3(nb), dim3(128), s, a);
-    LAUNCH_COOP(k_sc_sum, dim3(1), dim3(256), s, d_sum.as<sc_st>(), d_part.as<sc_st>(), (int)nb, 2);
-    LAUNCH(k_sq_rlc_points, dim3((unsigned)((4 * D + 127) / 128)), dim3(128), s, a);
-    dev_buf d_win(sizeof(p3_st) * pl.out_count(1), s);
-    msm_args m = {}; m.v[0].scalars = d_scal.as<sc_st>(); m.split = 1; m.T = (uint32_t)(4 * D); m.scalar_stride = (uint32_t)(4 * D); m.nseg = 1; m.out = d_win.as<p3_st>();
-    m.v[0].seg[0] = mk_seg(d_pts.p, (uint32_t)(4 * D), 0, 1);
-    run_msm(e, s, m, pl, 1);
-    finalize_args f = {}; fin_windows(f, d_win.as<p3_st>(), pl); f.sBa = d_sum.as<sc_st>(); f.sHa = d_sum.as<sc_st>() + 1; f.tabB = e.sh->tabB; f.tabH = e.sh->tabH; f.is_id = d_id.as<int>(); f.count = 1;
-    run_finalize(s, f);
-    int flags = 0, id = 0; rt_d2h(&flags, d_flags.p, sizeof(int), s); rt_d2h(&id, d_id.p, sizeof(int), s);
-    rlc_tap::range r;
-    if (tap) {
-        r.n = D; r.c = pl.c; r.wbits = a.wbits; r.scal.resize(4 * D); tap->chal.resize(D);
-        rt_d2h(tap->root, cur, 32, s); rt_d2h(tap->chal.data(), d_chal.p, sizeof(sc_st) * D, s); rt_d2h(r.scal.data(), d_scal.p, sizeof(sc_st) * 4 * D, s);
-        rt_d2h(&r.sB[0], d_sum.p, sizeof(sc_st), s); rt_d2h(&r.sH[0], d_sum.as<sc_st>() + 1, sizeof(sc_st), s);
-    }
-    rt_sync(s);
-    const int held = (flags == 0 && id == 1) ? 1 : 0;
-    if (tap) { r.is_id[0] = id; r.bad = {flags}; tap->ranges.push_back(std::move(r)); tap->held = held; }
-    return held;
-}
-// verdicts of the square proofs of `D` elements in updates of `group` elements each (group = 0: one update): d_res = (all valid, format error) per
-// update, initialised to (1, 0) by the caller.  The batched check first; the per-element kernel only when it does not hold.
-static void square_verify_groups(rofl_engine &e, cudaStream_t s, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D, size_t group, int *d_res,
-                                 rlc_tap *tap = nullptr) {
-    void *tk = rt_prof_begin(PROF_SQUARE, s);
-    if (square_verify_rlc(e, s, d_proofs, d_commits, D, tap) != 1)
-        LAUNCH(k_square_verify, dim3((unsigned)((D + 127) / 128)), dim3(128), s, d_proofs, d_commits, D, e.sh->tabB, e.sh->tabH, d_res, group);
-    rt_prof_end(PROF_SQUARE, tk, s);
-}
-static int engine_square_verify(rofl_engine &e, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D) {
-    if (D == 0) return 1;
-    lane_guard lg(e);
-    cudaStream_t s = lg.s();
-    dev_buf d_res(2 * sizeof(int), s); int init[2] = {1, 0}; rt_h2d(d_res.p, init, sizeof(init), s);
-    square_verify_groups(e, s, d_proofs, d_commits, D, 0, d_res.as<int>());
-    int res[2]; rt_d2h(res, d_res.p, sizeof(res), s); rt_sync(s);
-    if (res[1]) return -1;
-    return res[0] ? 1 : 0;
-}
 
 // =============================================================================================================================
 // compressed_rand_proof::CompressedRandProof::{helper_prove, helper_prove_existing, helper_verify} (compressed_rand_proof/mod.rs:134-158)
@@ -1438,22 +1377,30 @@ static int engine_sigma_verify(rofl_engine &e, int kind, const uint8_t *d_proofs
     return res[0] ? 1 : 0;
 }
 
-// All N rand proofs (kind 1) or square-rand proofs (kind 2) of a call, in updates of `group` elements, in random linear combinations
-// (kernels.cuh, k_sigma_rlc_*): the weights come from one hash tree over all N elements; the elements are then checked in ranges of at most
-// e.sigma_rlc_terms MSM terms (4 or 6 per element), one MSM and one k_finalize per range.  A range may start or end inside an update.
-// failed (nullable) receives the element ranges [i0, i1) whose check did not hold or that touch an update with a malformed element.
-// Returns 1 when every range held and no element is malformed, else 0.  The caller holds a lane; s is its stream.  tap: the test hook's copies (rlc_tap)
+// calls of fewer elements go straight to the per-element kernel (sigma_verify_groups; rofl_debug_square_rlc answers 0 for them)
+#define SIGMA_RLC_MIN 256
+// All N square proofs (kind 0), rand proofs (kind 1) or square-rand proofs (kind 2) of a call, in updates of `group` elements, in random linear
+// combinations (kernels.cuh, k_sigma_rlc_*): the weights come from one hash tree over all N elements; the elements are then checked in ranges of
+// at most e.sigma_rlc_terms MSM terms (np per element, sigma_kind_of), one MSM and one k_finalize per range.  A range may start or end inside an
+// update.  Square proofs are checked in ONE range over the whole call, whose MSM's window width sets their weights' width; a call of more than
+// 2^31 - 1 of their terms is left to the per-element kernel whole.
+// seed: part of every key but kind 0's (nullable there).  failed (nullable) receives the element ranges [i0, i1) whose check did not hold or that
+// touch an update with a malformed element.  Returns 1 when every range held and no element is malformed, else 0.  The caller holds a lane; s is
+// its stream.  tap: the test hook's copies (rlc_tap)
 static int sigma_verify_rlc(rofl_engine &e, cudaStream_t s, int kind, const uint8_t *d_proofs, const uint8_t *d_commits, size_t N, const uint8_t seed[32],
                             size_t group = 0, std::vector<std::pair<size_t, size_t>> *failed = nullptr, rlc_tap *tap = nullptr) {
     if (!group) group = N;
-    const size_t np = kind == 1 ? 4 : 6, K = (N + group - 1) / group;
-    const size_t R = std::max<size_t>(1, std::min(e.sigma_rlc_terms, CRP_BATCH_TERMS) / np);          // elements per range
+    const sigma_kind sk = sigma_kind_of(kind);
+    const size_t np = sk.np, K = (N + group - 1) / group;
+    if (kind == 0 && np * N > 0x7fffffffu) { if (failed) failed->push_back({0, N}); return 0; }
+    const size_t R = kind == 0 ? N : std::max<size_t>(1, std::min(e.sigma_rlc_terms, CRP_BATCH_TERMS) / np);          // elements per range
     const size_t n1 = (N + 63) / 64, n2 = (n1 + 63) / 64, rmax = std::min(R, N), nbmax = (rmax + 127) / 128;
     dev_buf d_dig(32 * N, s), d_chal(sizeof(sc_st) * N, s), d_l1(32 * n1, s), d_l2(32 * n2, s), d_bad(sizeof(int) * K, s);
     dev_buf d_scal(sizeof(sc_st) * np * rmax, s), d_part(sizeof(sc_st) * 2 * nbmax, s), d_pts(sizeof(p3_st) * np * rmax, s), d_sum(sizeof(sc_st) * 2, s), d_id(sizeof(int), s);
     rt_memset(d_bad.p, 0, sizeof(int) * K, s);
-    sigma_rlc_args a = {}; a.kind = kind; a.proofs = d_proofs; a.commits = d_commits; a.N = N; a.group = group; a.tag = kind == 1 ? DOM_RP_RLC : DOM_SRP_RLC;
-    memcpy(a.seed, seed, 32);
+    static const uint32_t tags[3] = {DOM_SQ_RLC, DOM_RP_RLC, DOM_SRP_RLC};
+    sigma_rlc_args a = {}; a.kind = kind; a.proofs = d_proofs; a.commits = d_commits; a.N = N; a.group = group; a.tag = tags[kind];
+    if (sk.seeded) memcpy(a.seed, seed, 32);
     a.digest = d_dig.as<uint8_t>(); a.chal = d_chal.as<sc_st>(); a.scal = d_scal.as<sc_st>(); a.partial = d_part.as<sc_st>(); a.pts = d_pts.as<p3_st>(); a.bad = d_bad.as<int>();
     LAUNCH(k_sigma_rlc_prep, dim3((unsigned)((N + 127) / 128)), dim3(128), s, a);
     const uint8_t *cur = d_dig.as<uint8_t>(); size_t n = N; uint8_t *bufs[2] = {d_l1.as<uint8_t>(), d_l2.as<uint8_t>()}; int which = 0;
@@ -1491,28 +1438,43 @@ static int sigma_verify_rlc(rofl_engine &e, cudaStream_t s, int kind, const uint
     if (tap) tap->held = all;
     return all;
 }
-// verdicts of the rand / square-rand proofs of N elements in updates of `group` elements each (group = 0: one update): d_res = (all valid, format
-// error) per update, initialised to (1, 0) by the caller -- exactly what k_sigma_verify gives.  Calls of at least 256 elements go through the
-// batched check first; every update a failed range touches is then checked element by element (k_sigma_verify), each update at most once.
-// tap (test hook): the batched check also runs below 256 elements.
+// verdicts of the square / rand / square-rand proofs (kind 0 / 1 / 2) of N elements in updates of `group` elements each (group = 0: one update):
+// d_res = (all valid, format error) per update, initialised to (1, 0) by the caller -- exactly what the per-element kernel (k_square_verify for
+// kind 0, else k_sigma_verify) gives.  Calls of at least SIGMA_RLC_MIN elements go through the batched check first; every update a failed range
+// touches is then checked element by element, each update at most once.  tap (test hook): the batched check also runs below SIGMA_RLC_MIN.
 static void sigma_verify_groups(rofl_engine &e, cudaStream_t s, int kind, const uint8_t *d_proofs, const uint8_t *d_commits, size_t N, const uint8_t seed[32],
                                 size_t group, int *d_res, rlc_tap *tap = nullptr) {
     if (!N) return;
     if (!group) group = N;
-    const size_t pw = kind == 1 ? 128 : 192, cw = kind == 1 ? 64 : 96;
+    const sigma_kind sk = sigma_kind_of(kind);
+    const size_t pw = 32 * sk.pw, cw = 32 * sk.cw;
     void *tk = rt_prof_begin(PROF_SQUARE, s);
     std::vector<std::pair<size_t, size_t>> failed;
-    if (N < 256 && !tap) failed.push_back({0, N});
+    if (N < SIGMA_RLC_MIN && !tap) failed.push_back({0, N});
     else sigma_verify_rlc(e, s, kind, d_proofs, d_commits, N, seed, group, &failed, tap);
     size_t next = 0;                                       // first update not yet checked element by element
     for (const auto &rg : failed) {
         const size_t k0 = std::max(next, rg.first / group), k1 = (rg.second - 1) / group + 1;
         if (k0 >= k1) continue;
         const size_t j0 = k0 * group, n = std::min(N, k1 * group) - j0;
-        LAUNCH(k_sigma_verify, dim3((unsigned)((n + 127) / 128)), dim3(128), s, kind, d_proofs + pw * j0, d_commits + cw * j0, n, e.sh->tabB, e.sh->tabH, d_res + 2 * k0, group);
+        const dim3 g((unsigned)((n + 127) / 128));
+        if (kind == 0) LAUNCH(k_square_verify, g, dim3(128), s, d_proofs + pw * j0, d_commits + cw * j0, n, e.sh->tabB, e.sh->tabH, d_res + 2 * k0, group);
+        else LAUNCH(k_sigma_verify, g, dim3(128), s, kind, d_proofs + pw * j0, d_commits + cw * j0, n, e.sh->tabB, e.sh->tabH, d_res + 2 * k0, group);
         next = k1;
     }
     rt_prof_end(PROF_SQUARE, tk, s);
+}
+
+// square_proof_vec::verify_l2rangeproof_vec (square_proof_vec/mod.rs:130-160): the square proofs of one update, kind 0 of the batched check
+static int engine_square_verify(rofl_engine &e, const uint8_t *d_proofs, const uint8_t *d_commits, size_t D) {
+    if (D == 0) return 1;
+    lane_guard lg(e);
+    cudaStream_t s = lg.s();
+    dev_buf d_res(2 * sizeof(int), s); int init[2] = {1, 0}; rt_h2d(d_res.p, init, sizeof(init), s);
+    sigma_verify_groups(e, s, 0, d_proofs, d_commits, D, nullptr, 0, d_res.as<int>());
+    int res[2]; rt_d2h(res, d_res.p, sizeof(res), s); rt_sync(s);
+    if (res[1]) return -1;
+    return res[0] ? 1 : 0;
 }
 
 // sum of D compressed points -> compressed (device in, host out); -4 if one does not decode

@@ -945,100 +945,6 @@ KERNEL void LB(128, 1) k_square_verify(const uint8_t *proofs, const uint8_t *com
 KLAUNCH(k_square_verify, false, (const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result, size_t group), (proofs, commits, D, tabB, tabH, result, group))
 #endif
 
-// ---- the same verdict for ALL square proofs of a call with ONE random linear combination (square_proof/mod.rs:77-112 checks, per element,
-//        z_m B + z_r1 H == C'_l + c C_l          and          z_m C_l + z_r2 H == C'_sq + c C_sq ):
-//   sum_i rho_i [first] + sigma_i [second]  <=>
-//   sum_i [ rho_i C'_l,i + (rho_i c_i - sigma_i z_m,i) C_l,i + sigma_i C'_sq,i + sigma_i c_i C_sq,i ] - (sum rho_i z_m,i) B - (sum rho_i z_r1,i + sigma_i z_r2,i) H == 0
-//   with ~128-bit weights (rho_i, sigma_i) = ChaCha20(SHA3-256(root | "sqrl" | D | i)), root = a hash tree (leaves and inner nodes tagged) over SHA3-256(commitments_i | proof_i) of every
-//   element: the weights are Fiat-Shamir outputs over ALL proofs of the call.  One MSM over 4 D points replaces, per element, two fixed-base and two
-//   variable-base scalar multiplications (~7 100 field multiplications -> ~1 700 incl. the four decompressions).  A failing combination (or any
-//   malformed element) sends the caller to k_square_verify for the exact per-update verdicts.
-//   k_sq_rlc_prep:    format checks, challenge c_i, digest_i                         (one thread per element)
-//   k_hash_tree:      out[j] = SHA3-256(in[64 j .. 64 j + 63])                        (levels until one digest is left)
-//   k_sq_rlc_scalars: weights, the four point scalars of the element, block sums of the B and H scalars
-//   k_sq_rlc_points:  the 4 D points, extended coordinates                           (one thread per point)
-struct sq_rlc_args { const uint8_t *proofs, *commits; size_t D; uint8_t *digest; sc_st *chal; const uint8_t *root; sc_st *scal, *partial; p3_st *pts; int *flags; int wbits; };
-#ifdef KG_SQUARE
-KERNEL void LB(128, 1) k_sq_rlc_prep(sq_rlc_args a) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.D) return;
-    uint8_t buf[224];
-    ld_bytes32(buf, a.commits + 64 * i); ld_bytes32(buf + 32, a.commits + 64 * i + 32);
-    for (int k = 0; k < 5; k++) ld_bytes32(buf + 64 + 32 * k, a.proofs + 160 * i + 32 * k);
-    sc z; bool ok = true;
-    for (int k = 0; k < 3; k++) { sc_frombytes(z, buf + 128 + 32 * k); ok = ok && sc_is_canonical(z); }
-    if (!ok) atomicOr(a.flags, 1);
-    sc c; sq_transcript_challenge(c, buf, buf + 32, buf + 64, buf + 96);
-    st_sc(a.chal + i, c);
-    // leaf of the hash tree: tag 0x00 (inner nodes absorb 0x01 first, so that no element's bytes can pass for a node of the tree)
-    uint8_t dg[32]; { sponge sp; sponge_init(sp, 136); const uint8_t tag = 0x00; sponge_absorb(sp, &tag, 1); sponge_absorb(sp, buf, 224); sponge_finish(sp, 0x06); sponge_squeeze(sp, dg, 32); }
-    st_bytes32(a.digest + 32 * i, dg);
-}
-KLAUNCH(k_sq_rlc_prep, false, (sq_rlc_args a), (a))
-KERNEL void LB(128, 1) k_hash_tree(uint8_t *out, const uint8_t *in, size_t n) {
-    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x, lo = 64 * j;
-    if (lo >= n) return;
-    const size_t cnt = n - lo < 64 ? n - lo : 64;
-    sponge sp; sponge_init(sp, 136);
-    { const uint8_t tag = 0x01; sponge_absorb(sp, &tag, 1); }
-    for (size_t k = 0; k < cnt; k++) { uint8_t d[32]; ld_bytes32(d, in + 32 * (lo + k)); sponge_absorb(sp, d, 32); }
-    sponge_finish(sp, 0x06);
-    uint8_t o[32]; sponge_squeeze(sp, o, 32); st_bytes32(out + 32 * j, o);
-}
-KLAUNCH(k_hash_tree, false, (uint8_t *out, const uint8_t *in, size_t n), (out, in, n))
-KERNEL void LB(128, 1) k_sq_rlc_scalars(sq_rlc_args a) {
-    __shared__ sc_st buf[128];
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; const int tid = threadIdx.x;
-    sc sB, sH; sc_0(sB); sc_0(sH);
-    if (i < a.D) {
-        uint8_t kb[52], key[32]; ld_bytes32(kb, a.root);
-        kb[32] = 's'; kb[33] = 'q'; kb[34] = 'r'; kb[35] = 'l';
-        for (int k = 0; k < 8; k++) { kb[36 + k] = (uint8_t)((uint64_t)a.D >> (8 * k)); kb[44 + k] = (uint8_t)((uint64_t)i >> (8 * k)); }
-        sha3_256(key, kb, 52);
-        uint32_t kw[8], w[16];
-        for (int k = 0; k < 8; k++) kw[k] = (uint32_t)key[4 * k] | ((uint32_t)key[4 * k + 1] << 8) | ((uint32_t)key[4 * k + 2] << 16) | ((uint32_t)key[4 * k + 3] << 24);
-        chacha20_block_words(w, kw, 0);
-        // weights of wbits = c * ceil(126 / c) - 1 bits (125 .. 134, engine.cuh rlc_wbits) for the MSM's window width c: their top window then holds c - 1 uniform bits and the
-        // recoding never carries out of it.  (With 128-bit weights at c = 16 half of all short scalars got the digit +1 in the window above -- ONE bucket
-        // with millions of points, seconds of serial additions; at other widths the few-bit top window had the same effect on a smaller scale.)
-        sc rho, sig; sc_0(rho); sc_0(sig);
-        for (int k = 0; k < 5; k++) { rho.v[k] = w[k]; sig.v[k] = w[5 + k]; }
-        { const int full = a.wbits >> 5, rem = a.wbits & 31;
-          for (int k = 0; k < 5; k++) { const uint32_t m = k < full ? 0xffffffffu : (k == full ? ((1u << rem) - 1u) : 0u); rho.v[k] &= m; sig.v[k] &= m; } }
-        uint8_t zb[32]; sc zm, zr1, zr2, c, t, u;
-        ld_bytes32(zb, a.proofs + 160 * i + 64); sc_frombytes(zm, zb);
-        ld_bytes32(zb, a.proofs + 160 * i + 96); sc_frombytes(zr1, zb);
-        ld_bytes32(zb, a.proofs + 160 * i + 128); sc_frombytes(zr2, zb);
-        ld_sc(c, a.chal + i);
-        sc_st *o = a.scal + 4 * i;
-        // (the whole combination is negated so that the 128-bit weights stay SHORT scalars: their upper windows are zero digits and are skipped.  Negated
-        //  weights l - rho share their upper 125 bits: every term fell into the same bucket of the upper windows and one thread added millions of points.)
-        st_sc(o, rho);                                                             // C'_l:  rho
-        sc_mul(t, rho, c); sc_mul(u, sig, zm); sc_sub(t, t, u); st_sc(o + 1, t);   // C_l:   rho c - sigma z_m
-        st_sc(o + 2, sig);                                                         // C'_sq: sigma
-        sc_mul(t, sig, c); st_sc(o + 3, t);                                        // C_sq:  sigma c
-        sc_mul(sB, rho, zm); sc_neg(sB, sB);                                       // B:     -rho z_m
-        sc_mul(t, rho, zr1); sc_mul(u, sig, zr2); sc_add(sH, t, u); sc_neg(sH, sH); // H:     -(rho z_r1 + sigma z_r2)
-    }
-    block_sum_sc(sB, buf, tid, 128);
-    if (tid == 0) st_sc(a.partial + 2 * (size_t)blockIdx.x, sB);
-    block_sum_sc(sH, buf, tid, 128);
-    if (tid == 0) st_sc(a.partial + 2 * (size_t)blockIdx.x + 1, sH);
-}
-KLAUNCH(k_sq_rlc_scalars, true, (sq_rlc_args a), (a))
-KERNEL void LB(128, 2) k_sq_rlc_points(sq_rlc_args a) {
-    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 4 * a.D) return;
-    const size_t i = t >> 2; const int w = (int)(t & 3);
-    const uint8_t *src = w == 0 ? a.proofs + 160 * i : w == 1 ? a.commits + 64 * i : w == 2 ? a.proofs + 160 * i + 32 : a.commits + 64 * i + 32;
-    uint8_t enc[32]; ld_bytes32(enc, src);
-    ge_p3 P;
-    if (!ge_decompress(P, enc)) { atomicOr(a.flags, 1); ge_p3_0(P); }
-    st_p3(a.pts + t, P);
-}
-KLAUNCH(k_sq_rlc_points, false, (sq_rlc_args a), (a))
-#endif
-
 // the un-optimised encodings' per-element proofs (enc types 2 and 3): same shape as K8, one thread per element.
 //   kind 1 = RandProof (pair 64 B, proof 128 B), kind 2 = SquareRandProof (commitments 96 B, proof 192 B)
 struct sigma_args {
@@ -1080,23 +986,36 @@ KLAUNCH(k_sigma_verify, false, (int kind, const uint8_t *proofs, const uint8_t *
         (kind, proofs, commits, D, tabB, tabH, result, group))
 #endif
 
-// ---- the same verdict for ALL rand proofs (kind 1) or square-rand proofs (kind 2) of a call with ONE random linear combination per range of
-//        elements (engine.cuh, sigma_verify_groups).  Per element, kind 1 checks (rand_verify_one)
-//          z_m B + z_r H == C'_L + c L          z_r B == C'_R + c R
-//        and kind 2 (square_rand_verify_one) additionally            z_m L + z_r2 H == C'_sq + c C_sq       (z_r = z_r1).
-//   Weighted by rho_i, sigma_i (and tau_i) and negated, the sum over the elements of a range is one MSM plus two fixed-base terms:
-//     kind 1:  sum_i rho C'_L + rho c L + sigma C'_R + sigma c R                                          - (sum rho z_m + sigma z_r) B - (sum rho z_r) H == 0
-//     kind 2:  sum_i rho C'_L + (rho c - tau z_m) L + sigma C'_R + sigma c R + tau C'_sq + tau c C_sq     - (sum rho z_m + sigma z_r1) B - (sum rho z_r1 + tau z_r2) H == 0
-//   Weights: key_i = SHA3-256(root | seed | tag | LE64 N | LE64 i) over the N elements of the call, root = the hash tree (k_hash_tree) over
-//   leaf_i = SHA3-256(0x00 | commitments_i | proof_i); one ChaCha20 block of key_i gives rho = words 0..4, sigma = 5..9, tau = 10..14, each masked
-//   to wbits bits.  They stay short and positive: the signs live in the fixed-base coefficients only (see k_sq_rlc_scalars).
+// ---- the same verdict for ALL square proofs (kind 0), rand proofs (kind 1) or square-rand proofs (kind 2) of a call with ONE random linear
+//        combination per range of elements (engine.cuh, sigma_verify_groups).  Per element, every kind checks the L equation, kind 1 and kind 2
+//        the R equation, kind 0 and kind 2 the square equation (square_verify_one, rand_verify_one, square_rand_verify_one; z_r = z_r1, and
+//        L = C_l for a square proof):
+//          L:  z_m B + z_r H == C'_L + c L          R:  z_r B == C'_R + c R          square:  z_m L + z_r2 H == C'_sq + c C_sq
+//   Weighted by a_i (L), b_i (R) and q_i (square) and negated, the sum over the elements of a range is one MSM plus two fixed-base terms:
+//     kind 0:  sum_i a C'_l + (a c - q z_m) C_l + q C'_sq + q c C_sq                                   - (sum a z_m) B - (sum a z_r1 + q z_r2) H == 0
+//     kind 1:  sum_i a C'_L + a c L + b C'_R + b c R                                                     - (sum a z_m + b z_r) B - (sum a z_r) H == 0
+//     kind 2:  sum_i a C'_L + (a c - q z_m) L + b C'_R + b c R + q C'_sq + q c C_sq                    - (sum a z_m + b z_r1) B - (sum a z_r1 + q z_r2) H == 0
+//   Weights: key_i = SHA3-256(root | seed | tag | LE64 N | LE64 i) over the N elements of the call (kind 0: no seed), root = the hash tree
+//   (k_hash_tree) over leaf_i = SHA3-256(0x00 | commitments_i | proof_i); one ChaCha20 block of key_i gives the weights of the equations the kind
+//   checks, in the order a, b, q, from words 0..4, 5..9, 10..14 (kind 0: a = 0..4, q = 5..9), each masked to wbits bits.  They stay short and
+//   positive, so that their upper windows are zero digits the MSM skips: the signs live in the fixed-base coefficients only.  (Negated weights
+//   l - w share their upper 125 bits: every term fell into the same bucket of the upper windows and one thread added millions of points.)
+//   For square proofs one MSM over 4 N points replaces, per element, two fixed-base and two variable-base scalar multiplications (~7 100 field
+//   multiplications -> ~1 700 incl. the four decompressions).
 //   A malformed element (non-canonical response, undecodable point) sets the bad flag of its update (element i belongs to update i / group).
 //   k_sigma_rlc_prep:    format checks, challenge c_i, leaf digest_i                         (one thread per element of the call)
-//   k_hash_tree:         the tree above
-//   k_sigma_rlc_scalars: weights, the 4 / 6 point scalars of the element, block sums of the B and H scalars      (elements [i0, i0 + n))
-//   k_sigma_rlc_points:  the 4 / 6 points of each element of the range                       (one thread per point)
-//   Point (and scalar) w of element i, w < 2 * kind + 2: even w from the proof, odd w from the commitments, word w / 2 of each:
-//     C'_L, L, C'_R, R (, C'_sq, C_sq)
+//   k_hash_tree:         out[j] = SHA3-256(0x01 | in[64 j .. 64 j + 63])                    (levels until one digest is left)
+//   k_sigma_rlc_scalars: weights, the np point scalars of the element, block sums of the B and H scalars         (elements [i0, i0 + n))
+//   k_sigma_rlc_points:  the np points of each element of the range                          (one thread per point)
+// The layout of one element of each kind, in 32-byte words, and the equations it checks besides L.  Its np MSM points (and scalars) are, in this
+// order, C'_L, L (, C'_R, R) (, C'_sq, C_sq): even ones from the proof, odd ones from the commitments, word w / 2 of each; the responses
+// z_m, z_r (, z_r2) are the proof's words np / 2 .. pw - 1.
+struct sigma_kind { int cw, pw, np; bool req, sqeq, seeded; };
+HD constexpr sigma_kind sigma_kind_of(int kind) {
+    return kind == 0 ? sigma_kind{2, 5, 4, false, true, false}       // square proof:      C_l, C_sq      | C'_l, C'_sq, z_m, z_r1, z_r2
+         : kind == 1 ? sigma_kind{2, 4, 4, true, false, true}        // rand proof:        L, R           | C'_L, C'_R, z_m, z_r
+         :             sigma_kind{3, 6, 6, true, true, true};        // square-rand proof: L, R, C_sq     | C'_L, C'_R, C'_sq, z_m, z_r1, z_r2
+}
 struct sigma_rlc_args {
     int kind; const uint8_t *proofs, *commits; size_t N, group, i0, n; uint32_t tag; uint8_t seed[32];
     uint8_t *digest; sc_st *chal; const uint8_t *root; sc_st *scal, *partial; p3_st *pts; int *bad; int wbits;
@@ -1105,61 +1024,86 @@ struct sigma_rlc_args {
 KERNEL void LB(128, 1) k_sigma_rlc_prep(sigma_rlc_args a) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.N) return;
-    const int pw = a.kind == 1 ? 4 : 6, cw = a.kind == 1 ? 2 : 3;
+    const sigma_kind sk = sigma_kind_of(a.kind);
     uint8_t buf[288];                                                              // commitments | proof
-    for (int k = 0; k < cw; k++) ld_bytes32(buf + 32 * k, a.commits + 32 * (cw * i + k));
-    for (int k = 0; k < pw; k++) ld_bytes32(buf + 32 * (cw + k), a.proofs + 32 * (pw * i + k));
-    const uint8_t *com = buf, *proof = buf + 32 * cw;
+    for (int k = 0; k < sk.cw; k++) ld_bytes32(buf + 32 * k, a.commits + 32 * (sk.cw * i + k));
+    for (int k = 0; k < sk.pw; k++) ld_bytes32(buf + 32 * (sk.cw + k), a.proofs + 32 * (sk.pw * i + k));
+    const uint8_t *com = buf, *proof = buf + 32 * sk.cw;
     sc z; bool ok = true;
-    for (int k = pw / 2; k < pw; k++) { sc_frombytes(z, proof + 32 * k); ok = ok && sc_is_canonical(z); }
+    for (int k = sk.np / 2; k < sk.pw; k++) { sc_frombytes(z, proof + 32 * k); ok = ok && sc_is_canonical(z); }
     if (!ok) atomicOr(a.bad + i / a.group, 1);
     sc c;
-    if (a.kind == 1) rp_transcript_challenge(c, com, proof); else srp_transcript_challenge(c, com, proof);
+    if (a.kind == 0) sq_transcript_challenge(c, com, com + 32, proof, proof + 32);
+    else if (a.kind == 1) rp_transcript_challenge(c, com, proof);
+    else srp_transcript_challenge(c, com, proof);
     st_sc(a.chal + i, c);
-    uint8_t dg[32]; { sponge sp; sponge_init(sp, 136); const uint8_t tag = 0x00; sponge_absorb(sp, &tag, 1); sponge_absorb(sp, buf, 32 * (cw + pw)); sponge_finish(sp, 0x06); sponge_squeeze(sp, dg, 32); }
+    // leaf of the hash tree: tag 0x00 (inner nodes absorb 0x01 first, so that no element's bytes can pass for a node of the tree)
+    uint8_t dg[32]; { sponge sp; sponge_init(sp, 136); const uint8_t tag = 0x00; sponge_absorb(sp, &tag, 1); sponge_absorb(sp, buf, 32 * (sk.cw + sk.pw)); sponge_finish(sp, 0x06); sponge_squeeze(sp, dg, 32); }
     st_bytes32(a.digest + 32 * i, dg);
 }
 KLAUNCH(k_sigma_rlc_prep, false, (sigma_rlc_args a), (a))
+KERNEL void LB(128, 1) k_hash_tree(uint8_t *out, const uint8_t *in, size_t n) {
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x, lo = 64 * j;
+    if (lo >= n) return;
+    const size_t cnt = n - lo < 64 ? n - lo : 64;
+    sponge sp; sponge_init(sp, 136);
+    { const uint8_t tag = 0x01; sponge_absorb(sp, &tag, 1); }
+    for (size_t k = 0; k < cnt; k++) { uint8_t d[32]; ld_bytes32(d, in + 32 * (lo + k)); sponge_absorb(sp, d, 32); }
+    sponge_finish(sp, 0x06);
+    uint8_t o[32]; sponge_squeeze(sp, o, 32); st_bytes32(out + 32 * j, o);
+}
+KLAUNCH(k_hash_tree, false, (uint8_t *out, const uint8_t *in, size_t n), (out, in, n))
 KERNEL void LB(128, 1) k_sigma_rlc_scalars(sigma_rlc_args a) {
     __shared__ sc_st buf[128];
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; const int tid = threadIdx.x;
     sc sB, sH; sc_0(sB); sc_0(sH);
     if (t < a.n) {
         const size_t i = a.i0 + t;
-        const int pw = a.kind == 1 ? 4 : 6;
+        const sigma_kind sk = sigma_kind_of(a.kind);
         uint8_t kb[84], key[32]; ld_bytes32(kb, a.root);
-        for (int k = 0; k < 32; k++) kb[32 + k] = a.seed[k];
-        for (int k = 0; k < 4; k++) kb[64 + k] = (uint8_t)(a.tag >> (8 * k));
-        for (int k = 0; k < 8; k++) { kb[68 + k] = (uint8_t)((uint64_t)a.N >> (8 * k)); kb[76 + k] = (uint8_t)((uint64_t)i >> (8 * k)); }
-        sha3_256(key, kb, 84);
+        int kt = 32;                                                               // where the tag goes: after the seed, if the kind has one
+        if (sk.seeded) { for (int k = 0; k < 32; k++) kb[32 + k] = a.seed[k]; kt = 64; }
+        for (int k = 0; k < 4; k++) kb[kt + k] = (uint8_t)(a.tag >> (8 * k));
+        for (int k = 0; k < 8; k++) { kb[kt + 4 + k] = (uint8_t)((uint64_t)a.N >> (8 * k)); kb[kt + 12 + k] = (uint8_t)((uint64_t)i >> (8 * k)); }
+        sha3_256(key, kb, kt + 20);
         uint32_t kw[8], w[16];
         for (int k = 0; k < 8; k++) kw[k] = (uint32_t)key[4 * k] | ((uint32_t)key[4 * k + 1] << 8) | ((uint32_t)key[4 * k + 2] << 16) | ((uint32_t)key[4 * k + 3] << 24);
         chacha20_block_words(w, kw, 0);
-        sc rho, sig, tau; sc_0(rho); sc_0(sig); sc_0(tau);
-        for (int k = 0; k < 5; k++) { rho.v[k] = w[k]; sig.v[k] = w[5 + k]; tau.v[k] = w[10 + k]; }
+        // weights of wbits = c * ceil(126 / c) - 1 bits (125 .. 134, engine.cuh rlc_wbits) for the MSM's window width c: their top window then holds c - 1 uniform bits and the
+        // recoding never carries out of it.  (With 128-bit weights at c = 16 half of all short scalars got the digit +1 in the window above -- ONE bucket
+        // with millions of points, seconds of serial additions; at other widths the few-bit top window had the same effect on a smaller scale.)
+        sc wa, wb, wq; sc_0(wa); sc_0(wb); sc_0(wq);                             // weights of the L, R and square equations (0 where the kind has none)
+        for (int k = 0; k < 5; k++) {
+            wa.v[k] = w[k];
+            if (sk.req) wb.v[k] = w[5 + k];
+            if (sk.sqeq) wq.v[k] = sk.req ? w[10 + k] : w[5 + k];
+        }
         { const int full = a.wbits >> 5, rem = a.wbits & 31;
-          for (int k = 0; k < 5; k++) { const uint32_t m = k < full ? 0xffffffffu : (k == full ? ((1u << rem) - 1u) : 0u); rho.v[k] &= m; sig.v[k] &= m; tau.v[k] &= m; } }
+          for (int k = 0; k < 5; k++) { const uint32_t m = k < full ? 0xffffffffu : (k == full ? ((1u << rem) - 1u) : 0u); wa.v[k] &= m; wb.v[k] &= m; wq.v[k] &= m; } }
         uint8_t zb[32]; sc zm, zr, c, u, v;
-        const uint8_t *pf = a.proofs + 32 * (pw * i + pw / 2);                     // z_m | z_r (| z_r2)
+        const uint8_t *pf = a.proofs + 32 * (sk.pw * i + sk.np / 2);               // z_m | z_r (| z_r2)
         ld_bytes32(zb, pf); sc_frombytes(zm, zb);
         ld_bytes32(zb, pf + 32); sc_frombytes(zr, zb);
         ld_sc(c, a.chal + i);
-        sc_st *o = a.scal + pw * t;
-        st_sc(o, rho);                                                             // C'_L: rho
-        sc_mul(u, rho, c);
-        st_sc(o + 2, sig);                                                         // C'_R: sigma
-        sc_mul(v, sig, c); st_sc(o + 3, v);                                        // R:    sigma c
-        sc_mul(sB, rho, zm); sc_mul(v, sig, zr); sc_add(sB, sB, v); sc_neg(sB, sB); // B:    -(rho z_m + sigma z_r)
-        sc_mul(sH, rho, zr);                                                       // H:    -(rho z_r (+ tau z_r2))
-        if (a.kind == 2) {
-            sc zr2; ld_bytes32(zb, pf + 64); sc_frombytes(zr2, zb);
-            sc_mul(v, tau, zm); sc_sub(u, u, v);                                   // L:    rho c - tau z_m
-            st_sc(o + 4, tau);                                                     // C'_sq: tau
-            sc_mul(v, tau, c); st_sc(o + 5, v);                                    // C_sq: tau c
-            sc_mul(v, tau, zr2); sc_add(sH, sH, v);
+        sc_st *o = a.scal + sk.np * t;
+        st_sc(o, wa);                                                              // C'_L:  a
+        sc_mul(u, wa, c);                                                          // L:     a c (- q z_m)
+        sc_mul(sB, wa, zm);                                                        // B:     -(a z_m (+ b z_r))
+        sc_mul(sH, wa, zr);                                                        // H:     -(a z_r (+ q z_r2))
+        if (sk.req) {
+            st_sc(o + 2, wb);                                                      // C'_R:  b
+            sc_mul(v, wb, c); st_sc(o + 3, v);                                     // R:     b c
+            sc_mul(v, wb, zr); sc_add(sB, sB, v);
         }
-        st_sc(o + 1, u);                                                           // L:    rho c (kind 1)
-        sc_neg(sH, sH);
+        if (sk.sqeq) {
+            sc zr2; ld_bytes32(zb, pf + 64); sc_frombytes(zr2, zb);
+            sc_mul(v, wq, zm); sc_sub(u, u, v);
+            st_sc(o + sk.np - 2, wq);                                              // C'_sq: q
+            sc_mul(v, wq, c); st_sc(o + sk.np - 1, v);                             // C_sq:  q c
+            sc_mul(v, wq, zr2); sc_add(sH, sH, v);
+        }
+        st_sc(o + 1, u);
+        sc_neg(sB, sB); sc_neg(sH, sH);
     }
     block_sum_sc(sB, buf, tid, 128);
     if (tid == 0) st_sc(a.partial + 2 * (size_t)blockIdx.x, sB);
@@ -1169,10 +1113,10 @@ KERNEL void LB(128, 1) k_sigma_rlc_scalars(sigma_rlc_args a) {
 KLAUNCH(k_sigma_rlc_scalars, true, (sigma_rlc_args a), (a))
 KERNEL void LB(128, 2) k_sigma_rlc_points(sigma_rlc_args a) {
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int pw = a.kind == 1 ? 4 : 6, cw = a.kind == 1 ? 2 : 3;
-    if (t >= (size_t)pw * a.n) return;
-    const size_t i = a.i0 + t / pw; const int w = (int)(t % pw);
-    const uint8_t *src = (w & 1) ? a.commits + 32 * (cw * i + (w >> 1)) : a.proofs + 32 * (pw * i + (w >> 1));
+    const sigma_kind sk = sigma_kind_of(a.kind);
+    if (t >= (size_t)sk.np * a.n) return;
+    const size_t i = a.i0 + t / sk.np; const int w = (int)(t % sk.np);
+    const uint8_t *src = (w & 1) ? a.commits + 32 * (sk.cw * i + (w >> 1)) : a.proofs + 32 * (sk.pw * i + (w >> 1));
     uint8_t enc[32]; ld_bytes32(enc, src);
     ge_p3 P;
     if (!ge_decompress(P, enc)) { atomicOr(a.bad + i / a.group, 1); ge_p3_0(P); }
@@ -1472,10 +1416,7 @@ void launch_k_sigma_rlc_prep(dim3 g_, dim3 b_, cudaStream_t s_, sigma_rlc_args a
 void launch_k_sigma_rlc_scalars(dim3 g_, dim3 b_, cudaStream_t s_, sigma_rlc_args a);
 void launch_k_sigma_rlc_points(dim3 g_, dim3 b_, cudaStream_t s_, sigma_rlc_args a);
 void launch_k_square_verify(dim3 g_, dim3 b_, cudaStream_t s_, const uint8_t *proofs, const uint8_t *commits, size_t D, const niels_st *tabB, const niels_st *tabH, int *result, size_t group);
-void launch_k_sq_rlc_prep(dim3 g_, dim3 b_, cudaStream_t s_, sq_rlc_args a);
 void launch_k_hash_tree(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const uint8_t *in, size_t n);
-void launch_k_sq_rlc_scalars(dim3 g_, dim3 b_, cudaStream_t s_, sq_rlc_args a);
-void launch_k_sq_rlc_points(dim3 g_, dim3 b_, cudaStream_t s_, sq_rlc_args a);
 void launch_k_aggregate(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const uint8_t *pts, size_t n_clients, size_t D, int init_base, int *bad);
 void launch_k_bsgs_build(dim3 g_, dim3 b_, cudaStream_t s_, unsigned long long *keys, uint32_t *vals, uint32_t cap, uint32_t m, const niels_st *tabB, int *distinct);
 void launch_k_bsgs_solve(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out_sc, float *out_f32, const uint8_t *pts, size_t D, const unsigned long long *keys, const uint32_t *vals, uint32_t cap, uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags);

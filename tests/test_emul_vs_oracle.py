@@ -106,7 +106,7 @@ def test_tail_tables_in_batches_of_chunks(api, oracle):
 
 
 def test_square_proofs_batched_check(api, oracle):
-    """All square proofs of a call in ONE random linear combination (k_sq_rlc_*): it holds for honest proofs, fails when any element is tampered with
+    """All square proofs of a call in ONE random linear combination (k_sigma_rlc_*, kind 0): it holds for honest proofs, fails when any element is tampered with
     (commitment, proof point or response) or malformed, and rofl_square_verify's verdict stays the reference's in every case."""
     rng = np.random.default_rng(15)
     D = 260

@@ -2,7 +2,7 @@
 
 A batched check accepts a whole round when ONE weighted sum is the identity, so it is only sound while every weight is an unpredictable function
 of every byte it checks.  Verdict tests cannot see that: honest rounds pass under any weights, one tampered element fails under any nonzero
-weight.  Here the production code of each check (square_verify_rlc, sigma_verify_rlc, crp_batch_end, through the test hook rofl_debug_rlc_terms,
+weight.  Here the production code of each check (sigma_verify_rlc for families 0-2, crp_batch_end, through the test hook rofl_debug_rlc_terms,
 which copies what those functions computed and derives nothing) is compared with this file's reference -- hashlib SHA3-256, the oracle's ChaCha20
 and challenges (its own radix-2^51 transcript code), Python integers mod l -- for the root, every challenge, every MSM scalar, every fixed-base
 coefficient and the weight width; then the weights are shown to move with every byte of a record and with the seed, and an adaptive forgery that
@@ -161,7 +161,7 @@ def weights_of(blocks, wbits):
 
 
 def sigma_terms(fam, w, z, c):
-    """the MSM scalars of one element and its B / H contributions (before negation), kernels.cuh k_sq_rlc_scalars / k_sigma_rlc_scalars"""
+    """the MSM scalars of one element and its B / H contributions (before negation), kernels.cuh k_sigma_rlc_scalars"""
     rho, sig, tau = w
     if fam == 0:
         zm, zr1, zr2 = z
