@@ -46,6 +46,7 @@ enum {
     ROFL_ERR_DLOG = -5,                /* no discrete log in range (bsgs32.rs:69-70 unwrap panic)                         */
     ROFL_ERR_TOO_MANY = -6,            /* more than 900 000 pairs in a compressed rand proof (the reference's label table ends there) */
     ROFL_ERR_BITSIZE = -7,             /* ProofError::InvalidBitsize (range not in {8,16,32,64}), prove and verify side   */
+    ROFL_ERR_UNBALANCED = -8,          /* an accumulated R is not B at extract (params.rs:133-138, el_gamal.rs:101-103)   */
     ROFL_ERR_NAN = -98,                /* NaN input (Fix::saturating_from_float panics)                                   */
     ROFL_ERR_PARTITION = -99,          /* n_partition gives non power-of-two chunks (range_proof_vec/mod.rs:137-140 panic) */
     ROFL_ERR_CUDA = -100               /* CUDA runtime error / no device                                                   */
@@ -230,6 +231,33 @@ int rofl_aggregate_dev(rofl_ctx *, const uint8_t *points32 /*dev*/, size_t n_cli
  *      (8 for fp8, else 16).  out_scalars32 / out_f32 may be NULL.  The table is built once per (table_size, bsgs_bits). */
 int rofl_dlog(rofl_ctx *, const uint8_t *points32, size_t D, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *out_scalars32, float *out_f32);
 int rofl_dlog_dev(rofl_ctx *, const uint8_t *points32 /*dev*/, size_t D, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *out_scalars32 /*dev*/, float *out_f32 /*dev*/);
+
+/* ---- round accumulator: EncModelParamsAccumulator (params.rs:74-148) on the device, for D elements.  Clients are added as they arrive
+ *      (accumulate_other, params.rs:81-124); the accumulated points stay in HBM between calls, O(D) state whatever the number of clients.
+ *   rec_bytes 32: Pedersen commitments (L only; pedersen_ops::add_rp_vec_vec, pedersen_ops.rs:56-69)
+ *             64: ElGamal pairs L | R (EncRange / EncRangeCompressed enc_values)
+ *             96: L | R | c_sq (EncL2 / EncL2Compressed enc_values): c_sq must decode, it is not accumulated
+ *   init_unity 1: every element starts at ElGamalPair::unity = (B, B) (params.rs:165-179, el_gamal.rs:83-88); 0: at the identity.
+ * The state (two extended points per element, one for rec_bytes 32: 256 B / 128 B) is allocated at create and never enters the scratch cache.
+ * The accumulator keeps a pointer to its context: the context must outlive it.  Calls on one accumulator from several threads are serialised
+ * by the accumulator's own mutex.  Group addition is commutative and export writes canonical encodings, so no result depends on the order
+ * of the adds or on how the clients are split over calls.  Return values: 0 / counts as stated, ROFL_ERR_ARGS for bad arguments. */
+typedef struct rofl_acc rofl_acc;
+int rofl_acc_create(rofl_ctx *, size_t D, int rec_bytes, int init_unity, rofl_acc **out);
+void rofl_acc_destroy(rofl_acc *);
+int rofl_acc_reset(rofl_acc *);                 /* back to the initial state, count 0, memory kept (the next round) */
+/* records: n_clients x D x rec_bytes, client-major.  mask (nullable): add client k only where mask[k] == 1 (the out_ok of a *_verify_batch call
+ * can be passed as it is).  out_added (nullable): per client 1 added, 0 skipped by the mask, ROFL_ERR_POINT a point of its record does not decode
+ * (then nothing of that client is added: the reference's from_bytes fails before accumulate).  Returns the number of clients added, or < 0. */
+int rofl_acc_add(rofl_acc *, const uint8_t *records, size_t n_clients, const int *mask, int *out_added);
+int rofl_acc_add_dev(rofl_acc *, const uint8_t *records /*dev*/, size_t n_clients, const int *mask /*host*/, int *out_added /*host*/);
+size_t rofl_acc_count(const rofl_acc *);        /* clients added since create / reset */
+/* the accumulated values, compressed: D x 32 (rec_bytes 32) or D x 64 (L | R) */
+int rofl_acc_export(rofl_acc *, uint8_t *out);
+/* EncModelParamsAccumulator::extract (params.rs:126-147): first every accumulated R must equal B (Ristretto equality; not checked for rec_bytes 32),
+ * else ROFL_ERR_UNBALANCED and nothing is written; then BSGS on L exactly as rofl_dlog(table_size, bsgs_bits, n_bits, frac): ROFL_ERR_DLOG when
+ * an element has no log in range (the reference's unwrap panic).  out_scalars32 (D x 32) / out_f32 (D) nullable.  The accumulator is not changed. */
+int rofl_acc_extract(rofl_acc *, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *out_scalars32, float *out_f32);
 
 /* ---- measurement hooks (bench.py): CUDA-event time per kernel family and launch counts since the last reset ------- */
 enum { ROFL_PROF_FOLD = 0, ROFL_PROF_MSM = 1, ROFL_PROF_COMMIT = 2, ROFL_PROF_SQUARE = 3 };

@@ -59,6 +59,14 @@ _SIGS = {
     "rofl_aggregate_dev": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, C.c_int, c_u8p]),
     "rofl_dlog": (C.c_int, [c_vp, c_u8p, c_sz, C.c_uint64, C.c_int, C.c_int, C.c_int, c_u8p, c_f32p]),
     "rofl_dlog_dev": (C.c_int, [c_vp, c_u8p, c_sz, C.c_uint64, C.c_int, C.c_int, C.c_int, c_u8p, c_f32p]),
+    "rofl_acc_create": (C.c_int, [c_vp, c_sz, C.c_int, C.c_int, C.POINTER(c_vp)]),
+    "rofl_acc_destroy": (None, [c_vp]),
+    "rofl_acc_reset": (C.c_int, [c_vp]),
+    "rofl_acc_add": (C.c_int, [c_vp, c_u8p, c_sz, c_vp, c_vp]),
+    "rofl_acc_add_dev": (C.c_int, [c_vp, c_u8p, c_sz, c_vp, c_vp]),
+    "rofl_acc_count": (c_sz, [c_vp]),
+    "rofl_acc_export": (C.c_int, [c_vp, c_u8p]),
+    "rofl_acc_extract": (C.c_int, [c_vp, C.c_uint64, C.c_int, C.c_int, C.c_int, c_u8p, c_f32p]),
     "rofl_prof_enable": (None, [C.c_int]),
     "rofl_prof_reset": (None, []),
     "rofl_prof_ms": (C.c_double, [C.c_int]),
@@ -519,6 +527,79 @@ class Api:
         a = _u8(pts).reshape(-1, 32); s = np.zeros_like(a); f = np.zeros(a.shape[0], np.float32)
         rc = self.lib.rofl_dlog(self.h, _ptr(a), a.shape[0], table_size, bsgs_bits, n_bits, frac, _ptr(s), _ptr(f))
         if rc <= ROFL_ERR_CUDA: raise self._err(rc)
+        return rc, s, f
+
+    def accumulator(self, D, rec_bytes, init_unity=1):
+        """A device-resident round accumulator (EncModelParamsAccumulator) of D elements over rec_bytes-wide records (32, 64 or 96)."""
+        return Accumulator(self, D, rec_bytes, init_unity)
+
+
+class Accumulator:
+    """rofl_acc: clients are added as they arrive, the sums stay on the device; extract() checks R == B and decrypts L.
+    Keep the Api (its context) alive while the accumulator is in use; close() or a with-block frees the device state."""
+
+    def __init__(self, api, D, rec_bytes, init_unity=1):
+        self.api, self.D, self.rec_bytes = api, D, rec_bytes
+        h = c_vp()
+        rc = api.lib.rofl_acc_create(api.h, D, rec_bytes, init_unity, C.byref(h))
+        if rc != 0:
+            raise api._err(rc)
+        self.h = h
+
+    def close(self):
+        if self.h:
+            self.api.lib.rofl_acc_destroy(self.h); self.h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def _mask(self, mask, K):
+        if mask is None:
+            return None
+        m = np.ascontiguousarray(mask, np.int32)
+        if m.size != K:
+            raise ValueError(f"mask has {m.size} entries for {K} clients")
+        return m
+
+    def add(self, records, mask=None):
+        """records [K, D, rec_bytes] (or [D, rec_bytes] for one client) -> out_added int32[K]: 1 added, 0 masked out, ROFL_ERR_POINT"""
+        r = _u8(records).reshape(-1, self.D, self.rec_bytes); K = r.shape[0]
+        m = self._mask(mask, K); added = np.zeros(K, np.int32)
+        rc = self.api.lib.rofl_acc_add(self.h, _ptr(r), K, _ptr(m), _ptr(added))
+        if rc < 0: raise self.api._err(rc)
+        return added
+
+    def add_dev(self, ptr, n_clients, mask=None):
+        """records already on the device (n_clients x D x rec_bytes at address ptr, e.g. a torch CUDA tensor's data_ptr()) -> out_added"""
+        m = self._mask(mask, n_clients); added = np.zeros(n_clients, np.int32)
+        rc = self.api.lib.rofl_acc_add_dev(self.h, ptr, n_clients, _ptr(m), _ptr(added))
+        if rc < 0: raise self.api._err(rc)
+        return added
+
+    @property
+    def count(self):
+        return self.api.lib.rofl_acc_count(self.h)
+
+    def reset(self):
+        """back to the initial state with count 0, the device memory kept (the next round)"""
+        rc = self.api.lib.rofl_acc_reset(self.h)
+        if rc: raise self.api._err(rc)
+
+    def export(self):
+        """-> uint8 [D, 32] (rec_bytes 32) or [D, 64] (L | R): canonical encodings of the accumulated values"""
+        o = np.zeros((self.D, 32 if self.rec_bytes == 32 else 64), np.uint8)
+        rc = self.api.lib.rofl_acc_export(self.h, _ptr(o))
+        if rc: raise self.api._err(rc)
+        return o
+
+    def extract(self, table_size=1 << 16, bsgs_bits=16, n_bits=16, frac=7):
+        """-> (rc, scalars [D, 32], f32 [D]); rc 0, ROFL_ERR_UNBALANCED (-8, an R is not B: outputs stay zero), ROFL_ERR_DLOG (-5) or ROFL_ERR_ARGS"""
+        s = np.zeros((self.D, 32), np.uint8); f = np.zeros(self.D, np.float32)
+        rc = self.api.lib.rofl_acc_extract(self.h, table_size, bsgs_bits, n_bits, frac, _ptr(s), _ptr(f))
+        if rc <= ROFL_ERR_CUDA: raise self.api._err(rc)
         return rc, s, f
 
 

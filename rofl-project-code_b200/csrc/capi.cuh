@@ -489,6 +489,66 @@ extern "C" int rofl_dlog(rofl_ctx *c, const uint8_t *pts, size_t D, uint64_t ts,
     API_CATCH
 }
 
+// ---- device-resident round accumulator (EncModelParamsAccumulator, params.rs:74-148): one mutex per accumulator serialises its calls,
+//      each call runs on a lane of the accumulator's context like every other call
+#define ACC_TRY if (!a) return ROFL_ERR_ARGS; try { rt_set_device(a->e->device); std::lock_guard<std::mutex> acc_lk_(a->mu);
+extern "C" int rofl_acc_create(rofl_ctx *c, size_t D, int rec_bytes, int init_unity, rofl_acc **out) {
+    if (out) *out = nullptr;
+    API_TRY
+    if (!out || !D || (rec_bytes != 32 && rec_bytes != 64 && rec_bytes != 96) || (init_unity != 0 && init_unity != 1)) return ROFL_ERR_ARGS;
+    *out = engine_acc_create(c->e, D, rec_bytes, init_unity);
+    return ROFL_OK;
+    API_CATCH
+}
+extern "C" void rofl_acc_destroy(rofl_acc *a) {
+    if (!a) return;
+    try { rt_set_device(a->e->device); } catch (...) {}
+    engine_acc_destroy(a);
+}
+extern "C" int rofl_acc_reset(rofl_acc *a) {
+    ACC_TRY engine_acc_reset(*a); return ROFL_OK; API_CATCH
+}
+extern "C" size_t rofl_acc_count(const rofl_acc *a) {
+    if (!a) return 0;
+    std::lock_guard<std::mutex> lk(const_cast<rofl_acc *>(a)->mu); return a->count;
+}
+extern "C" int rofl_acc_add_dev(rofl_acc *a, const uint8_t *records, size_t n_clients, const int *mask, int *out_added) {
+    ACC_TRY
+    if (!records) return ROFL_ERR_ARGS;
+    return engine_acc_add(*a, records, n_clients, mask, out_added);
+    API_CATCH
+}
+extern "C" int rofl_acc_add(rofl_acc *a, const uint8_t *records, size_t n_clients, const int *mask, int *out_added) {
+    ACC_TRY
+    if (!records) return ROFL_ERR_ARGS;
+    if (!n_clients) return 0;
+    lane_guard lg(*a->e);
+    staged_in dr(records, (size_t)a->rec_bytes * a->D * n_clients, lg.s());
+    return engine_acc_add(*a, dr.b.as<uint8_t>(), n_clients, mask, out_added);
+    API_CATCH
+}
+extern "C" int rofl_acc_export(rofl_acc *a, uint8_t *out) {
+    ACC_TRY
+    if (!out) return ROFL_ERR_ARGS;
+    lane_guard lg(*a->e); cudaStream_t s = lg.s();
+    const size_t n = 32 * a->D * a->ncols;
+    dev_buf o(n, s);
+    engine_acc_export(*a, o.as<uint8_t>());
+    rt_d2h(out, o.p, n, s); rt_sync(s);
+    return ROFL_OK;
+    API_CATCH
+}
+extern "C" int rofl_acc_extract(rofl_acc *a, uint64_t ts, int bb, int n_bits, int frac, uint8_t *osc, float *of) {
+    ACC_TRY
+    lane_guard lg(*a->e); cudaStream_t s = lg.s();
+    dev_buf o(32 * a->D, s), f(4 * a->D, s);
+    int rc = engine_acc_extract(*a, ts, bb, n_bits, frac, o.as<uint8_t>(), f.as<float>());
+    if (rc != 0 && rc != ROFL_ERR_DLOG) return rc;
+    if (osc) rt_d2h(osc, o.p, 32 * a->D, s); if (of) rt_d2h(of, f.p, 4 * a->D, s); rt_sync(s);
+    return rc;
+    API_CATCH
+}
+
 // ---- server side: all clients of a round in one call (rofl_service/src/flserver/server.rs:516-522,666-667 fans EncModelParams::verify out over a
 //      rayon pool, one task per client; on a GPU the clients share ONE batched check instead) ------------------------------------------------------
 extern "C" int rofl_range_verify_batch(rofl_ctx *c, const uint8_t *proofs, size_t plen, size_t n_proofs, const uint8_t *commits32, size_t D, size_t n_clients, int range,

@@ -1551,3 +1551,87 @@ static int engine_dlog(rofl_engine &e, const uint8_t *d_pts, size_t D, uint64_t 
     if (flags & 8) return -5;
     return 0;
 }
+
+// =============================================================================================================================
+// device-resident round accumulator: EncModelParamsAccumulator (params.rs:74-148) -- accumulate_other per arriving client, extract at
+// the round's end.  The state (ncols x D extended points, kernels.cuh K9b) is allocated once, outside the scratch cache, so `trim` and
+// table eviction never touch it.  Every call holds the accumulator's mutex and ends in a synchronise of its lane, so the next call may
+// run on another lane (stream) of the context.
+// =============================================================================================================================
+enum { ROFL_ERR_UNBALANCED_ = -8 };       // include/rofl_b200.h ROFL_ERR_UNBALANCED
+struct rofl_acc {
+    rofl_engine *e = nullptr; size_t D = 0; int rec_bytes = 0, ncols = 0, init_unity = 0; size_t count = 0;
+    p3_st *st = nullptr; std::mutex mu;
+};
+static void engine_acc_reset(rofl_acc &a) {
+    lane_guard lg(*a.e); cudaStream_t s = lg.s();
+    const size_t n = a.D * a.ncols;
+    LAUNCH(k_acc_init, dim3((unsigned)((n + 255) / 256)), dim3(256), s, a.st, n, a.init_unity);
+    rt_sync(s);
+    a.count = 0;
+}
+static rofl_acc *engine_acc_create(rofl_engine &e, size_t D, int rec_bytes, int init_unity) {
+    rofl_acc *a = new rofl_acc();
+    a->e = &e; a->D = D; a->rec_bytes = rec_bytes; a->ncols = rec_bytes == 32 ? 1 : 2; a->init_unity = init_unity ? 1 : 0;
+    try {
+        a->st = (p3_st *)rt_raw_malloc(sizeof(p3_st) * D * a->ncols);
+        engine_acc_reset(*a);
+    } catch (...) { rt_raw_free(a->st); delete a; throw; }
+    return a;
+}
+static void engine_acc_destroy(rofl_acc *a) { if (a) { rt_raw_free(a->st); delete a; } }
+// d_rec: n_clients x D x rec_bytes [dev].  Clients with mask[k] != 1 (mask may be null: all) are skipped; the points of the others are validated
+// first (one flag per client), and only clients whose every point decodes are added.  out_added[k]: 1 / 0 skipped / ROFL_ERR_POINT.  Returns the
+// number of clients added.
+static int engine_acc_add(rofl_acc &a, const uint8_t *d_rec, size_t n_clients, const int *mask, int *out_added) {
+    rofl_engine &e = *a.e;
+    lane_guard lg(e); cudaStream_t s = lg.s();
+    const size_t pts = a.rec_bytes / 32, D = a.D;
+    std::vector<int> bad(n_clients, 0);
+    dev_buf d_bad(sizeof(int) * (n_clients ? n_clients : 1), s); rt_memset(d_bad.p, 0, sizeof(int) * n_clients, s);
+    // validate each run of consecutive selected clients in one launch: the masked-out clients cost nothing
+    for (size_t k0 = 0; k0 < n_clients;) {
+        if (mask && mask[k0] != 1) { k0++; continue; }
+        size_t k1 = k0 + 1; while (k1 < n_clients && (!mask || mask[k1] == 1)) k1++;
+        const size_t np = pts * D * (k1 - k0);
+        LAUNCH(k_validate_points, dim3((unsigned)((np + 127) / 128)), dim3(128), s, d_rec + a.rec_bytes * D * k0, (size_t)32, (size_t)0, np, d_bad.as<int>() + k0, pts * D);
+        k0 = k1;
+    }
+    rt_d2h(bad.data(), d_bad.p, sizeof(int) * n_clients, s); rt_sync(s);
+    std::vector<uint32_t> acc;
+    for (size_t k = 0; k < n_clients; k++) {
+        const int r = (mask && mask[k] != 1) ? 0 : bad[k] ? -4 : 1;
+        if (r == 1) acc.push_back((uint32_t)k);
+        if (out_added) out_added[k] = r;
+    }
+    if (!acc.empty()) {
+        dev_buf d_list(sizeof(uint32_t) * acc.size(), s);
+        rt_h2d(d_list.p, acc.data(), sizeof(uint32_t) * acc.size(), s);
+        LAUNCH(k_acc_add, dim3((unsigned)((D + 127) / 128)), dim3(128), s, a.st, D, a.ncols, d_rec, (size_t)a.rec_bytes, d_list.as<uint32_t>(), (uint32_t)acc.size());
+        rt_sync(s);
+    }
+    a.count += acc.size();
+    return (int)acc.size();
+}
+// d_out: D x 32 ncols [dev], the canonical encodings of the accumulated values
+static void engine_acc_export(rofl_acc &a, uint8_t *d_out) {
+    lane_guard lg(*a.e); cudaStream_t s = lg.s();
+    const size_t n = a.D * a.ncols;
+    LAUNCH(k_acc_export, dim3((unsigned)((n + 127) / 128)), dim3(128), s, d_out, a.st, a.D, a.ncols);
+}
+// EncModelParamsAccumulator::extract: 0, ROFL_ERR_UNBALANCED (some R != B; nothing is written), -5 no discrete log in range (as engine_dlog), -2 bad table
+static int engine_acc_extract(rofl_acc &a, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *d_out_sc, float *d_out_f32) {
+    if (table_size == 0 || table_size > (1ull << 28) || bsgs_bits < 1 || bsgs_bits > 32) return -2;
+    rofl_engine &e = *a.e;
+    lane_guard lg(e); cudaStream_t s = lg.s();
+    tables_use tu(*e.sh);
+    const bsgs_entry b = engine_bsgs(e, tu, s, table_size, bsgs_bits);
+    uint64_t max_it = b.size ? (1ULL << bsgs_bits) / b.size : 0;                  // bsgs32.rs:60-62
+    dev_buf d_flags(sizeof(int), s); rt_memset(d_flags.p, 0, sizeof(int), s);
+    LAUNCH(k_acc_extract, dim3((unsigned)((a.D + 127) / 128)), dim3(128), s, d_out_sc, d_out_f32, a.st, a.D, a.ncols == 2 ? 1 : 0, b.keys, b.vals, b.cap,
+           (uint32_t)table_size, b.size, max_it, bsgs_bits, n_bits, frac, e.sh->tabB, d_flags.as<int>());
+    int flags = 0; rt_d2h(&flags, d_flags.p, sizeof(int), s); rt_sync(s);
+    if (flags & 16) return ROFL_ERR_UNBALANCED_;
+    if (flags & 8) return -5;
+    return 0;
+}

@@ -1192,13 +1192,10 @@ HD bool bsgs_lookup(uint32_t &val, const unsigned long long *keys, const uint32_
 }
 // solve_discrete_log_with_neg (bsgs32.rs:48-73): up to max_it giant steps for M, then for -M.
 //   size = distinct - 1 (get_size), mG = (m & vmask) B, result (it*size + val) & vmask; miss on both signs -> flag 8
-#ifdef KG_BSGS
-KERNEL void LB(128, 2) k_bsgs_solve(uint8_t *out_sc, float *out_f32, const uint8_t *pts, size_t D, const unsigned long long *keys, const uint32_t *vals, uint32_t cap,
-                                   uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= D) return;
-    uint8_t b[32]; ld_bytes32(b, pts + 32 * i);
-    ge_p3 M; if (!ge_decompress(M, b)) { atomicOr(flags, 4); return; }
+// Element i of a point M already in extended coordinates: shared by k_bsgs_solve (M decompressed from the wire) and k_acc_extract (M = the
+// accumulated L, resident on the device).
+DEV void bsgs_solve_point(uint8_t *out_sc, float *out_f32, size_t i, const ge_p3 &M, const unsigned long long *keys, const uint32_t *vals, uint32_t cap,
+                         uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags) {
     uint64_t vmask = (1ULL << bsgs_bits) - 1;
     ge_p3 mG; ge_p3_0(mG); { sc s; sc_from_u64(s, (uint64_t)m & vmask); fb_mul_acc(mG, tabB, s, 32); }
     int found = 0; uint64_t val = 0;
@@ -1216,7 +1213,75 @@ KERNEL void LB(128, 2) k_bsgs_solve(uint8_t *out_sc, float *out_f32, const uint8
     if (out_sc) { uint8_t o[32]; sc_tobytes(o, r); st_bytes32(out_sc + 32 * i, o); }
     if (out_f32) out_f32[i] = found ? scalar_to_f32(r, n_bits, frac) : 0.0f;
 }
+#ifdef KG_BSGS
+KERNEL void LB(128, 2) k_bsgs_solve(uint8_t *out_sc, float *out_f32, const uint8_t *pts, size_t D, const unsigned long long *keys, const uint32_t *vals, uint32_t cap,
+                                   uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= D) return;
+    uint8_t b[32]; ld_bytes32(b, pts + 32 * i);
+    ge_p3 M; if (!ge_decompress(M, b)) { atomicOr(flags, 4); return; }
+    bsgs_solve_point(out_sc, out_f32, i, M, keys, vals, cap, m, size, max_it, bsgs_bits, n_bits, frac, tabB, flags);
+}
 KLAUNCH(k_bsgs_solve, false, (uint8_t *out_sc, float *out_f32, const uint8_t *pts, size_t D, const unsigned long long *keys, const uint32_t *vals, uint32_t cap, uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags), (out_sc, out_f32, pts, D, keys, vals, cap, m, size, max_it, bsgs_bits, n_bits, frac, tabB, flags))
+#endif
+
+// ===================================================================================================================
+// K9b / K10b: device-resident round accumulator (EncModelParamsAccumulator, params.rs:74-148).  The state is `ncols` columns of
+//   D extended points, column-major: st[col * D + i] (col 0 = L, col 1 = R).  Records are the wire records of the clients
+//   (rec_bytes = 32 | 64 | 96, client-major, L at offset 0, R at 32, c_sq at 64 -- c_sq is validated by the caller, never added).
+// ===================================================================================================================
+#ifdef KG_COMMIT
+// every element at the unity (B, B) (ElGamalPair::unity, el_gamal.rs:83-88) or at the identity
+KERNEL void LB(256, 2) k_acc_init(p3_st *st, size_t n, int init_base) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    ge_p3 p; if (init_base) ge_base(p); else ge_p3_0(p);
+    st_p3(st + i, p);
+}
+KLAUNCH(k_acc_init, false, (p3_st *st, size_t n, int init_base), (st, n, init_base))
+// adds the accepted clients `clients[0 .. n_acc)` of one call: their points were all validated before (k_validate_points), so every
+// decompression here succeeds -- a client is added entirely or not at all
+KERNEL void LB(128, 2) k_acc_add(p3_st *st, size_t D, int ncols, const uint8_t *rec, size_t rec_bytes, const uint32_t *clients, uint32_t n_acc) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= D) return;
+    for (int col = 0; col < ncols; col++) {
+        ge_p3 acc; ld_p3(acc, st + col * D + i);
+        for (uint32_t c = 0; c < n_acc; c++) {
+            uint8_t b[32]; ld_bytes32(b, rec + rec_bytes * ((size_t)clients[c] * D + i) + 32 * col);
+            ge_p3 p; ge_decompress(p, b);
+            ge_add(acc, acc, p);
+        }
+        st_p3(st + col * D + i, acc);
+    }
+}
+KLAUNCH(k_acc_add, false, (p3_st *st, size_t D, int ncols, const uint8_t *rec, size_t rec_bytes, const uint32_t *clients, uint32_t n_acc), (st, D, ncols, rec, rec_bytes, clients, n_acc))
+// canonical encodings: out[i * 32 ncols + 32 col] = compress(st[col * D + i])  (D x 32 or D x 64 = L | R)
+KERNEL void LB(128, 2) k_acc_export(uint8_t *out, const p3_st *st, size_t D, int ncols) {
+    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= D * ncols) return;
+    const size_t i = t / ncols, col = t % ncols;
+    ge_p3 p; ld_p3(p, st + col * D + i);
+    uint8_t o[32]; ge_compress(o, p); st_bytes32(out + 32 * t, o);
+}
+KLAUNCH(k_acc_export, false, (uint8_t *out, const p3_st *st, size_t D, int ncols), (out, st, D, ncols))
+#endif
+#ifdef KG_BSGS
+// EncModelParamsAccumulator::extract (params.rs:126-147): R == B (Ristretto equality, el_gamal.rs:101-103) for every element when check_R,
+// else flag 16; then BSGS on the resident L exactly as k_bsgs_solve after its decompression.  Once a wrong R has been seen, later threads
+// skip their discrete log (the host returns ROFL_ERR_UNBALANCED and hands out no result).
+KERNEL void LB(128, 2) k_acc_extract(uint8_t *out_sc, float *out_f32, const p3_st *st, size_t D, int check_R, const unsigned long long *keys, const uint32_t *vals, uint32_t cap,
+                                     uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= D) return;
+    if (check_R) {
+        ge_p3 R, B; ld_p3(R, st + D + i); ge_base(B);
+        if (!ge_eq(R, B)) { atomicOr(flags, 16); return; }
+    }
+    if (*(volatile int *)flags & 16) return;
+    ge_p3 M; ld_p3(M, st + i);
+    bsgs_solve_point(out_sc, out_f32, i, M, keys, vals, cap, m, size, max_it, bsgs_bits, n_bits, frac, tabB, flags);
+}
+KLAUNCH(k_acc_extract, false, (uint8_t *out_sc, float *out_f32, const p3_st *st, size_t D, int check_R, const unsigned long long *keys, const uint32_t *vals, uint32_t cap, uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags), (out_sc, out_f32, st, D, check_R, keys, vals, cap, m, size, max_it, bsgs_bits, n_bits, frac, tabB, flags))
 #endif
 
 // K1: conversions exposed on their own (conversion32.rs:11-38, range_proof_vec/mod.rs:104-111)
@@ -1420,6 +1485,10 @@ void launch_k_hash_tree(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const u
 void launch_k_aggregate(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const uint8_t *pts, size_t n_clients, size_t D, int init_base, int *bad);
 void launch_k_bsgs_build(dim3 g_, dim3 b_, cudaStream_t s_, unsigned long long *keys, uint32_t *vals, uint32_t cap, uint32_t m, const niels_st *tabB, int *distinct);
 void launch_k_bsgs_solve(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out_sc, float *out_f32, const uint8_t *pts, size_t D, const unsigned long long *keys, const uint32_t *vals, uint32_t cap, uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags);
+void launch_k_acc_init(dim3 g_, dim3 b_, cudaStream_t s_, p3_st *st, size_t n, int init_base);
+void launch_k_acc_add(dim3 g_, dim3 b_, cudaStream_t s_, p3_st *st, size_t D, int ncols, const uint8_t *rec, size_t rec_bytes, const uint32_t *clients, uint32_t n_acc);
+void launch_k_acc_export(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const p3_st *st, size_t D, int ncols);
+void launch_k_acc_extract(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out_sc, float *out_f32, const p3_st *st, size_t D, int check_R, const unsigned long long *keys, const uint32_t *vals, uint32_t cap, uint32_t m, uint64_t size, uint64_t max_it, int bsgs_bits, int n_bits, int frac, const niels_st *tabB, int *flags);
 void launch_k_f32_to_scalar(dim3 g_, dim3 b_, cudaStream_t s_, uint8_t *out, const float *v, size_t D, int n_bits, int frac, int *flags);
 void launch_k_scalar_to_f32(dim3 g_, dim3 b_, cudaStream_t s_, float *out, const uint8_t *in, size_t D, int n_bits, int frac);
 void launch_k_l2_sums(dim3 g_, dim3 b_, cudaStream_t s_, sc_st *partial, const float *v, const uint8_t *blind, size_t D, int n_bits, int frac, int *flags);

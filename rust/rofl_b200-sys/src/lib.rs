@@ -4,6 +4,9 @@ use libc::{c_char, c_float, c_int, c_long, c_void, size_t};
 
 #[repr(C)]
 pub struct rofl_ctx { _private: [u8; 0] }
+/// device-resident round accumulator (`rofl_acc_*`); the context it was created on must outlive it
+#[repr(C)]
+pub struct rofl_acc { _private: [u8; 0] }
 
 pub const ROFL_OK: c_int = 0;
 pub const ROFL_ERR_VALUE_OUT_OF_RANGE: c_int = 2;
@@ -16,6 +19,7 @@ pub const ROFL_ERR_POINT: c_int = -4;
 pub const ROFL_ERR_DLOG: c_int = -5;
 pub const ROFL_ERR_TOO_MANY: c_int = -6;
 pub const ROFL_ERR_BITSIZE: c_int = -7;
+pub const ROFL_ERR_UNBALANCED: c_int = -8;
 pub const ROFL_ERR_NAN: c_int = -98;
 pub const ROFL_ERR_PARTITION: c_int = -99;
 pub const ROFL_ERR_CUDA: c_int = -100;
@@ -77,5 +81,13 @@ extern "C" {
                                     seed32: *const u8, out_ok: *mut c_int) -> c_int;
     pub fn rofl_aggregate(ctx: *mut rofl_ctx, points32: *const u8, n_clients: size_t, d: size_t, init_unity: c_int, out32: *mut u8) -> c_int;
     pub fn rofl_dlog(ctx: *mut rofl_ctx, points32: *const u8, d: size_t, table_size: u64, bsgs_bits: c_int, n_bits: c_int, frac: c_int, out_scalars32: *mut u8, out_f32: *mut c_float) -> c_int;
+    pub fn rofl_acc_create(ctx: *mut rofl_ctx, d: size_t, rec_bytes: c_int, init_unity: c_int, out: *mut *mut rofl_acc) -> c_int;
+    pub fn rofl_acc_destroy(acc: *mut rofl_acc);
+    pub fn rofl_acc_reset(acc: *mut rofl_acc) -> c_int;
+    pub fn rofl_acc_add(acc: *mut rofl_acc, records: *const u8, n_clients: size_t, mask: *const c_int, out_added: *mut c_int) -> c_int;
+    pub fn rofl_acc_add_dev(acc: *mut rofl_acc, records_dev: *const u8, n_clients: size_t, mask: *const c_int, out_added: *mut c_int) -> c_int;
+    pub fn rofl_acc_count(acc: *const rofl_acc) -> size_t;
+    pub fn rofl_acc_export(acc: *mut rofl_acc, out: *mut u8) -> c_int;
+    pub fn rofl_acc_extract(acc: *mut rofl_acc, table_size: u64, bsgs_bits: c_int, n_bits: c_int, frac: c_int, out_scalars32: *mut u8, out_f32: *mut c_float) -> c_int;
     pub fn rofl_ctx_stream(ctx: *mut rofl_ctx) -> *mut c_void;
 }
