@@ -228,7 +228,9 @@ int rofl_aggregate_dev(rofl_ctx *, const uint8_t *points32 /*dev*/, size_t n_cli
 
 /* ---- decryption: pedersen_ops::discrete_log_vec_table + BSGSTable (pedersen_ops.rs:47-53, bsgs32.rs:20-73;
  *      bindings32.rs:213 `extract_values`).  table_size = BSGSTable::new(m); bsgs_bits = width of BSGS_URawFix
- *      (8 for fp8, else 16).  out_scalars32 / out_f32 may be NULL.  The table is built once per (table_size, bsgs_bits). */
+ *      (8 for fp8, else 16).  out_scalars32 / out_f32 may be NULL.  The table is built once per (table_size, bsgs_bits).
+ *      ROFL_ERR_ARGS, with nothing built or written, for a table outside 1 .. 2^28 entries, bsgs_bits outside 1 .. 32 or an unsupported
+ *      fixed-point format (n_bits not in {8,16,32,64}, frac not in 0..12). */
 int rofl_dlog(rofl_ctx *, const uint8_t *points32, size_t D, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *out_scalars32, float *out_f32);
 int rofl_dlog_dev(rofl_ctx *, const uint8_t *points32 /*dev*/, size_t D, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *out_scalars32 /*dev*/, float *out_f32 /*dev*/);
 
@@ -256,7 +258,8 @@ size_t rofl_acc_count(const rofl_acc *);        /* clients added since create / 
 int rofl_acc_export(rofl_acc *, uint8_t *out);
 /* EncModelParamsAccumulator::extract (params.rs:126-147): first every accumulated R must equal B (Ristretto equality; not checked for rec_bytes 32),
  * else ROFL_ERR_UNBALANCED and nothing is written; then BSGS on L exactly as rofl_dlog(table_size, bsgs_bits, n_bits, frac): ROFL_ERR_DLOG when
- * an element has no log in range (the reference's unwrap panic).  out_scalars32 (D x 32) / out_f32 (D) nullable.  The accumulator is not changed. */
+ * an element has no log in range (the reference's unwrap panic); ROFL_ERR_ARGS, with nothing written, for a table or fixed-point format rofl_dlog
+ * refuses.  out_scalars32 (D x 32) / out_f32 (D) nullable.  The accumulator is not changed. */
 int rofl_acc_extract(rofl_acc *, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *out_scalars32, float *out_f32);
 
 /* ---- measurement hooks (bench.py): CUDA-event time per kernel family and launch counts since the last reset ------- */

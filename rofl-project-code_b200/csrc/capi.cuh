@@ -484,6 +484,7 @@ extern "C" int rofl_dlog(rofl_ctx *c, const uint8_t *pts, size_t D, uint64_t ts,
     lane_guard lg(c->e); cudaStream_t s = lg.s();
     staged_in dp(pts, 32 * D, s); dev_buf o(32 * D, s), f(4 * D, s);
     int rc = engine_dlog(c->e, dp.b.as<uint8_t>(), D, ts, bb, n_bits, frac, o.as<uint8_t>(), f.as<float>());
+    if (rc == ROFL_ERR_ARGS) return rc;
     if (osc) rt_d2h(osc, o.p, 32 * D, s); if (of) rt_d2h(of, f.p, 4 * D, s); rt_sync(s);
     return rc;
     API_CATCH

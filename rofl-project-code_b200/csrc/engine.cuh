@@ -1534,9 +1534,10 @@ static bsgs_entry engine_bsgs(rofl_engine &e, tables_use &tu, cudaStream_t s, ui
         sh.bsgs[key] = b;
     }
 }
-// returns 0, -4 undecodable point, -5 where the reference panics (no discrete log within range for either sign, bsgs32.rs:69-70)
+// returns 0, -2 bad table or fixed-point format, -4 undecodable point, -5 where the reference panics (no discrete log within range for either
+// sign, bsgs32.rs:69-70)
 static int engine_dlog(rofl_engine &e, const uint8_t *d_pts, size_t D, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *d_out_sc, float *d_out_f32) {
-    if (table_size == 0 || table_size > (1ull << 28) || bsgs_bits < 1 || bsgs_bits > 32) return -2;
+    if (!fp_ok(n_bits, frac) || table_size == 0 || table_size > (1ull << 28) || bsgs_bits < 1 || bsgs_bits > 32) return -2;
     if (D == 0) return 0;
     lane_guard lg(e);
     cudaStream_t s = lg.s();
@@ -1619,9 +1620,10 @@ static void engine_acc_export(rofl_acc &a, uint8_t *d_out) {
     const size_t n = a.D * a.ncols;
     LAUNCH(k_acc_export, dim3((unsigned)((n + 127) / 128)), dim3(128), s, d_out, a.st, a.D, a.ncols);
 }
-// EncModelParamsAccumulator::extract: 0, ROFL_ERR_UNBALANCED (some R != B; nothing is written), -5 no discrete log in range (as engine_dlog), -2 bad table
+// EncModelParamsAccumulator::extract: 0, ROFL_ERR_UNBALANCED (some R != B; nothing is written), -5 no discrete log in range (as engine_dlog),
+// -2 bad table or fixed-point format
 static int engine_acc_extract(rofl_acc &a, uint64_t table_size, int bsgs_bits, int n_bits, int frac, uint8_t *d_out_sc, float *d_out_f32) {
-    if (table_size == 0 || table_size > (1ull << 28) || bsgs_bits < 1 || bsgs_bits > 32) return -2;
+    if (!fp_ok(n_bits, frac) || table_size == 0 || table_size > (1ull << 28) || bsgs_bits < 1 || bsgs_bits > 32) return -2;
     rofl_engine &e = *a.e;
     lane_guard lg(e); cudaStream_t s = lg.s();
     tables_use tu(*e.sh);
