@@ -295,6 +295,21 @@ int rofl_debug_verify_weights(rofl_ctx *, const uint8_t *proofs, size_t proof_le
 int rofl_debug_rlc_terms(rofl_ctx *, int family, size_t n_clients, size_t D, const uint8_t *proofs, const uint8_t *commits, const uint8_t seed[32],
                          uint8_t *root32, uint8_t *chal32, int64_t *ranges, uint8_t *scalars32, uint8_t *coef32, int *bad, int *verdicts,
                          const size_t cap[3], size_t cnt[3]);
+/* the range-proof batched check (verify_chunks) of one public call, as its production code computed it (nothing is derived by the hook).
+ *   mode 0: rofl_range_verify (proofs n_proofs x plen, commits32 D x 32), or rofl_range_verify_shard when chunk_len > 0 (D = the shard's real elements);
+ *   1: rofl_range_verify_batch over n_clients updates (proofs n_clients x n_proofs x plen, commits32 n_clients x D x 32);
+ *   2: rofl_l2_verify (one proof, one commitment); 3: the L2 batch of the server calls over n_clients proofs / commitments.
+ *   verdicts: per client what the public call returns (modes 0 and 2: one value, its return code).
+ *   recs: 12 int64 per verify_chunks invocation, in call order (a failing batch is followed by its per-client re-checks): C, n, m, lgN, c_off,
+ *     domain, fixed-generator path (1 generator tables, 0 bucket MSM), its window width, identity test (1 = the equation held), index of the
+ *     record's first scalar in scalars32, its scalar count, index of its first chunk in digest32 / bad.
+ *   scalars32: per record y z x w u_0 .. u_(lgN-1) of every chunk | c_i of every chunk | rho_i | the (5 + 2 lgN)-scalar block of every chunk |
+ *     the C m commitment scalars | the C (6 + 2 lgN) proof-point scalars | g_k | h_k (2 N).  digest32 / bad: the per-chunk digest and bad flag.
+ *   cap / cnt: capacities of recs, scalars32 and digest32 / bad (chunks), and what the call produced.
+ * returns 0, or ROFL_ERR_ARGS (also when a capacity is short: cnt tells the need) */
+int rofl_debug_range_terms(rofl_ctx *, int mode, const uint8_t *proofs, size_t plen, size_t n_proofs, const uint8_t *commits32, size_t D, size_t n_clients,
+                           int range, size_t chunk_len, size_t chunk_begin, const uint8_t seed[32], int *verdicts, int64_t *recs, uint8_t *scalars32,
+                           uint8_t *digest32, int *bad, const size_t cap[3], size_t cnt[3]);
 /* the MSM front end alone (production plan / forced window width / generator tables, then k_finalize): out32[k] = sum_t s[k][t] P_t + sB[k] B + sH[k] H.
  * scalars32: n_msm x T canonical scalars; points32: T shared or n_msm x T (points_per_msm) encodings, or NULL for BulletproofGens(gen_n, T / (2 gen_n));
  * path 0 = msm_plan_for(T, n_msm, big_min), 1 = window width c with `knob` slices (c <= 8) / parts (c >= 9), 2 = generator tables.  sB32 / sH32 may be NULL.

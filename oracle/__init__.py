@@ -135,6 +135,15 @@ def range_prove(values, blind, rng, n_partition, n_bits=16, frac=7, seed=SEED0):
     proofs = np.zeros((nc, plen), np.uint8); commits = np.zeros((D, 32), np.uint8)
     rc = lib().orc_range_prove(_p(proofs), _p(commits), _p(v), _p(b), C.c_size_t(D), rng, C.c_size_t(n_partition), n_bits, frac, _p(_u8(seed, 32)))
     return rc, proofs, commits
+def range_prove_tx_bl_shifted(values, blind, rng, n_partition, shifts, n_bits=16, frac=7, seed=SEED0):
+    """range_prove with t_x_blinding of chunk c shifted by the scalar shifts[c] (32 bytes each) before it is absorbed: otherwise honest proofs
+    whose verification equations are off by exactly -c shift B_blinding (adaptive-forgery tests of the batched verifier)"""
+    v = _f32(values); D = v.size; b = _u8(blind, 32 * D)
+    Dp = next_pow2(D); nc = min(Dp, n_partition); chunk = Dp // nc
+    proofs = np.zeros((nc, rp_proof_len(rng * chunk)), np.uint8); commits = np.zeros((D, 32), np.uint8)
+    rc = lib().orc_range_prove_tx_bl_shifted(_p(proofs), _p(commits), _p(v), _p(b), C.c_size_t(D), rng, C.c_size_t(n_partition), n_bits, frac,
+                                             _p(_u8(seed, 32)), _p(_u8(shifts, 32 * nc)))
+    return rc, proofs, commits
 def range_verify(proofs, commits, rng, seed=SEED0):
     p = _u8(proofs); c = _u8(commits).reshape(-1, 32)
     p = p.reshape(p.shape[0], -1) if p.ndim > 1 else p
@@ -193,6 +202,13 @@ def srp_challenge(commits96, proof192):
     return _challenge("orc_srp_challenge", _u8(commits96, 96), _u8(proof192, 192)[:96])
 def crp_challenge(proof128, pairs):
     p = _u8(pairs).reshape(-1, 64); return _challenge("orc_crp_challenge", p, _u8(proof128, 128)[:64], C.c_size_t(p.shape[0]))
+def rp_challenges(proof, V32, n, m, label_id=0):
+    """the range-proof verifier's transcript replayed by the oracle -> (rc, [y, z, x, w, u_0 .. u_(lgN-1)] as 32-byte scalars, the 32-byte
+    "rofl-batch" digest); rc 1, or 0 when a proof point is the identity encoding (the transcript still absorbs it)"""
+    p = _u8(proof); v = _u8(V32, 32 * m); lg = (p.size // 32 - 9) // 2
+    ch = np.zeros((4 + lg, 32), np.uint8); dg = np.zeros(32, np.uint8)
+    rc = lib().orc_rp_challenges(_p(p), C.c_size_t(p.size), _p(v), n, m, label_id, _p(ch), _p(dg))
+    return rc, [bytes(x) for x in ch], dg.tobytes()
 def aggregate(pts, init=0):
     a = _u8(pts); assert a.ndim == 3 and a.shape[2] == 32
     o = np.zeros((a.shape[1], 32), np.uint8); rc = lib().orc_aggregate(_p(o), _p(a), C.c_size_t(a.shape[0]), C.c_size_t(a.shape[1]), init); assert rc == 0; return o

@@ -195,8 +195,10 @@ static inline size_t rp_proof_len(size_t N) { return 32 * (9 + 2 * (size_t)ilog2
 /* ---- RangeProof::prove_multiple_with_rng (A.3).  values < 2^n, m = power of two.
  * proof_out: rp_proof_len(n*m) bytes; V_out: m*32 bytes compressed commitments.
  * returns 0 ok, -7 invalid bitsize, -2 invalid aggregation ------------------------------------ */
-static inline int rp_prove_multiple(uint8_t *proof_out, uint8_t *V_out, const bp_gens_t *bg, const pc_gens_t *pc,
-                                    transcript *t, const uint64_t *values, const sc *blindings, int m, int n, rng_t *rng) {
+/* tx_bl_shift (nullable, tests only): added to t_x_blinding before it is absorbed -- an otherwise honest proof whose verification equation
+ * is off by exactly -c shift B_blinding (the adaptive-forgery tests of the batched verifier) */
+static inline int rp_prove_multiple_ex(uint8_t *proof_out, uint8_t *V_out, const bp_gens_t *bg, const pc_gens_t *pc,
+                                       transcript *t, const uint64_t *values, const sc *blindings, int m, int n, rng_t *rng, const sc *tx_bl_shift) {
     if (!(n == 8 || n == 16 || n == 32 || n == 64)) return -7;
     if (m <= 0 || (m & (m - 1)) || bg->n < n || bg->m < m) return -2;
     size_t N = (size_t)n * m;
@@ -270,6 +272,7 @@ static inline int rp_prove_multiple(uint8_t *proof_out, uint8_t *V_out, const bp
     }
     for (size_t k = 0; k < N; k++) { sc_muladd(&l[k], &sL[k], &x, &l0[k]); sc_muladd(&r[k], &r1[k], &x, &r0[k]); }
     sc_tobytes(o, &t_x); transcript_append(t, "t_x", o, 32); o += 32;
+    if (tx_bl_shift) sc_add(&t_x_bl, &t_x_bl, tx_bl_shift);
     sc_tobytes(o, &t_x_bl); transcript_append(t, "t_x_blinding", o, 32); o += 32;
     sc_tobytes(o, &e_bl); transcript_append(t, "e_blinding", o, 32); o += 32;
     sc w; ts_challenge(t, "w", &w);
@@ -282,6 +285,11 @@ static inline int rp_prove_multiple(uint8_t *proof_out, uint8_t *V_out, const bp
     free(G); free(H); free(l0); free(r0); free(r1); free(offset_zz); free(ms); free(mp);
     free(sL); free(sR); free(a_bl); free(s_bl); free(t1_bl); free(t2_bl);
     return 0;
+}
+
+static inline int rp_prove_multiple(uint8_t *proof_out, uint8_t *V_out, const bp_gens_t *bg, const pc_gens_t *pc,
+                                    transcript *t, const uint64_t *values, const sc *blindings, int m, int n, rng_t *rng) {
+    return rp_prove_multiple_ex(proof_out, V_out, bg, pc, t, values, blindings, m, n, rng, NULL);
 }
 
 /* ---- RangeProof::from_bytes + verify_multiple_with_rng (A.3).
@@ -367,5 +375,34 @@ static inline int rp_verify_multiple(const uint8_t *proof, size_t proof_len, con
     if (ok) { ge chk; ge_msm(&chk, ms, mp, npts); res = ge_is_identity(&chk); }
     free(ms); free(mp); free(s); free(u_sq); free(u_inv_sq);
     return res;
+}
+
+/* ---- the transcript of rp_verify_multiple alone, replayed over every point also when one is the identity encoding (the batched verifier still
+ * draws its challenges then and rejects the chunk separately).  out_chal: y z x w u_0 .. u_(lg-1), 32 bytes each; out_digest: the 32-byte
+ * "rofl-batch" challenge drawn after a and b, the per-chunk digest the batched verifier keys its weights from (DESIGN.md §2).
+ * returns 1 when every point of the proof is a non-identity encoding, 0 when one is the identity, -1 on a malformed length */
+static inline int rp_challenges(const uint8_t *proof, size_t proof_len, const uint8_t *V, transcript *t, int m, int n, uint8_t *out_chal, uint8_t out_digest[32]) {
+    if (proof_len % 32 || proof_len < 7 * 32) return -1;
+    size_t ne = proof_len / 32 - 7;
+    if (ne < 2 || (ne - 2) % 2) return -1;
+    size_t lg = (ne - 2) / 2; if (lg >= 32) return -1;
+    const uint8_t *ipp = proof + 224;
+    int ok = 1; sc ch; int q = 0;
+#define RPC_POINT(label, b) do { uint8_t z_ = 0; for (int i_ = 0; i_ < 32; i_++) z_ |= (b)[i_]; ok &= z_ != 0; transcript_append(t, label, b, 32); } while (0)
+#define RPC_CHAL(label) do { ts_challenge(t, label, &ch); sc_tobytes(out_chal + 32 * q++, &ch); } while (0)
+    transcript_append(t, "dom-sep", (const uint8_t *)"rangeproof v1", 13);
+    transcript_append_u64(t, "n", n); transcript_append_u64(t, "m", m);
+    for (int j = 0; j < m; j++) transcript_append(t, "V", V + 32 * j, 32);
+    RPC_POINT("A", proof); RPC_POINT("S", proof + 32); RPC_CHAL("y"); RPC_CHAL("z");
+    RPC_POINT("T_1", proof + 64); RPC_POINT("T_2", proof + 96); RPC_CHAL("x");
+    transcript_append(t, "t_x", proof + 128, 32); transcript_append(t, "t_x_blinding", proof + 160, 32); transcript_append(t, "e_blinding", proof + 192, 32);
+    RPC_CHAL("w");
+    transcript_append(t, "dom-sep", (const uint8_t *)"ipp v1", 6); transcript_append_u64(t, "n", (uint64_t)n * m);
+    for (size_t k = 0; k < lg; k++) { RPC_POINT("L", ipp + 64 * k); RPC_POINT("R", ipp + 64 * k + 32); RPC_CHAL("u"); }
+    transcript_append(t, "a", ipp + 64 * lg, 32); transcript_append(t, "b", ipp + 64 * lg + 32, 32);
+    transcript_challenge(t, "rofl-batch", out_digest, 32);
+#undef RPC_POINT
+#undef RPC_CHAL
+    return ok;
 }
 #endif

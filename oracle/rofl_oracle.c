@@ -178,8 +178,8 @@ EXPORT size_t orc_rp_proof_len(size_t N) { return rp_proof_len(N); }
 /* create_rangeproof (:16-102).  proofs_out: n_chunks * rp_proof_len(range*chunk) bytes, commits_out: D*32.
  * returns 0 ok, 1 WrongNumBlindingFactors (n/a here), 2 ValueOutOfRangeError, -7 InvalidBitsize,
  * -99 where the reference panics ("Should not get here": non power-of-two chunking), -2 bad fp config */
-EXPORT int orc_range_prove(uint8_t *proofs_out, uint8_t *commits_out, const float *values, const uint8_t *blind, size_t D,
-                           int range, size_t n_partition, int n_bits, int frac, const uint8_t seed[32]) {
+static int range_prove_impl(uint8_t *proofs_out, uint8_t *commits_out, const float *values, const uint8_t *blind, size_t D,
+                            int range, size_t n_partition, int n_bits, int frac, const uint8_t seed[32], const uint8_t *tx_bl_shift32) {
     if (!fp_ok(n_bits, frac) || D == 0 || range < 1 || range > n_bits) return -2;
     init_pc();
     float mx = clip_max(range, n_bits, frac), mn = -mx;
@@ -202,7 +202,9 @@ EXPORT int orc_range_prove(uint8_t *proofs_out, uint8_t *commits_out, const floa
     for (size_t c = 0; c < n_chunks; c++) {                                                      /* :75-78, helper :118-142 */
         transcript t; transcript_init(&t, "RangeProof");
         uint8_t key[32]; rng_t rng; orc_derive_key(key, seed, DOM_RANGE_PROVE, c); rng_init(&rng, key);
-        int r = rp_prove_multiple(proofs_out + plen * c, V + 32 * chunk * c, &bg, &PC, &t, vals + chunk * c, bl + chunk * c, (int)chunk, range, &rng);
+        sc shift; if (tx_bl_shift32) sc_from_bytes_mod_order(&shift, tx_bl_shift32 + 32 * c);
+        int r = rp_prove_multiple_ex(proofs_out + plen * c, V + 32 * chunk * c, &bg, &PC, &t, vals + chunk * c, bl + chunk * c, (int)chunk, range, &rng,
+                                     tx_bl_shift32 ? &shift : NULL);
         if (r) rc = r;
     }
     if (!rc) {
@@ -212,6 +214,16 @@ EXPORT int orc_range_prove(uint8_t *proofs_out, uint8_t *commits_out, const floa
     }
     bp_gens_free(&bg); free(V); free(vals); free(bl);
     return rc;
+}
+EXPORT int orc_range_prove(uint8_t *proofs_out, uint8_t *commits_out, const float *values, const uint8_t *blind, size_t D,
+                           int range, size_t n_partition, int n_bits, int frac, const uint8_t seed[32]) {
+    return range_prove_impl(proofs_out, commits_out, values, blind, D, range, n_partition, n_bits, frac, seed, NULL);
+}
+/* the same proofs with t_x_blinding of chunk c shifted by tx_bl_shift32[c] (n_chunks x 32 bytes) before it is absorbed: each chunk's
+ * verification equation is then off by exactly -c_verifier shift B_blinding (tests of the batched verifier only) */
+EXPORT int orc_range_prove_tx_bl_shifted(uint8_t *proofs_out, uint8_t *commits_out, const float *values, const uint8_t *blind, size_t D,
+                                         int range, size_t n_partition, int n_bits, int frac, const uint8_t seed[32], const uint8_t *tx_bl_shift32) {
+    return range_prove_impl(proofs_out, commits_out, values, blind, D, range, n_partition, n_bits, frac, seed, tx_bl_shift32);
 }
 /* verify_rangeproof (:149-191).  returns 1 true, 0 false, <0 error (-1 format, -7 bitsize, -3 gens length, -4 bad point) */
 EXPORT int orc_range_verify(const uint8_t *proofs, size_t proof_len, size_t n_proofs, const uint8_t *commits, size_t D,
@@ -239,6 +251,13 @@ EXPORT int orc_range_verify(const uint8_t *proofs, size_t proof_len, size_t n_pr
     }
     bp_gens_free(&bg); free(V);
     return err ? err : res;
+}
+
+/* the verifier's transcript challenges and batch digest of one range proof (bp.h rp_challenges); V32: its m commitments as the transcript sees them
+ * (shifted for L-infinity, padding = identity encodings); label_id 0 "RangeProof", 1 "L2RangeProof" */
+EXPORT int orc_rp_challenges(const uint8_t *proof, size_t proof_len, const uint8_t *V32, int n, int m, int label_id, uint8_t *out_chal, uint8_t out_digest[32]) {
+    transcript t; transcript_init(&t, label_id ? "L2RangeProof" : "RangeProof");
+    return rp_challenges(proof, proof_len, V32, &t, m, n, out_chal, out_digest);
 }
 
 /* ============================ l2_range_proof_vec (l2_range_proof_vec/mod.rs) ==================== */

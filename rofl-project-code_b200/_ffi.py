@@ -88,6 +88,7 @@ _SIGS = {
     "rofl_debug_verify_weights": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, c_sz, C.c_int, c_u8p, c_u8p]),
     "rofl_debug_msm": (C.c_int, [c_vp, c_u8p, c_sz, c_sz, c_u8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_sz, c_u8p, c_u8p, c_u8p, c_vp]),
     "rofl_debug_rlc_terms": (C.c_int, [c_vp, C.c_int, c_sz, c_sz, c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_vp, c_u8p, c_u8p, c_vp, c_vp, c_vp, c_vp]),
+    "rofl_debug_range_terms": (C.c_int, [c_vp, C.c_int, c_u8p, c_sz, c_sz, c_u8p, c_sz, c_sz, C.c_int, c_sz, c_sz, c_u8p, c_vp, c_vp, c_u8p, c_u8p, c_vp, c_vp, c_vp]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGS)
 
@@ -389,6 +390,43 @@ class Api:
             ranges.append(dict(i0=i0, n=n, c=w, wbits=wbits, is_id=(id0, id1), scal=sc[os_:os_ + T], sB=(coef[j, 0].tobytes(), coef[j, 1].tobytes()),
                                sH=(coef[j, 2].tobytes(), coef[j, 3].tobytes()), bad=bad[ob:ob + nb].tolist()))
         return dict(held=rc, root=root.tobytes(), chal=chal, verdicts=verd.tolist(), ranges=ranges)
+    def debug_range_terms(self, mode, proofs, commits, rng, seed, chunk_len=0, chunk_begin=0):
+        """The range-proof batched check of one public call, record by record (rofl_debug_range_terms).  mode 0 range_verify (chunk_len > 0: the
+        shard call), proofs [n_proofs, plen], commits [D, 32]; 1 range_verify_batch, proofs [K, n_proofs, plen], commits [K, D, 32]; 2 l2_verify,
+        proof [plen], commit [32]; 3 the L2 batch, proofs [K, plen], commits [K, 32].
+        -> dict(verdicts [K], recs: list of dicts (C, n, m, lgN, c_off, dom, rt (1 generator tables), win (window width), id, vch [C, 4 + lgN, 32], cs [C, 32], rho [C, 32],
+        chal [C, 5 + 2 lgN, 32], var [C m, 32], small [C, 6 + 2 lgN, 32], g [N, 32], h [N, 32], digest [C, 32], bad [C]))"""
+        p = _u8(proofs)
+        if mode == 1:
+            K = p.shape[0]; p = p.reshape(K, p.shape[1], -1); c = _u8(commits).reshape(K, -1, 32); npf, plen, D = p.shape[1], p.shape[2], c.shape[1]
+        elif mode == 3:
+            K = p.shape[0]; p = p.reshape(K, -1); c = _u8(commits).reshape(K, 32); npf, plen, D = 1, p.shape[1], 1
+        elif mode == 0:
+            K = 1; p = p.reshape(p.shape[0], -1); c = _u8(commits).reshape(-1, 32); npf, plen, D = p.shape[0], p.shape[1], c.shape[0]
+        else:
+            K = 1; p = p.reshape(-1); c = _u8(commits, 32); npf, plen, D = 1, p.size, 1
+        cap = np.array([4 + K, 1 << 16, 4 * K * npf], np.uintp)
+        for _ in range(2):                                   # a second call only when the first capacities were short
+            cnt = np.zeros(3, np.uintp); verd = np.zeros(K, np.int32); info = np.zeros((int(cap[0]), 12), np.int64)
+            sc = np.zeros((int(cap[1]), 32), np.uint8); dig = np.zeros((int(cap[2]), 32), np.uint8); bad = np.zeros(int(cap[2]), np.int32)
+            rc = self.lib.rofl_debug_range_terms(self.h, mode, _ptr(p), plen, npf, _ptr(c), D, K, rng, chunk_len, chunk_begin, _ptr(_u8(seed, 32)), _ptr(verd),
+                                                 _ptr(info), _ptr(sc), _ptr(dig), _ptr(bad), _ptr(cap), _ptr(cnt))
+            if rc == -2 and (cnt > cap).any():
+                cap = np.maximum(cap, cnt); continue
+            break
+        if rc < 0: raise self._err(rc)
+        recs = []
+        for j in range(int(cnt[0])):
+            Cn, n, m, lgN, c_off, dom, rt, cw, ok, os_, ns, oc = (int(x) for x in info[j])
+            N, chs, nsm = 1 << lgN, 5 + 2 * lgN, 6 + 2 * lgN
+            parts, o = {}, os_
+            for name, size in (("vch", Cn * (4 + lgN)), ("cs", Cn), ("rho", Cn), ("chal", Cn * chs), ("var", Cn * m), ("small", Cn * nsm), ("g", N), ("h", N)):
+                parts[name] = sc[o:o + size]; o += size
+            assert o == os_ + ns
+            recs.append(dict(C=Cn, n=n, m=m, lgN=lgN, c_off=c_off, dom=dom, rt=rt, win=cw, id=ok, vch=parts["vch"].reshape(Cn, 4 + lgN, 32), cs=parts["cs"],
+                             rho=parts["rho"], chal=parts["chal"].reshape(Cn, chs, 32), var=parts["var"], small=parts["small"].reshape(Cn, nsm, 32),
+                             g=parts["g"], h=parts["h"], digest=dig[oc:oc + Cn], bad=bad[oc:oc + Cn].tolist()))
+        return dict(verdicts=verd.tolist(), recs=recs)
     def debug_verify_weights(self, proofs, commits, rng, seed):
         p = _u8(proofs); p = p.reshape(p.shape[0], -1); c = _u8(commits).reshape(-1, 32); w = np.zeros((2, p.shape[0], 32), np.uint8)
         rc = self.lib.rofl_debug_verify_weights(self.h, _ptr(p), p.shape[1], p.shape[0], _ptr(c), c.shape[0], rng, _ptr(_seed(seed)), _ptr(w))

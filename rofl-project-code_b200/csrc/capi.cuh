@@ -815,7 +815,56 @@ extern "C" int rofl_debug_verify_weights(rofl_ctx *c, const uint8_t *proofs, siz
     if (!D) return ROFL_ERR_ARGS;
     lane_guard lg(c->e);
     staged_in dc(commits, 32 * D, lg.s());
-    return engine_range_verify(c->e, proofs, plen, np, dc.b.as<uint8_t>(), D, range, seed, nullptr, out_weights);
+    range_tap tap;
+    const int rc = engine_range_verify(c->e, proofs, plen, np, dc.b.as<uint8_t>(), D, range, seed, nullptr, &tap);
+    if (!tap.recs.empty()) memcpy(out_weights, tap.recs[0].ccrho.data(), sizeof(sc_st) * tap.recs[0].ccrho.size());
+    return rc;
+    API_CATCH
+}
+// the range-proof batched check of one public call, record by record (engine.cuh range_tap; derived by nothing here).  mode 0 rofl_range_verify
+// (chunk_len > 0: rofl_range_verify_shard), 1 rofl_range_verify_batch, 2 rofl_l2_verify, 3 the L2 batch of the server calls.  See include/rofl_b200.h.
+extern "C" int rofl_debug_range_terms(rofl_ctx *c, int mode, const uint8_t *proofs, size_t plen, size_t n_proofs, const uint8_t *commits32, size_t D, size_t n_clients,
+                                      int range, size_t chunk_len, size_t chunk_begin, const uint8_t seed[32], int *verdicts, int64_t *recs, uint8_t *scalars32,
+                                      uint8_t *digest32, int *bad, const size_t cap[3], size_t cnt[3]) {
+    API_TRY
+    const size_t K = n_clients;
+    if (mode < 0 || mode > 3 || !K || !proofs || !commits32 || !seed || !verdicts || !recs || !scalars32 || !digest32 || !bad || !cap || !cnt) return ROFL_ERR_ARGS;
+    if ((mode == 0 || mode == 2) && K != 1) return ROFL_ERR_ARGS;
+    if (mode <= 1 && (!D || !n_proofs)) return ROFL_ERR_ARGS;
+    range_tap tap;
+    {
+        lane_guard lg(c->e);
+        const size_t ncom = mode <= 1 ? K * D : K;
+        staged_in dc(commits32, 32 * ncom, lg.s());
+        if (mode == 0) {
+            shard_spec sh = {chunk_len, chunk_begin, n_proofs};
+            verdicts[0] = engine_range_verify(c->e, proofs, plen, n_proofs, dc.b.as<uint8_t>(), D, range, seed, chunk_len ? &sh : nullptr, &tap);
+        } else if (mode == 1) {
+            const int rc = engine_range_verify_batch(c->e, proofs, plen, n_proofs, dc.b.as<uint8_t>(), D, K, range, seed, verdicts, &tap);
+            if (rc < 0) return rc;
+        } else if (mode == 2) {
+            verdicts[0] = engine_l2_verify(c->e, proofs, plen, commits32, range, seed, &tap);
+        } else {
+            const int rc = engine_l2_verify_batch(c->e, proofs, plen, commits32, K, range, seed, verdicts, &tap);
+            if (rc < 0) return rc;
+        }
+    }
+    size_t nsc = 0, nch = 0;
+    for (const auto &r : tap.recs) { nsc += r.vch.size() + r.ccrho.size() + r.chal.size() + r.var.size() + r.gh.size(); nch += (size_t)r.C; }
+    cnt[0] = tap.recs.size(); cnt[1] = nsc; cnt[2] = nch;
+    if (cnt[0] > cap[0] || nsc > cap[1] || nch > cap[2]) return ROFL_ERR_ARGS;
+    size_t os = 0, oc = 0;
+    for (size_t j = 0; j < tap.recs.size(); j++) {
+        const range_tap::rec &r = tap.recs[j];
+        const size_t ns = r.vch.size() + r.ccrho.size() + r.chal.size() + r.var.size() + r.gh.size();
+        const int64_t info[12] = {r.C, r.n, r.m, r.lgN, (int64_t)r.c_off, r.dom, r.rt, r.c, r.id, (int64_t)os, (int64_t)ns, (int64_t)oc};
+        memcpy(recs + 12 * j, info, sizeof(info));
+        for (const std::vector<sc_st> *v : {&r.vch, &r.ccrho, &r.chal, &r.var, &r.gh}) { memcpy(scalars32 + 32 * os, v->data(), sizeof(sc_st) * v->size()); os += v->size(); }
+        memcpy(digest32 + 32 * oc, r.digest.data(), r.digest.size());
+        memcpy(bad + oc, r.bad.data(), sizeof(int) * r.bad.size());
+        oc += (size_t)r.C;
+    }
+    return 0;
     API_CATCH
 }
 // the MSM front end alone: out32[k] = sum_t s[k][t] P_t (+ sB[k] B + sH[k] H), k < n_msm, through the production plan / kernels / k_finalize.

@@ -797,8 +797,20 @@ static inline int range_proof_format_check(const uint8_t *h_proofs, size_t plen,
     if (lg_out) *lg_out = lg;
     return 0;
 }
+// Test hook (rofl_debug_range_terms): every verify_chunks invocation that builds the batched equation appends one record, copied from the device
+// buffers it already filled; nothing is derived here.  With a null tap verify_chunks issues exactly its production launches and copies.
+struct range_tap {
+    struct rec {
+        int C = 0, n = 0, m = 0, lgN = 0; uint64_t c_off = 0; uint32_t dom = 0;
+        int rt = 0, c = 0;                              // fixed-generator MSM: 1 generator tables (k_rt_msm), 0 bucket MSM; its window width
+        std::vector<sc_st> vch, ccrho, chal, var, gh;   // y z x w u_0.. per chunk | c_i, rho_i | chal blocks | C m commitment + C nsmall small-point scalars | g, h
+        std::vector<uint8_t> digest; std::vector<int> bad; int id = 0;
+    };
+    std::vector<rec> recs;
+};
 static int verify_chunks(rofl_engine &e, cudaStream_t s, int label_id, int n, int m, int C, const gens_entry &g, const rt_tables *rt, const p3_st *d_Vp3, const uint8_t *d_V32,
-                         const uint8_t *h_proofs, size_t plen, const uint8_t seed[32], uint32_t dom, uint64_t c_off, std::vector<int> &verdict, const int *d_xbad = nullptr, int *h_xbad = nullptr, uint8_t *h_weights = nullptr, size_t nx = 1) {
+                         const uint8_t *h_proofs, size_t plen, const uint8_t seed[32], uint32_t dom, uint64_t c_off, std::vector<int> &verdict, const int *d_xbad = nullptr, int *h_xbad = nullptr,
+                         range_tap *tap = nullptr, size_t nx = 1) {
     verdict.assign(C, 0);
     phase_trace tr(s);
     size_t lg = 0;
@@ -872,9 +884,17 @@ static int verify_chunks(rofl_engine &e, cudaStream_t s, int label_id, int n, in
     std::vector<int> h_bad(C); int h_id = 0;
     rt_d2h(&h_id, d_id.p, sizeof(int), s); rt_d2h(h_bad.data(), d_bad.p, sizeof(int) * C, s);
     if (d_xbad) rt_d2h(h_xbad, d_xbad, sizeof(int) * nx, s);
-    if (h_weights) rt_d2h(h_weights, d_ccrho.p, sizeof(sc_st) * 2 * (size_t)C, s);
     rt_sync(s);
     tr.mark("v_final");
+    if (tap) {
+        range_tap::rec r; r.C = C; r.n = n; r.m = m; r.lgN = lgN; r.c_off = c_off; r.dom = dom; r.rt = rt ? 1 : 0; r.c = rt ? rt->c : plF.c; r.id = h_id; r.bad = h_bad;
+        auto get = [&](std::vector<sc_st> &v, const dev_buf &d, size_t count) { v.resize(count); rt_d2h(v.data(), d.p, sizeof(sc_st) * count, s); };
+        get(r.vch, d_vch, (size_t)C * (4 + lgN)); get(r.ccrho, d_ccrho, 2 * (size_t)C); get(r.chal, d_chal, (size_t)C * chs);
+        get(r.var, d_var, (size_t)C * vstride); get(r.gh, d_gh, 2 * N);
+        r.digest.resize(32 * (size_t)C); rt_d2h(r.digest.data(), d_digest.p, 32 * (size_t)C, s);
+        rt_sync(s);
+        tap->recs.push_back(std::move(r));
+    }
     int all_ok = h_id;
     for (int c = 0; c < C; c++) all_ok &= h_bad[c] ? 0 : 1;
     for (int c = 0; c < C; c++) verdict[c] = all_ok;
@@ -884,7 +904,7 @@ static int verify_chunks(rofl_engine &e, cudaStream_t s, int label_id, int n, in
 // range_proof_vec::verify_rangeproof (range_proof_vec/mod.rs:149-191).  d_commits: D compressed points (device).
 // returns 1 true, 0 false, -1 FormatError, -7 InvalidBitsize, -2 bad args, -3 InvalidGeneratorsLength, -4 undecodable commitment
 static int engine_range_verify(rofl_engine &e, const uint8_t *h_proofs, size_t plen, size_t n_proofs, const uint8_t *d_commits, size_t D,
-                               int range, const uint8_t seed[32], const shard_spec *shard = nullptr, uint8_t *h_weights = nullptr) {
+                               int range, const uint8_t seed[32], const shard_spec *shard = nullptr, range_tap *tap = nullptr) {
     if (n_proofs == 0 || range < 1 || range > 64) return -2;
     if (shard ? (shard->m == 0 || shard->n_chunks != n_proofs || D > shard->m * shard->n_chunks) : D == 0) return -2;
     lane_guard lg(e);
@@ -910,7 +930,7 @@ static int engine_range_verify(rofl_engine &e, const uint8_t *h_proofs, size_t p
     const gens_entry g = engine_gens(e, tu, s, range, (int)m);
     // one group: every chunk goes into the same batched check (kernels.cuh, k_verify_scalars), splitting would repeat the generator MSM
     std::vector<int> verdict; int bad = 0;
-    const int rc = verify_chunks(e, s, 0, range, (int)m, (int)C, g, have_rt ? &rt : nullptr, d_Vp3.as<p3_st>(), d_V32.as<uint8_t>(), h_proofs, plen, seed, DOM_RANGE_VERIFY, c_off, verdict, d_bad.as<int>(), &bad, h_weights);
+    const int rc = verify_chunks(e, s, 0, range, (int)m, (int)C, g, have_rt ? &rt : nullptr, d_Vp3.as<p3_st>(), d_V32.as<uint8_t>(), h_proofs, plen, seed, DOM_RANGE_VERIFY, c_off, verdict, d_bad.as<int>(), &bad, tap);
     if (bad) return -4;
     if (rc < 0) return rc;
     int res = 1; for (int v : verdict) res &= v;                               // :183-190
@@ -926,7 +946,7 @@ static int engine_range_verify(rofl_engine &e, const uint8_t *h_proofs, size_t p
 // re-checked one by one, so that the verdict names the offender exactly as the reference's per-client results do.
 // =============================================================================================================================
 static int engine_range_verify_batch(rofl_engine &e, const uint8_t *h_proofs, size_t plen, size_t n_proofs, const uint8_t *d_commits, size_t D, size_t K,
-                                     int range, const uint8_t seed[32], int *out) {
+                                     int range, const uint8_t seed[32], int *out, range_tap *tap = nullptr) {
     if (n_proofs == 0 || D == 0 || range < 1 || range > 64 || !out) return -2;
     if (K == 0) return 0;
     lane_guard lg(e);
@@ -947,16 +967,17 @@ static int engine_range_verify_batch(rofl_engine &e, const uint8_t *h_proofs, si
         const gens_entry g = engine_gens(e, tu, s, range, (int)m);
         std::vector<int> verdict, bad(K, 0);
         const int rc = verify_chunks(e, s, 0, range, (int)m, (int)(K * n_proofs), g, have_rt ? &rt : nullptr, d_Vp3.as<p3_st>(), d_V32.as<uint8_t>(), h_proofs, plen, seed, DOM_RANGE_VERIFY, 0, verdict,
-                                     d_bad.as<int>(), bad.data(), nullptr, K);
+                                     d_bad.as<int>(), bad.data(), tap, K);
         bool all = rc == 0; for (int v : verdict) all = all && v == 1; for (int b : bad) all = all && !b;
         if (all) { for (size_t k = 0; k < K; k++) out[k] = 1; return 0; }
     }
-    for (size_t k = 0; k < K; k++) out[k] = engine_range_verify(e, h_proofs + k * n_proofs * plen, plen, n_proofs, d_commits + 32 * k * D, D, range, seed);
+    for (size_t k = 0; k < K; k++) out[k] = engine_range_verify(e, h_proofs + k * n_proofs * plen, plen, n_proofs, d_commits + 32 * k * D, D, range, seed, nullptr, tap);
     return 0;
 }
-static int engine_l2_verify(rofl_engine &e, const uint8_t *h_proof, size_t plen, const uint8_t *h_commit, int range, const uint8_t seed[32]);
+static int engine_l2_verify(rofl_engine &e, const uint8_t *h_proof, size_t plen, const uint8_t *h_commit, int range, const uint8_t seed[32], range_tap *tap = nullptr);
 // K sum-of-squares proofs (l2_range_proof_vec::verify_rangeproof_l2, :185-228) in one batched check; h_commits: K x 32
-static int engine_l2_verify_batch(rofl_engine &e, const uint8_t *h_proofs, size_t plen, const uint8_t *h_commits, size_t K, int range, const uint8_t seed[32], int *out) {
+static int engine_l2_verify_batch(rofl_engine &e, const uint8_t *h_proofs, size_t plen, const uint8_t *h_commits, size_t K, int range, const uint8_t seed[32], int *out,
+                                  range_tap *tap = nullptr) {
     if (!out) return -2;
     if (K == 0) return 0;
     lane_guard lg(e);
@@ -969,11 +990,11 @@ static int engine_l2_verify_batch(rofl_engine &e, const uint8_t *h_proofs, size_
         tables_use tu(*e.sh);
         const gens_entry g = engine_gens(e, tu, s, range, 1);
         std::vector<int> verdict, bad(K, 0);
-        const int rc = verify_chunks(e, s, 1, range, 1, (int)K, g, nullptr, d_Vp3.as<p3_st>(), d_V32.as<uint8_t>(), h_proofs, plen, seed, DOM_L2_VERIFY, 0, verdict, d_bad.as<int>(), bad.data(), nullptr, K);
+        const int rc = verify_chunks(e, s, 1, range, 1, (int)K, g, nullptr, d_Vp3.as<p3_st>(), d_V32.as<uint8_t>(), h_proofs, plen, seed, DOM_L2_VERIFY, 0, verdict, d_bad.as<int>(), bad.data(), tap, K);
         bool all = rc == 0; for (int v : verdict) all = all && v == 1; for (int b : bad) all = all && !b;
         if (all) { for (size_t k = 0; k < K; k++) out[k] = 1; return 0; }
     }
-    for (size_t k = 0; k < K; k++) out[k] = engine_l2_verify(e, h_proofs + k * plen, plen, h_commits + 32 * k, range, seed);
+    for (size_t k = 0; k < K; k++) out[k] = engine_l2_verify(e, h_proofs + k * plen, plen, h_commits + 32 * k, range, seed, tap);
     return 0;
 }
 
@@ -1026,7 +1047,7 @@ static int engine_l2_prove(rofl_engine &e, const float *h_values, const float *d
     return 0;
 }
 // verify_rangeproof_l2 (:185-228)
-static int engine_l2_verify(rofl_engine &e, const uint8_t *h_proof, size_t plen, const uint8_t *h_commit, int range, const uint8_t seed[32]) {
+static int engine_l2_verify(rofl_engine &e, const uint8_t *h_proof, size_t plen, const uint8_t *h_commit, int range, const uint8_t seed[32], range_tap *tap) {
     lane_guard lg(e);
     cudaStream_t s = lg.s();
     if (range_proof_format_check(h_proof, plen, 1, nullptr)) return -1;
@@ -1040,7 +1061,7 @@ static int engine_l2_verify(rofl_engine &e, const uint8_t *h_proof, size_t plen,
     tables_use tu(*e.sh);
     const gens_entry g = engine_gens(e, tu, s, range, 1);
     std::vector<int> verdict; int bad = 0;
-    const int rc = verify_chunks(e, s, 1, range, 1, 1, g, nullptr, d_Vp3.as<p3_st>(), d_V32.as<uint8_t>(), h_proof, plen, seed, DOM_L2_VERIFY, 0, verdict, d_bad.as<int>(), &bad);
+    const int rc = verify_chunks(e, s, 1, range, 1, 1, g, nullptr, d_Vp3.as<p3_st>(), d_V32.as<uint8_t>(), h_proof, plen, seed, DOM_L2_VERIFY, 0, verdict, d_bad.as<int>(), &bad, tap);
     if (bad) return -4;
     if (rc < 0) return rc;
     return verdict.empty() ? 0 : verdict[0];
